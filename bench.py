@@ -1,7 +1,17 @@
 """Headline benchmark: 3D patch pairs/s of the full G+D WGAN train step (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs bench_outputs]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+`--dump-outputs DIR` (one GPU): after every measurement, the trainer is put back into its seeded initial state (weights,
+BatchNorm statistics, empty Adam state) and runs the timed step once more on the same resident inputs, eagerly: the same
+Trainer.train_step calls that the CUDA graph of the headline loop replays.  What that step hands its caller is written as
+DIR/<name>.npy: the returned losses (`loss_<key>`) and the generator / critic state it leaves behind
+(`generator.<state_dict key>`, `critic.<state_dict key>`), float32 (integer counters float64), about 5 MB.  Two runs, or
+two builds, with the same arguments can be compared file by file.  The last step of a timed loop is not dumped because it
+is not reproducible: weight gradients are summed with floating-point atomics, and the Adam steps before it (28 by the end
+of the headline loop at the defaults) amplify that rounding noise to whole learning-rate steps in the weights; two runs of
+one build on a B200 differed there by up to a third of a weight tensor's largest entry.
 
 Workload (SURVEY §8d): per GPU 16 opt + 8 low + 8 high synthetic HU-scaled 1x128^3 patches (BASELINE config C3;
 weak scaling: the same per GPU at N>1 with the gradients of G and D averaged over ranks), bf16 storage / fp32
@@ -147,6 +157,17 @@ def raw_hu_batch(batch, pin=True):
     return out
 
 
+def step_outputs(tr, logs):
+    """Host copies of what one Trainer.train_step gives its caller: the loss dict it returns and the generator / critic
+    state_dict it leaves behind."""
+    out = {f"loss_{k}": v.detach().float().cpu().numpy() for k, v in logs.items()}
+    for net, mod in (("generator", tr.generator), ("critic", tr.critic)):
+        for k, v in mod.state_dict().items():
+            v = v.detach().cpu()
+            out[f"{net}.{k}"] = (v.float() if v.is_floating_point() else v.double()).numpy()
+    return out
+
+
 def bench_c2(generator, dev, pk):
     """BASELINE config C2: generator-only correction of one synthetic 512 x 512 x 256 int16 CCTA volume tiled into 32 128^3
     patches, batches of 16 (reference eval/CCTAContrastCorrector.py:60-106), through CCTAContrastCorrector.__call__ (host
@@ -274,7 +295,7 @@ def run_reference(args):
     cores = len(os.sched_getaffinity(0))
     patch = (args.patch,) * 3
     n_opt, n_low, n_high = 2, 1, 1
-    steps = max(args.steps, 5) if not args.quick_cpu else args.steps
+    steps = args.steps
     warmup = max(args.warmup, 2) if not args.quick_cpu else args.warmup
     t, kind = _time_cpu_steps(patch, n_opt, n_low, n_high, warmup, steps, cores)
     v = n_opt / t
@@ -299,7 +320,8 @@ def run_reference(args):
 def shutdown(tr=None, dist=None, world=1):
     """Leave without hanging: CUDA graphs that recorded NCCL kernels must be gone before the communicator is torn down
     (destroying the process group under a live graph blocked the NCCL watchdog for minutes), and the teardown itself runs
-    in a helper thread with a deadline; the process then exits with status 0 whatever NCCL does."""
+    in a helper thread with a deadline; a rank of a multi-GPU run then exits with status 0 whatever NCCL does.  A single
+    process has no communicator to wait for and returns to the normal interpreter exit, which runs the exit handlers."""
     import gc
 
     import torch
@@ -314,7 +336,8 @@ def shutdown(tr=None, dist=None, world=1):
         t.start()
         t.join(timeout=20)
     sys.stdout.flush(); sys.stderr.flush()
-    os._exit(0)
+    if world > 1:
+        os._exit(0)
 
 
 def main():
@@ -328,11 +351,18 @@ def main():
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "f32"])
     ap.add_argument("--conv-impl", default="auto", choices=["auto", "generic", "tc"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--quick-cpu", action="store_true", help="reference arm: exactly --steps/--warmup steps, no 1-thread line")
+    ap.add_argument("--quick-cpu", action="store_true", help="reference arm: exactly --warmup warm-up steps, no 1-thread line")
     ap.add_argument("--breakdown", default=None, help="write the per-conv-kernel device-time table of the timed region here")
     ap.add_argument("--no-graph", action="store_true", help="run every step eagerly (default: the step is replayed from a CUDA graph)")
     ap.add_argument("--no-extras", action="store_true", help="skip the c4 (8 pairs per GPU) and c2 (whole-volume inference) objects")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the measurements, write the losses and post-step weights of one timed step from the seeded "
+                         "initial state as DIR/<name>.npy (one GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.gpus != 1:
+        ap.error("--dump-outputs needs --gpus 1")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
@@ -374,6 +404,7 @@ def main():
                  hu_scaler=FactorZeroCenterScaler(-1024, 1500, 600))
     broadcast_module(tr.generator); broadcast_module(tr.critic)
     tr.generator.train(); tr.critic.train()
+    initial = [{k: v.detach().clone() for k, v in m.state_dict().items()} for m in (tr.generator, tr.critic)] if args.dump_outputs else None
 
     gen = torch.Generator().manual_seed(1 + rank)
     host = synth_batch(gen, n_opt, n_low, n_high, patch, pin=True)
@@ -583,6 +614,19 @@ def main():
         "cuda_graph": not args.no_graph,
         "losses_last_step": {k: float(v.detach()) for k, v in logs.items()},
     }
+    if args.dump_outputs:  # after every measurement: this resets the trainer
+        import numpy as np
+
+        # eager: a captured step would keep its device-side Adam step count; an eager FusedAdam step mirrors the host's
+        tr.release_cuda_graphs()
+        for m, sd in zip((tr.generator, tr.critic), initial):
+            m.load_state_dict(sd)
+        tr.optimizer_G.state.clear(); tr.optimizer_D.state.clear()
+        dump = step_outputs(tr, tr.train_step(resident, 0))
+        d = Path(args.dump_outputs)
+        d.mkdir(parents=True, exist_ok=True)
+        for name, a in dump.items():
+            np.save(d / f"{name}.npy", a)
     print(json.dumps(out), flush=True)
     shutdown(tr, dist, world)
 

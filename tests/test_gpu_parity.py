@@ -658,6 +658,38 @@ def test_cuda_graphed_step_equals_eager_step(dtype):
             assert float((va.float() - vb.float()).abs().mean()) < 1e-4, k
 
 
+def test_step_after_reset_to_initial_state_is_a_first_step():
+    """What bench.py --dump-outputs relies on: after graph-replayed steps (which advance FusedAdam's device-side step
+    count without running its Python code), releasing the graphs, loading the initial state_dicts and clearing the
+    optimizers' state make the next step the first step of a fresh trainer (host and device step counts included)."""
+    a, b = _make_trainer(torch.float32), _make_trainer(torch.float32)
+    initial = [{k: v.detach().clone() for k, v in m.state_dict().items()} for m in (b.generator, b.critic)]
+    opt, low, high, ml, mh = _batches(torch.Generator().manual_seed(17), (32, 32, 32))
+    p = [dict(data=opt, seg=None, name=[]), dict(data=low, seg=ml, name=[]), dict(data=high, seg=mh, name=[])]
+    la = {k: float(v) for k, v in a.train_step(p, 0).items()}
+    b.enable_cuda_graph(warmup=2)
+    for _ in range(4):  # two eager warm-ups, the capture, one replay
+        b.train_step(p, 0)
+    assert all(e["graph"] is not None for e in b._graphs["entries"].values())
+    b.release_cuda_graphs()
+    for m, sd in zip((b.generator, b.critic), initial):
+        m.load_state_dict(sd)
+    b.optimizer_G.state.clear(); b.optimizer_D.state.clear()
+    lb = {k: float(v) for k, v in b.train_step(p, 0).items()}
+    for k in la:  # same kernels; fp atomics order differs between runs
+        assert abs(la[k] - lb[k]) <= 2e-3 * abs(la[k]) + 1e-4, (k, la[k], lb[k])
+    for o in (b.optimizer_G, b.optimizer_D):
+        assert {o.state[q]["step"] for q in o.param_groups[0]["params"]} == {1}
+        assert float(o._dev[id(o.param_groups[0])]["hyper"][1]) == 1.0
+    for ma, mb in ((a.generator, b.generator), (a.critic, b.critic)):
+        for (k, va), vb in zip(ma.state_dict().items(), mb.state_dict().values()):
+            if "num_batches" in k:
+                assert int(va) == int(vb), k
+            else:  # one Adam step moves a weight by at most lr; a near-zero gradient may flip its sign
+                assert_close32(vb, va, rtol=1e-3, atol=2 * 2e-4, msg=k)
+                assert float((va.float() - vb.float()).abs().mean()) < 1e-5, k
+
+
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16], ids=["f32", "bf16"])
 def test_rmsprop_small_patch_configuration_against_oracle(dtype):
     """The reference's rmsprop_conf.py (RMSprop for both networks, which star-imports small_patch_size.py: non-cubic
