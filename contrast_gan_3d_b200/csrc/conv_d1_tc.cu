@@ -22,18 +22,12 @@ namespace cg {
 using bf16 = __nv_bfloat16;
 constexpr uint32_t kSmemLimitD1 = 232448 - 1024;
 
-typedef CUresult (*EncodeTiledFnD)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-void *tc_encode_fn_ptr();  // conv_tc.cu
-CUtensorMapL2promotion tc_l2_promo();  // conv_tc.cu
-
 static int encode_map_d1(CUtensorMap *tm, const void *ptr, int rank, const cuuint64_t *gdim, const cuuint64_t *gstr,
                          const cuuint32_t *box, const cuuint32_t *estr) {
-  EncodeTiledFnD enc = reinterpret_cast<EncodeTiledFnD>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, tc_l2_promo(),
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (critic first layer) failed with %d", (int)r);
   return 0;

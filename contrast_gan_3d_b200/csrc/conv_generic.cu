@@ -936,9 +936,7 @@ int reflect_pad_backward(const void *gp, void *gi, int dtype, int B, int X, int 
   const int esz = dtype == CGAN3D_F32 ? 4 : 2;
   if ((C * esz) % 16 == 0 && !((uintptr_t)gp & 15) && !((uintptr_t)gi & 15) && X <= 65535 && B <= 65535) {
     const int cpv = C * esz / 16;
-    static int lpb_env = -1;
-    if (lpb_env < 0) { const char *e = getenv("CGAN3D_PADBWD_LPB"); lpb_env = e ? mx(1, atoi(e)) : 0; }
-    const int lpb = lpb_env ? lpb_env : ((int64_t)B * X * Y >= 65536 && Z * cpv <= 512 ? 4 : 1);
+    const int lpb = (int64_t)B * X * Y >= 65536 && Z * cpv <= 512 ? 4 : 1;
     const dim3 bl((unsigned)((Y + lpb - 1) / lpb), (unsigned)X, (unsigned)B);
     if (dtype == CGAN3D_F32)
       reflect_pad_bwd_vec_kernel<float><<<bl, 256, 0, st>>>((const uint4 *)gp, (uint4 *)gi, B, X, Y, Z, cpv, pad, lpb);

@@ -21,7 +21,6 @@
 #include "common.cuh"
 #include "conv_internal.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace cg {
 
@@ -691,11 +690,7 @@ __global__ void repack_b_kernel(const bf16 *__restrict__ wp, bf16 *__restrict__ 
 }
 
 // ---------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                  const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeTiledFn encode_fn() {
+EncodeTiledFn tc_encode_fn() {
   static EncodeTiledFn fn = nullptr;
   static bool tried = false;
   if (!tried) {
@@ -709,32 +704,8 @@ static EncodeTiledFn encode_fn() {
   return fn;
 }
 
-void *tc_encode_fn_ptr() { return reinterpret_cast<void *>(encode_fn()); }
-
-// L2 fetch granularity of every TMA tensor map.  CGAN3D_L2PROMO = 0 (none) / 64 / 128 / 256 overrides the default.
-CUtensorMapL2promotion tc_l2_promo() {
-  static int v = -1;
-  if (v < 0) {
-    const char *e = getenv("CGAN3D_L2PROMO");
-    v = e ? atoi(e) : 128;
-  }
-  return v == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE
-                : (v == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B : (v == 256 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : CU_TENSOR_MAP_L2_PROMOTION_L2_128B));
-}
-
-// conv_tc_prog.cu
-bool tc_prog_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t tc_prog_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                cudaStream_t st, double *bn_sums = nullptr);
-bool tc_prog_fuses_bnstats(const cgan3d_conv_geom &g, int scatter);
-
 // CTA pairs need whole-voxel swizzled planes (one TMA box per plane), N/2 a multiple of 16 and 256-byte weight-map rows.
-static bool pair_ok(int Cin, int N) {
-  static int off = -1;
-  if (off < 0) off = getenv("CGAN3D_NO_PAIR") ? 1 : 0;
-  return !off && Cin <= 64 && N % 32 == 0 && (Cin * N) % 256 == 0;
-}
+static bool pair_ok(int Cin, int N) { return Cin <= 64 && N % 32 == 0 && (Cin * N) % 256 == 0; }
 
 static bool plan_s1(int B, int X, int Y, int Z, int Cin, int N, TcPlan &best) {
   if (N % 16 || N > 256 || N < 16) return false;
@@ -746,11 +717,7 @@ static bool plan_s1(int B, int X, int Y, int Z, int Cin, int N, TcPlan &best) {
   p.Zt = (Z + p.nzt - 1) / p.nzt;
   p.Zh = p.Zt + 2;
   p.btile_bytes = (uint32_t)Cin * N * 2 / (p.pair ? 2 : 1);
-  {
-    static int tps_env = -1;
-    if (tps_env < 0) { const char *e = getenv("CGAN3D_TPS"); tps_env = e ? atoi(e) : 0; }
-    p.tps = tps_env == 1 ? 1 : (3 * p.btile_bytes <= 16384 ? 3 : 1);
-  }
+  p.tps = 3 * p.btile_bytes <= 16384 ? 3 : 1;
   const uint32_t stage_b = (uint32_t)p.tps * p.btile_bytes;
   p.b_stages = stage_b <= 8192 ? 4 : (stage_b <= 16384 ? 3 : 2);
   double best_eff = 0;
@@ -777,9 +744,7 @@ static bool plan_s1(int B, int X, int Y, int Z, int Cin, int N, TcPlan &best) {
   TcPlan &q = best;
   {  // a deeper weight ring when shared memory is left over: one tap is consumed in mtiles * Cin/16 MMAs (~600 cycles for a
      // CTA pair at Cin = 64), well below the L2 latency of the next tile
-    static int max_stages = -1;
-    if (max_stages < 0) { const char *e = getenv("CGAN3D_B_STAGES"); max_stages = e ? atoi(e) : 12; }
-    while (q.b_stages < max_stages && q.smem_bytes + q.tps * q.btile_bytes <= kSmemLimit) { q.b_stages += 1; q.smem_bytes += q.tps * q.btile_bytes; }
+    while (q.b_stages < 12 && q.smem_bytes + q.tps * q.btile_bytes <= kSmemLimit) { q.b_stages += 1; q.smem_bytes += q.tps * q.btile_bytes; }
   }
   q.a_swz = Cin <= 64 ? 2 * Cin : 0;
   q.box_bytes = (q.a_swz ? (uint32_t)q.a_swz : 16u) * q.Zh * q.Yh;
@@ -794,11 +759,9 @@ static bool plan_s1(int B, int X, int Y, int Z, int Cin, int N, TcPlan &best) {
 
 
 // Tiling of the dz-stacked kernel: CTA pairs, whole-voxel swizzled planes, two M tiles of 2N accumulator columns, double
-// buffered.  CGAN3D_NO_STACK=1 keeps the one-tap-per-MMA kernel (A/B timing).
+// buffered.
 static bool plan_s1_stack(int B, int X, int Y, int Z, int Cin, int N, TcPlan &best) {
-  static int off = -1;
-  if (off < 0) off = getenv("CGAN3D_NO_STACK") ? 1 : 0;
-  if (off || !pair_ok(Cin, N)) return false;
+  if (!pair_ok(Cin, N)) return false;
   if (N > 64 || N % 32 || (Cin != 16 && Cin != 32 && Cin != 64)) return false;
   TcPlan p{};
   p.B = B; p.X = X; p.Y = Y; p.Z = Z; p.Cin = Cin; p.N = N;
@@ -844,30 +807,6 @@ static bool plan_s1_stack(int B, int X, int Y, int Z, int Cin, int N, TcPlan &be
   return true;
 }
 
-// conv_thin_tc.cu (7x7x7 thin-channel layers)
-bool thin_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t thin_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-int thin_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-             cudaStream_t st, double *bn_sums = nullptr);
-bool thin_fuses_bnstats(const cgan3d_conv_geom &g, int op);
-int thin_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-                   cudaStream_t st);
-
-// conv_d1_tc.cu (first critic layer: 1 -> 8 channels, k4 s2)
-bool d1_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t d1_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-int d1_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes, cudaStream_t st);
-int d1_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-                 cudaStream_t st);
-
-// wgrad_s2_tc.cu (stride-2 layers with Cs in {32, 64}, Cb in {16, 32}: swizzled whole-voxel operands, N = 4*Cb)
-bool tc_wgrad_s2_supported(const cgan3d_conv_geom &g);
-int tc_wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
-
-// wgrad_tc.cu
-bool tc_wgrad_supported(const cgan3d_conv_geom &g);
-int tc_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
-
 static bool s1_shape_ok(const cgan3d_conv_geom &g, int dtype, int op) {
   if (dtype != CGAN3D_BF16 || op < 0 || op > 1) return false;
   if (g.k != 3 || g.stride != 1 || g.pad != 1) return false;
@@ -876,7 +815,7 @@ static bool s1_shape_ok(const cgan3d_conv_geom &g, int dtype, int op) {
 }
 
 bool tc_supported(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (!cgan3d_device_supports_tc() || encode_fn() == nullptr) return false;
+  if (!cgan3d_device_supports_tc() || tc_encode_fn() == nullptr) return false;
   if (thin_supported(g, dtype, op) || d1_supported(g, dtype, op)) return true;
   if (op == 2) return dtype == CGAN3D_BF16 && (tc_wgrad_s2_supported(g) || tc_wgrad_supported(g));
   if (!s1_shape_ok(g, dtype, op)) return tc_prog_supported(g, dtype, op);
@@ -902,7 +841,7 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
   if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 31) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 conv: input / workspace must be 16-byte aligned, the output 32-byte aligned (256-bit stores)");
-  EncodeTiledFn enc = encode_fn();
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   bf16 *wb = reinterpret_cast<bf16 *>(ws);
   TcPlan ps;
@@ -924,8 +863,7 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
   const CUtensorMapSwizzle swz = p.a_swz == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
                                  : (p.a_swz == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : (p.a_swz == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE));
   CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(in), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, tc_l2_promo(),
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled failed with %d", (int)r);
   CUtensorMap tmw{};
   if (p.pair) {  // the repacked weights as rows of 256 bytes: one (tap, half) tile is btile_bytes / 256 rows
@@ -933,7 +871,7 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
     const cuuint64_t wstr[1] = {256};
     const cuuint32_t wbox[2] = {64, (cuuint32_t)(p.btile_bytes >> 8)};
     r = enc(&tmw, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wb, wdim, wstr, wbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, tc_l2_promo(), CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (weights) failed with %d", (int)r);
   }
   const long long work = (long long)(p.pair ? (p.nitems + 1) / 2 : p.nitems) * p.X;
@@ -1071,7 +1009,7 @@ int tc_wgrad(const cgan3d_conv_geom &g, const void *big, const void *small, floa
              cudaStream_t st) {
   if (thin_supported(g, CGAN3D_BF16, 2)) return thin_wgrad_run(g, big, small, dw, beta, ws, ws_bytes, st);
   if (d1_supported(g, CGAN3D_BF16, 2)) return d1_wgrad_run(g, big, small, dw, beta, ws, ws_bytes, st);
-  if (tc_wgrad_s2_supported(g) && !getenv("CGAN3D_WGRAD_V1")) return tc_wgrad_s2_run(g, big, small, dw, beta, st);
+  if (tc_wgrad_s2_supported(g)) return tc_wgrad_s2_run(g, big, small, dw, beta, st);
   return tc_wgrad_run(g, big, small, dw, beta, st);
 }
 

@@ -23,7 +23,6 @@
 //     the layers of this model), so the only streamed operand is the activation slab; each slab is released as soon
 //     as its taps are issued (ring of slots, no cross-plane reuse: these layers are L2/HBM-bound, SURVEY App. B).
 #include "conv_tc_prog_kernel.cuh"
-#include <stdlib.h>
 
 namespace cg {
 
@@ -263,9 +262,7 @@ static bool plan_prog_split(const cgan3d_conv_geom &g, int scatter, ProgPlan &be
   p.btile_bytes = (uint32_t)(paired ? 16 : Cin) * N * 2;
   p.Nmma = N; p.acc_stride = 0; p.mt_stride = N;  // acc_stride of the unstacked layout depends on mtiles (set below)
   // CTA pairs: one TMA box per slab (swizzled whole voxels or the 8-channel critic slabs) and N/2 a multiple of 16
-  static int pair_off = -1;
-  if (pair_off < 0) pair_off = getenv("CGAN3D_NO_PAIR") ? 1 : 0;
-  const bool pair_base = !pair_off && (paired || Cin <= 64);
+  const bool pair_base = paired || Cin <= 64;
   p.pair = (pair_base && N % 32 == 0) ? 1 : 0;
   if (p.pair) p.btile_bytes /= 2;
   if (scatter && 8 * N <= 256) {
@@ -277,9 +274,7 @@ static bool plan_prog_split(const cgan3d_conv_geom &g, int scatter, ProgPlan &be
   }
   const uint32_t b_total = (p.nbt * p.btile_bytes + 1023) / 1024 * 1024;
   if (b_total + 40000 > kSmemLimitProg) return false;
-  static int zpair_off = -1;
-  if (zpair_off < 0) zpair_off = getenv("CGAN3D_NO_ZPAIR") ? 1 : 0;  // A/B timing: per-class strided slab loads
-  const bool zpair = !zpair_off && !scatter && !paired && (Cin == 16 || Cin == 32) && g.k == 3 && g.Zb % 2 == 0;
+  const bool zpair = !scatter && !paired && (Cin == 16 || Cin == 32) && g.k == 3 && g.Zb % 2 == 0;
   p.zpair = zpair ? 1 : 0;
   const int a_swz = zpair ? 4 * Cin : ((!paired && Cin <= 64) ? 2 * Cin : 0);
   double best_score = 0;
@@ -344,8 +339,6 @@ size_t tc_prog_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
   return (((size_t)p.nbt * p.btile_bytes * (p.pair ? 2 : 1) + 255) / 256 * 256) * nsplit + 256;
 }
 
-void *tc_encode_fn_ptr();  // conv_tc.cu
-
 bool tc_prog_fuses_bnstats(const cgan3d_conv_geom &g, int scatter) {
   ProgPlan p;
   return plan_prog(g, scatter, p) && p.Nout <= 64;
@@ -361,7 +354,7 @@ int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const vo
   if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 strided conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 strided conv: pointers must be 16-byte aligned");
-  EncodeTiledFn2 enc = reinterpret_cast<EncodeTiledFn2>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   // input tensor: gather reads the big side with element strides 2 on z and y; scatter reads the small side densely
   const int Xi = scatter ? g.Xs : g.Xb, Yi = scatter ? g.Ys : g.Yb, Zi = scatter ? g.Zs : g.Zb, Ci = p.Cin;
@@ -379,8 +372,7 @@ int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const vo
   const CUtensorMapSwizzle swz = p.a_swz == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
                                  : (p.a_swz == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : (p.a_swz == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE));
   CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(in), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, tc_l2_promo(),
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (strided) failed with %d", (int)r);
   const long long total = (long long)p.B * p.nzt * p.nslabs * p.Xg;
   const int grid = p.pair ? 2 * (int)mn<long long>((total + 1) / 2, (long long)(num_sms() / 2)) : (int)mn<long long>(total, (long long)num_sms());

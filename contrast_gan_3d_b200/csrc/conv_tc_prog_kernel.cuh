@@ -27,7 +27,6 @@
 #include "common.cuh"
 #include "conv_internal.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace cg {
 
@@ -379,10 +378,6 @@ conv_prog_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 // ---------------------------------------------------------------- launcher
 // All kernel instantiations of one KSTEPS value (4 M-tile counts x 3 statistics widths x single CTA / CTA pair) are
 // compiled in their own translation unit (conv_tc_prog_ks<K>.cu): in one file they took 3.5 minutes of serial nvcc time.
-typedef CUresult (*EncodeTiledFn2)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-CUtensorMapL2promotion tc_l2_promo();  // conv_tc.cu
 // conv_tc_prog.cu: enqueue repack_prog_kernel (generic packed filter -> resident tiles of plan p)
 int repack_prog_launch(const bf16 *wp, bf16 *wb, int Cb, int Cs, int scatter, const ProgPlan &p, cudaStream_t st);
 
@@ -395,7 +390,7 @@ struct ProgLaunchArgs {
   size_t part_bytes;
   double *bn_sums;
   cudaStream_t st;
-  EncodeTiledFn2 enc;
+  EncodeTiledFn enc;
 };
 
 template <int KS_>
@@ -408,7 +403,7 @@ int prog_launch_ks(ProgPlan &p, const ProgLaunchArgs &a) {
   const size_t part_bytes = a.part_bytes;
   double *bn_sums = a.bn_sums;
   cudaStream_t st = a.st;
-  EncodeTiledFn2 enc = a.enc;
+  EncodeTiledFn enc = a.enc;
   auto launch_s = [&](auto ks_tag, auto mt_tag, auto st_tag, auto pair_tag) -> int {
     constexpr int KS = decltype(ks_tag)::value;
     constexpr int MT = decltype(mt_tag)::value;
@@ -432,7 +427,7 @@ int prog_launch_ks(ProgPlan &p, const ProgLaunchArgs &a) {
         const cuuint32_t wbox[2] = {64, (cuuint32_t)(p.btile_bytes >> 8)};
         const cuuint32_t we[2] = {1, 1};
         CUresult rw = enc(&tmw, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wb, wdim, wstr, wbox, we, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_NONE, tc_l2_promo(), CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (rw != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (strided, filters) failed with %d", (int)rw);
       }
       cudaLaunchConfig_t cfg{};

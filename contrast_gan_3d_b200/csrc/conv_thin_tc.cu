@@ -8,16 +8,15 @@
 //  (A) 1 -> 16 channels (fprop of `first`, dgrad of `last_conv`): TOEPLITZ-IN-Z implicit GEMM.
 //      The 1-channel input is a scalar field with z contiguous, so a window of 16 consecutive z values of one (x,y)
 //      line is a 32-byte K-major operand row.  GEMM rows = flattened (x', y') positions of a halo slab (TMA box
-//      8z x Yh x Xh lands as [row][8 z] == the SWIZZLE_NONE core-matrix layout), K = 16 input z, N = 4 output z x 16
-//      channels = 64, and the B operand of tap (dx,dy) is the banded matrix T[zi][(zo,co)] = W[dx,dy,zi-zo,co].
-//      The 49 (dx,dy) taps are pure row shifts of the A descriptor (dx*Yh+dy rows), all 49 Toeplitz tiles (2 KB each)
-//      stay resident in shared memory, and a TMEM lane (= output (x,y)) ends up with 4 z x 16 channels = 128
+//      8z x Yh x Xh lands as [row][8 z] == the SWIZZLE_NONE core-matrix layout), K = 16 input z, N = 8 output z x 16
+//      channels = 128, and the B operand of tap (dx,dy) is the banded matrix T[zi][(zo,co)] = W[dx,dy,zi-zo,co].
+//      The 49 (dx,dy) taps are pure row shifts of the A descriptor (dx*Yh+dy rows), all 49 Toeplitz tiles (4 KB each)
+//      stay resident in shared memory, and a TMEM lane (= output (x,y)) ends up with 8 z x 16 channels = 256
 //      contiguous output bytes.  7 of every 16 K rows are non-zero: useful MMA fraction 44 %, no im2col, no expansion
 //      of the input in HBM.  Zero padding (dgrad) is TMA out-of-bounds fill.
 #include "common.cuh"
 #include "conv_internal.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace cg {
 
@@ -25,8 +24,9 @@ using bf16 = __nv_bfloat16;
 
 constexpr uint32_t kSmemLimitThin = 232448 - 1024;
 constexpr int kTapTilesA = 49;
-constexpr uint32_t kTileBytesA = 2048;  // [2 z-chunks][64 n][8 z] bf16 (4 output z per item); 4096 with 8 output z (N = 128)
-constexpr uint32_t kTileBytesAMax = 4096;
+constexpr int kZbA = 8;                  // output z per work item
+constexpr uint32_t kTileBytesA = 4096;  // [2 z-chunks][128 n = 8 z x 16 ch][8 z] bf16
+constexpr double kHaloWeightA = 0.02;   // weight of the halo overhead (Xh*Yh / Xt*Yt) in the tile score of plan_thin_a
 
 struct ThinAPlan {
   int B, Xi, Yi, Zi;  // 1-channel input
@@ -35,30 +35,26 @@ struct ThinAPlan {
   int Xt, Yt, Xh, Yh, nxt, nyt, nzb;
   int mtiles, rows_alloc, nslots;
   uint32_t slot_bytes, box_bytes, tmem_cols, smem_bytes;
-  int Zc;         // z extent of the two shifted copies: copy[s][row][c] = in[row][c - 8 + zshift[s]]
-  int zshift[2];
-  int debug;
-  int pair;       // CTA pairs (cta_group::2): consecutive work items go to the two CTAs, each holds half of the N rows
-  int zb;         // output z per item: 4 (N = 64) or 8 (N = 128, CTA pairs only: one 65-cycle MMA instead of two 59-cycle ones)
+  int Zc;      // z extent of the shifted copy: copy[row][c] = in[row][c - 8 + zshift]
+  int zshift;  // makes every 8-z window start on a 16-byte boundary of the copy
 };
 
-// PAIR: see conv_tc.cu — the two CTAs of a cluster process consecutive work items in lockstep; each holds the Toeplitz
-// rows of two of the four output z (32 of the 64 N rows), and the rank-0 CTA issues every MMA for both.
-// ZB = 8: an item covers 8 output z, N = 128.  A cta_group::2 MMA costs 59 cycles up to N = 96 and 65 at N = 128
-// (profiles/r01_mma2_microbench.txt), the 14-voxel input window of 8 outputs still fits K = 16, and every window then starts
-// on a 16-byte boundary of ONE shifted copy of the input.  Half the MMAs, half the slab loads, half the items.
-template <int MT, bool STATS, bool PAIR, int ZB = 4>
+// An item covers 8 output z, N = 128.  A cta_group::2 MMA costs 59 cycles up to N = 96 and 65 at N = 128
+// (profiles/r01_mma2_microbench.txt), the 14-voxel input window of 8 outputs still fits K = 16, and every window starts on a
+// 16-byte boundary of ONE shifted copy of the input.
+// CTA pairs (see conv_tc.cu): the two CTAs of a cluster process consecutive work items in lockstep; each holds the Toeplitz
+// rows of four of the eight output z (64 of the 128 N rows), and the rank-0 CTA issues every MMA for both.
+template <int MT, bool STATS>
 __global__ void __launch_bounds__(192, 1)
-conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, const bf16 *__restrict__ wT,
-                   bf16 *__restrict__ out, const __grid_constant__ ThinAPlan p, double *__restrict__ bn_sums) {
+conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, bf16 *__restrict__ out,
+                   const __grid_constant__ ThinAPlan p, double *__restrict__ bn_sums) {
   extern __shared__ __align__(1024) uint8_t smem[];
-  constexpr uint32_t NN = ZB * 16;                       // GEMM N = output z x 16 channels
-  constexpr uint32_t kTileFull = 2 * NN * 16;            // [2 z-chunks][NN n][8 z] bf16
-  constexpr uint32_t kTileB = PAIR ? kTileFull / 2 : kTileFull;
+  constexpr uint32_t NN = kZbA * 16;               // GEMM N = output z x 16 channels
+  constexpr uint32_t kTileB = kTileBytesA / 2;     // this CTA's half of a Toeplitz tile
   // accumulator ring: with one M tile per item an item is only ~2 us of MMAs, so the MMA -> epilogue -> MMA hand-off
   // latency must be hidden behind several buffers (all 512 TMEM columns are used)
   constexpr uint32_t NACC = 512 / (MT * NN);
-  uint8_t *bres = smem;                                    // 49 resident Toeplitz tiles
+  uint8_t *bres = smem;                                    // 49 resident Toeplitz half tiles
   uint8_t *ring = bres + kTapTilesA * kTileB;              // slab slots
   uint8_t *stage = ring + (size_t)p.nslots * p.slot_bytes; // epilogue store staging: 4 warps x 32 rows x 128 B
   uint64_t *bars = reinterpret_cast<uint64_t *>(stage + 16384);
@@ -70,58 +66,46 @@ conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   if (threadIdx.x == 0) {
     tc::mbar_init(b_ready, 1);
     for (int i = 0; i < p.nslots; ++i) { tc::mbar_init(&s_full[i], 1); tc::mbar_init(&s_empty[i], 1); }
-    for (int i = 0; i < (int)NACC; ++i) { tc::mbar_init(&tm_full[i], 1); tc::mbar_init(&tm_empty[i], PAIR ? 8 : 4); }
+    for (int i = 0; i < (int)NACC; ++i) { tc::mbar_init(&tm_full[i], 1); tc::mbar_init(&tm_empty[i], 8); }
     tc::fence_barrier_init();
   }
-  const uint32_t cta_rank = PAIR ? tc::cluster_ctarank() : 0u;
-  if constexpr (PAIR) {
-    __syncthreads();
-    tc::cluster_sync();
-  }
-  if (warp == 5) {
-    if constexpr (PAIR) { tc::tmem_alloc2(tmem_ptr, p.tmem_cols); tc::tmem_relinquish2(); }
-    else { tc::tmem_alloc(tmem_ptr, p.tmem_cols); tc::tmem_relinquish(); }
-  }
+  const uint32_t cta_rank = tc::cluster_ctarank();
+  __syncthreads();
+  tc::cluster_sync();
+  if (warp == 5) { tc::tmem_alloc2(tmem_ptr, p.tmem_cols); tc::tmem_relinquish2(); }
   tc::tc_fence_before();
   __syncthreads();
-  if constexpr (PAIR) tc::cluster_sync();
+  tc::cluster_sync();
   tc::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
 
-  // work items: PAIR -> the pair walks item pairs (2j, 2j+1); an odd total leaves the last odd CTA a dead copy of item 2j
+  // work items: the pair walks item pairs (2j, 2j+1); an odd total leaves the last odd CTA a dead copy of item 2j
   const long long total_items = (long long)p.B * p.nxt * p.nyt * p.nzb;
-  const long long total = PAIR ? (total_items + 1) / 2 : total_items;
-  const int nblk = PAIR ? (int)gridDim.x >> 1 : (int)gridDim.x, blk = PAIR ? (int)blockIdx.x >> 1 : (int)blockIdx.x;
+  const long long total = (total_items + 1) / 2;
+  const int nblk = (int)gridDim.x >> 1, blk = (int)blockIdx.x >> 1;
   const int i_begin = (int)(total * blk / nblk), i_end = (int)(total * (blk + 1) / nblk);
   auto decode = [&](int it, int &b, int &x0, int &xlen, int &y0, int &ylen, int &z0) -> bool {
     bool live = true;
-    if constexpr (PAIR) {
-      it = 2 * it + (int)cta_rank;
-      if (it >= total_items) { it = (int)total_items - 1; live = false; }
-    }
+    it = 2 * it + (int)cta_rank;
+    if (it >= total_items) { it = (int)total_items - 1; live = false; }
     const int zb = it % p.nzb; it /= p.nzb;
     const int yt = it % p.nyt; it /= p.nyt;
     const int xt = it % p.nxt;
     b = it / p.nxt;
     x0 = xt * p.Xt; xlen = min(p.Xt, p.Xo - x0);
     y0 = yt * p.Yt; ylen = min(p.Yt, p.Yo - y0);
-    z0 = zb * ZB;
+    z0 = zb * kZbA;
     return live;
   };
 
   if (warp == 4) {
     if (lane == 0) {
       tc::tma_prefetch_desc(&tmA);
-      if constexpr (PAIR) {  // boxes of 196 rows of 256 bytes (49 KB): this CTA's 49 half tiles, counted on the rank-0 barrier
-        if (cta_rank == 0) tc::mbar_expect_tx(b_ready, 2 * kTapTilesA * kTileB);
-        constexpr int rows_cta = (int)(kTapTilesA * kTileB / 256);
-        for (int r0 = 0; r0 < rows_cta; r0 += 196)
-          tc::tma_load_2d_2cta(bres + (size_t)r0 * 256, &tmW, b_ready, 0, (int)cta_rank * rows_cta + r0);
-      } else {
-        tc::mbar_expect_tx(b_ready, kTapTilesA * kTileFull);
-        for (int t = 0; t < kTapTilesA; ++t)
-          tc::bulk_g2s(bres + (size_t)t * kTileFull, reinterpret_cast<const uint8_t *>(wT) + (size_t)t * kTileFull, kTileFull, b_ready);
-      }
+      // boxes of 196 rows of 256 bytes (49 KB): this CTA's 49 half tiles, counted on the rank-0 barrier
+      if (cta_rank == 0) tc::mbar_expect_tx(b_ready, 2 * kTapTilesA * kTileB);
+      constexpr int rows_cta = (int)(kTapTilesA * kTileB / 256);
+      for (int r0 = 0; r0 < rows_cta; r0 += 196)
+        tc::tma_load_2d_2cta(bres + (size_t)r0 * 256, &tmW, b_ready, 0, (int)cta_rank * rows_cta + r0);
       uint32_t e = 0;
       for (int it = i_begin; it < i_end; ++it, ++e) {
         int b, x0, xlen, y0, ylen, z0;
@@ -129,26 +113,19 @@ conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
         const uint32_t slot = e % p.nslots, use = e / p.nslots;
         if (use > 0) tc::mbar_wait(&s_empty[slot], (use - 1) & 1);
         uint8_t *dst = ring + (size_t)slot * p.slot_bytes;
-        // TMA needs a 16-byte aligned start along z: block parity selects the copy whose z shift makes it so
-        const int cp = ZB == 8 ? 0 : (z0 >> 2) & 1;
-        const int c0 = z0 - p.P - p.zshift[cp] + 8;
-        if constexpr (PAIR) {
-          if (cta_rank == 0) tc::mbar_expect_tx(&s_full[slot], 2 * p.box_bytes);
-          tc::tma_load_5d_2cta(dst, &tmA, &s_full[slot], c0, y0 - p.P, x0 - p.P, b, cp);
-          continue;
-        }
-        if (p.debug & 1) { tc::mbar_arrive(&s_full[slot]); continue; }
-        tc::mbar_expect_tx(&s_full[slot], p.box_bytes);
-        tc::tma_load_5d(dst, &tmA, &s_full[slot], c0, y0 - p.P, x0 - p.P, b, cp);  // rows of 16 z = 32 bytes, SWIZZLE_32B
+        // TMA needs a 16-byte aligned start along z: the z shift of the copy makes it so.  Rows of 16 z = 32 bytes, SWIZZLE_32B
+        const int c0 = z0 - p.P - p.zshift + 8;
+        if (cta_rank == 0) tc::mbar_expect_tx(&s_full[slot], 2 * p.box_bytes);
+        tc::tma_load_5d_2cta(dst, &tmA, &s_full[slot], c0, y0 - p.P, x0 - p.P, b, 0);
       }
     }
   } else if (warp == 5 && cta_rank != 0) {
     // odd CTA of a pair: the rank-0 CTA issues the MMAs for both
   } else if (warp == 5) {
     const bool leader = tc::elect_one();
-    const uint32_t idesc = tc::make_idesc_bf16(PAIR ? 256 : 128, (int)NN, 0, 0);
+    const uint32_t idesc = tc::make_idesc_bf16(256, (int)NN, 0, 0);
     const uint32_t ring_u32 = tc::smem_u32(ring), b_u32 = tc::smem_u32(bres);
-    const uint64_t a_hi = tc::make_desc_sw(0, 256, 32), b_hi = tc::make_desc(0, (PAIR ? NN / 2 : NN) * 16, 128);
+    const uint64_t a_hi = tc::make_desc_sw(0, 256, 32), b_hi = tc::make_desc(0, NN / 2 * 16, 128);
     tc::mbar_wait(b_ready, 0);
     tc::tc_fence_after();
     uint32_t e = 0;
@@ -165,25 +142,19 @@ conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       for (int dx = 0; dx < 7; ++dx) {
         const uint64_t a_dx = a_it + (uint64_t)(2u * (uint32_t)(dx * p.Yh));             // 32-byte rows
         const uint64_t b_dx = b_it + (uint64_t)((uint32_t)(dx * 7) * (kTileB >> 4));
-        if (leader && !(p.debug & 2)) {
+        if (leader) {
 #pragma unroll
           for (int dy = 0; dy < 7; ++dy) {
 #pragma unroll
             for (int mt = 0; mt < MT; ++mt) {
               const uint32_t accum = dy != 0 ? 1u : (uint32_t)(dx != 0);
-              if constexpr (PAIR)
-                tc::umma_bf16_2cta(d_base + mt * NN, a_dx + (uint64_t)(2 * dy + mt * 256), b_dx + (uint64_t)(dy * (kTileB >> 4)), idesc, accum);
-              else
-                tc::umma_bf16(d_base + mt * NN, a_dx + (uint64_t)(2 * dy + mt * 256), b_dx + (uint64_t)(dy * (kTileB >> 4)), idesc, accum);
+              tc::umma_bf16_2cta(d_base + mt * NN, a_dx + (uint64_t)(2 * dy + mt * 256), b_dx + (uint64_t)(dy * (kTileB >> 4)), idesc, accum);
             }
           }
         }
         __syncwarp();
       }
-      if (leader) {
-        if constexpr (PAIR) { tc::umma_commit_2cta(&s_empty[slot], 3); tc::umma_commit_2cta(&tm_full[q], 3); }
-        else { tc::umma_commit(&s_empty[slot]); tc::umma_commit(&tm_full[q]); }
-      }
+      if (leader) { tc::umma_commit_2cta(&s_empty[slot], 3); tc::umma_commit_2cta(&tm_full[q], 3); }
       __syncwarp();
     }
   } else {
@@ -202,11 +173,11 @@ conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       tc::tc_fence_after();
       const uint32_t d_base = tmem_base + ((uint32_t)(warp * 32) << 16) + q * (uint32_t)(MT * NN);
 #pragma unroll
-      for (int mth = 0; mth < MT * (ZB / 4); ++mth) {  // (M tile, group of four output z)
-        const int mt = mth / (ZB / 4), zh = (mth % (ZB / 4)) * 4;
+      for (int mth = 0; mth < MT * 2; ++mth) {  // (M tile, group of four output z)
+        const int mt = mth >> 1, zh = (mth & 1) * 4;
         const int r = mt * 128 + warp * 32 + lane;
         const int xx = r / p.Yh, yy = r - xx * p.Yh;
-        const bool valid = live && xx < xlen && yy < ylen && !(p.debug & 4);
+        const bool valid = live && xx < xlen && yy < ylen;
         const int z0 = z0_item + zh;
         bf16 *dst = out + ((((size_t)b * p.Xo + (x0 + xx)) * p.Yo + (y0 + yy)) * p.Zo + z0) * 16;
         uint32_t v[4][16];  // four output z of this row: all TMEM loads in flight before one wait
@@ -251,10 +222,7 @@ conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
       }
       tc::tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if constexpr (PAIR) tc::mbar_arrive_cluster(&tm_empty[q], 0);
-        else tc::mbar_arrive(&tm_empty[q]);
-      }
+      if (lane == 0) tc::mbar_arrive_cluster(&tm_empty[q], 0);
     }
     if constexpr (STATS) {
 #pragma unroll
@@ -266,34 +234,23 @@ conv7_c1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constan
   }
   tc::tc_fence_before();
   __syncthreads();
-  if constexpr (PAIR) {
-    tc::cluster_sync();
-    if (warp == 5) tc::tmem_dealloc2(tmem_base, p.tmem_cols);
-  } else {
-    if (warp == 5) tc::tmem_dealloc(tmem_base, p.tmem_cols);
-  }
+  tc::cluster_sync();
+  if (warp == 5) tc::tmem_dealloc2(tmem_base, p.tmem_cols);
 }
 
-// Toeplitz tiles: T[(dx,dy)][zi/8][n = zo*16 + co][zi%8] = w(dx,dy,zi-zo,co) for 0 <= zi-zo < 7, else 0.
+// Toeplitz tiles: T[(dx,dy)][zi/8][n = zo*16 + co][zi%8] = w(dx,dy,zi-zo,co) for 0 <= zi-zo < 7, else 0, as the halves
+// held by the two CTAs of a pair: [half][(dx,dy)][zi/8][64 n][8], half = n / 64.
 // wp is the packed filter [tap][Cb][Cs] with Cb*Cs == 16; flip = 1 reverses the taps (transposed convolution).
-// split = 1 (CTA pairs): [half][(dx,dy)][zi/8][32 n][8], half = n / 32.
-// NN = 64 or 128 N rows (4 or 8 output z).
-__global__ void toeplitz_a_kernel(const bf16 *__restrict__ wp, bf16 *__restrict__ wt, int flip, int split, int NN) {
-  const int total = kTapTilesA * 2 * NN * 8, Nh = NN >> 1;
+__global__ void toeplitz_a_kernel(const bf16 *__restrict__ wp, bf16 *__restrict__ wt, int flip) {
+  constexpr int NN = kZbA * 16, Nh = NN >> 1;
+  const int total = kTapTilesA * 2 * NN * 8;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int z8 = i & 7;
     int t = i >> 3;
-    int n, chunk, tile;
-    if (split) {
-      const int nl = t % Nh; t /= Nh;
-      chunk = t & 1; t >>= 1;
-      tile = t % kTapTilesA;
-      n = (t / kTapTilesA) * Nh + nl;
-    } else {
-      n = t % NN; t /= NN;
-      chunk = t & 1;
-      tile = t >> 1;
-    }
+    const int nl = t % Nh; t /= Nh;
+    const int chunk = t & 1; t >>= 1;
+    const int tile = t % kTapTilesA;
+    const int n = (t / kTapTilesA) * Nh + nl;
     const int zi = chunk * 8 + z8, zo = n >> 4, co = n & 15, dz = zi - zo;
     bf16 v = __float2bfloat16_rn(0.f);
     if (dz >= 0 && dz < 7) {
@@ -305,12 +262,12 @@ __global__ void toeplitz_a_kernel(const bf16 *__restrict__ wp, bf16 *__restrict_
 }
 
 // TMA needs 16-byte aligned row pitches AND a 16-byte aligned start coordinate along the contiguous axis, but the z
-// windows start every 4 voxels.  Two z-shifted, zero-margined copies of the 1-channel input make every window start
-// aligned in one of them:  copy[s][row][c] = in[row][c - 8 + shift_s]  (0 outside), c in [0, Zc), Zc % 8 == 0.
+// windows start at z0 - P.  A z-shifted, zero-margined copy of the 1-channel input makes every window start aligned:
+// copy[row][c] = in[row][c - 8 + s]  (0 outside), c in [0, Zc), Zc % 8 == 0.
 // One WARP per input line (8 lines per block): the line is staged in shared memory (with zero margins) and written out as
 // 16-byte chunks.
 __global__ void __launch_bounds__(256)
-shifted_copies_kernel(const bf16 *__restrict__ in, bf16 *__restrict__ out, long long rows, int Z, int Zc, int s0, int s1, int ncopies) {
+shifted_copies_kernel(const bf16 *__restrict__ in, bf16 *__restrict__ out, long long rows, int Z, int Zc, int s) {
   extern __shared__ uint16_t lines[];  // per warp: line[8 + z] = in[z], zeros in [0, 8) and beyond Z
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n = (Zc + 24 + 7) & ~7;
@@ -323,14 +280,12 @@ shifted_copies_kernel(const bf16 *__restrict__ in, bf16 *__restrict__ out, long 
     line[i] = (z >= 0 && z < Z) ? src[z] : (uint16_t)0;
   }
   __syncwarp();
-  const int chunks = Zc >> 3;
-  for (int i = lane; i < ncopies * chunks; i += 32) {
-    const int cp = i >= chunks, j = i - cp * chunks;
-    const int base = j * 8 + (cp ? s1 : s0);  // out[c] = in[c - 8 + s] = line[c + s]
+  for (int j = lane; j < (Zc >> 3); j += 32) {
+    const int base = j * 8 + s;  // out[c] = in[c - 8 + s] = line[c + s]
     uint32_t w[4];
 #pragma unroll
     for (int k = 0; k < 4; ++k) w[k] = (uint32_t)line[base + 2 * k] | ((uint32_t)line[base + 2 * k + 1] << 16);
-    reinterpret_cast<uint4 *>(out + ((long long)cp * rows + r) * Zc)[j] = make_uint4(w[0], w[1], w[2], w[3]);
+    reinterpret_cast<uint4 *>(out + r * Zc)[j] = make_uint4(w[0], w[1], w[2], w[3]);
   }
 }
 
@@ -355,7 +310,6 @@ struct ThinBPlan {
   int Zt, nzt, Zh, Yt, nyt, Yh;
   int mtiles, rows_alloc, nslots;
   uint32_t slot_bytes, box_bytes, tmem_cols, smem_bytes;
-  int debug;  // CGAN3D_THIN_DEBUG (profiling aid): 1 = skip the MMAs, 2 = skip the epilogue math
 };
 
 struct SegIter {
@@ -379,10 +333,12 @@ struct SegIter {
   }
 };
 
-template <int MT, bool PAIR>
+// CTA pairs: the two CTAs of a cluster walk column pairs in lockstep, each holds 32 of the 64 N rows of every filter tile,
+// and the rank-0 CTA issues every MMA for both.
+template <int MT>
 __global__ void __launch_bounds__(320, 1)
-conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, const bf16 *__restrict__ wT,
-                    bf16 *__restrict__ out, const __grid_constant__ ThinBPlan p) {
+conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW, bf16 *__restrict__ out,
+                    const __grid_constant__ ThinBPlan p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t *bres = smem;                                                   // 7 resident filter tiles (14 KB)
   uint8_t *ring = smem + 14336;                                            // slab slots (multiple of 256 B)
@@ -395,31 +351,24 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   if (threadIdx.x == 0) {
     tc::mbar_init(b_ready, 1);
     for (int i = 0; i < p.nslots; ++i) { tc::mbar_init(&s_full[i], 1); tc::mbar_init(&s_empty[i], 1); }
-    for (int i = 0; i < 2; ++i) { tc::mbar_init(&tm_full[i], 1); tc::mbar_init(&tm_empty[i], PAIR ? 16 : 8); }
+    for (int i = 0; i < 2; ++i) { tc::mbar_init(&tm_full[i], 1); tc::mbar_init(&tm_empty[i], 16); }
     tc::fence_barrier_init();
   }
-  constexpr uint32_t kTileB = PAIR ? kTileBytesB / 2 : kTileBytesB;  // a CTA of a pair holds 32 of the 64 N rows of a tile
-  const uint32_t cta_rank = PAIR ? tc::cluster_ctarank() : 0u;
-  if constexpr (PAIR) {
-    __syncthreads();
-    tc::cluster_sync();
-  }
-  if (warp == 9) {
-    if constexpr (PAIR) { tc::tmem_alloc2(tmem_ptr, p.tmem_cols); tc::tmem_relinquish2(); }
-    else { tc::tmem_alloc(tmem_ptr, p.tmem_cols); tc::tmem_relinquish(); }
-  }
+  constexpr uint32_t kTileB = kTileBytesB / 2;  // this CTA's 32 of the 64 N rows of a tile
+  const uint32_t cta_rank = tc::cluster_ctarank();
+  __syncthreads();
+  tc::cluster_sync();
+  if (warp == 9) { tc::tmem_alloc2(tmem_ptr, p.tmem_cols); tc::tmem_relinquish2(); }
   tc::tc_fence_before();
   __syncthreads();
-  if constexpr (PAIR) tc::cluster_sync();
+  tc::cluster_sync();
   tc::tc_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   const long long ncols = (long long)p.B * p.nyt * p.nzt;
   auto decode = [&](int col, int &b, int &y0, int &ylen, int &z0, int &zlen) -> bool {
     bool live = true;
-    if constexpr (PAIR) {
-      col = 2 * col + (int)cta_rank;
-      if (col >= ncols) { col = (int)ncols - 1; live = false; }
-    }
+    col = 2 * col + (int)cta_rank;
+    if (col >= ncols) { col = (int)ncols - 1; live = false; }
     const int zt = col % p.nzt; col /= p.nzt;
     const int yt = col % p.nyt;
     b = col / p.nyt;
@@ -431,29 +380,19 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
   if (warp == 8) {
     if (lane == 0) {
       tc::tma_prefetch_desc(&tmA);
-      if constexpr (PAIR) {
-        // SWIZZLE_32B repeats every 256 bytes, so rows 32r..32r+31 of a tile are simply its r-th kilobyte (4 map rows)
-        if (cta_rank == 0) tc::mbar_expect_tx(b_ready, 2 * kTapTilesB * kTileB);
-        for (int t = 0; t < kTapTilesB; ++t) tc::tma_load_2d_2cta(bres + (size_t)t * kTileB, &tmW, b_ready, 0, t * 8 + (int)cta_rank * 4);
-      } else {
-        tc::mbar_expect_tx(b_ready, kTapTilesB * kTileBytesB);
-        tc::bulk_g2s(bres, wT, kTapTilesB * kTileBytesB, b_ready);
-      }
+      // SWIZZLE_32B repeats every 256 bytes, so rows 32r..32r+31 of a tile are simply its r-th kilobyte (4 map rows)
+      if (cta_rank == 0) tc::mbar_expect_tx(b_ready, 2 * kTapTilesB * kTileB);
+      for (int t = 0; t < kTapTilesB; ++t) tc::tma_load_2d_2cta(bres + (size_t)t * kTileB, &tmW, b_ready, 0, t * 8 + (int)cta_rank * 4);
       uint32_t e = 0;
       int col, x0, xlen;
-      for (SegIter it(ncols, p.Xo, PAIR); it.next(col, x0, xlen);) {
+      for (SegIter it(ncols, p.Xo, true); it.next(col, x0, xlen);) {
         int b, y0, ylen, z0, zlen;
         decode(col, b, y0, ylen, z0, zlen);
         for (int i = 0; i < xlen + 6; ++i, ++e) {
           const uint32_t slot = e % p.nslots, use = e / p.nslots;
           if (use > 0) tc::mbar_wait(&s_empty[slot], (use - 1) & 1);
-          if constexpr (PAIR) {
-            if (cta_rank == 0) tc::mbar_expect_tx(&s_full[slot], 2 * p.box_bytes);
-            tc::tma_load_5d_2cta(ring + (size_t)slot * p.slot_bytes, &tmA, &s_full[slot], 0, z0 - p.P, y0 - p.P, x0 - p.P + i, b);
-            continue;
-          }
-          tc::mbar_expect_tx(&s_full[slot], p.box_bytes);
-          tc::tma_load_5d(ring + (size_t)slot * p.slot_bytes, &tmA, &s_full[slot], 0, z0 - p.P, y0 - p.P, x0 - p.P + i, b);
+          if (cta_rank == 0) tc::mbar_expect_tx(&s_full[slot], 2 * p.box_bytes);
+          tc::tma_load_5d_2cta(ring + (size_t)slot * p.slot_bytes, &tmA, &s_full[slot], 0, z0 - p.P, y0 - p.P, x0 - p.P + i, b);
         }
       }
     }
@@ -461,14 +400,14 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     // odd CTA of a pair: the rank-0 CTA issues the MMAs of both
   } else if (warp == 9) {
     const bool leader = tc::elect_one();
-    const uint32_t idesc = tc::make_idesc_bf16(PAIR ? 256 : 128, 64, 0, 0);
+    const uint32_t idesc = tc::make_idesc_bf16(256, 64, 0, 0);
     const uint32_t ring_u32 = tc::smem_u32(ring), b_u32 = tc::smem_u32(bres);
     const uint64_t a_hi = tc::make_desc_sw(0, 256, 32), b_hi = tc::make_desc_sw(0, 256, 32);
     tc::mbar_wait(b_ready, 0);
     tc::tc_fence_after();
     uint32_t e = 0;
     int col, x0, xlen;
-    for (SegIter it(ncols, p.Xo, PAIR); it.next(col, x0, xlen);) {
+    for (SegIter it(ncols, p.Xo, true); it.next(col, x0, xlen);) {
       for (int i = 0; i < xlen + 6; ++i, ++e) {
         const uint32_t q = e & 1, uq = e >> 1, slot = e % p.nslots;
         if (uq > 0) tc::mbar_wait(&tm_empty[q], (uq - 1) & 1);
@@ -479,17 +418,14 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         if (leader) {
 #pragma unroll
           for (int dy = 0; dy < 7; ++dy) {
-            if (p.debug & 1) continue;
             const uint64_t a0 = a_hi | (uint64_t)((a_slot + 2u * (uint32_t)(dy * kPitchB)) & 0x3FFF);  // 32-byte rows
             const uint64_t b0 = b_hi | (uint64_t)(((b_u32 + (uint32_t)dy * kTileB) >> 4) & 0x3FFF);
 #pragma unroll
-            for (int mt = 0; mt < MT; ++mt) {
-              if constexpr (PAIR) tc::umma_bf16_2cta(d_base + mt * 64, a0 + (uint64_t)(mt * 256), b0, idesc, (uint32_t)(dy != 0));
-              else tc::umma_bf16(d_base + mt * 64, a0 + (uint64_t)(mt * 256), b0, idesc, (uint32_t)(dy != 0));
-            }
+            for (int mt = 0; mt < MT; ++mt)
+              tc::umma_bf16_2cta(d_base + mt * 64, a0 + (uint64_t)(mt * 256), b0, idesc, (uint32_t)(dy != 0));
           }
-          if constexpr (PAIR) { tc::umma_commit_2cta(&s_empty[slot], 3); tc::umma_commit_2cta(&tm_full[q], 3); }
-          else { tc::umma_commit(&s_empty[slot]); tc::umma_commit(&tm_full[q]); }
+          tc::umma_commit_2cta(&s_empty[slot], 3);
+          tc::umma_commit_2cta(&tm_full[q], 3);
         }
         __syncwarp();
       }
@@ -501,7 +437,7 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const int qd = warp & 3, grp = warp >> 2;
     uint32_t e = 0;
     int col, x0, xlen;
-    for (SegIter it(ncols, p.Xo, PAIR); it.next(col, x0, xlen);) {
+    for (SegIter it(ncols, p.Xo, true); it.next(col, x0, xlen);) {
       int b, y0, ylen, z0, zlen;
       const bool live = decode(col, b, y0, ylen, z0, zlen);
       float win[NK][7];
@@ -525,7 +461,7 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
         for (int k = 0; k < NK; ++k) {
           const int mt = 2 * k + grp;
-          if (mt >= MT || (p.debug & 2)) continue;
+          if (mt >= MT) continue;
           uint32_t v[7][8];
 #pragma unroll
           for (int dx = 0; dx < 7; ++dx) tc::tmem_ld8(d_base + (uint32_t)(mt * 64 + dx * 8), v[dx]);
@@ -549,21 +485,14 @@ conv7_to1_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         }
         tc::tc_fence_before();
         __syncwarp();
-        if (lane == 0) {
-          if constexpr (PAIR) tc::mbar_arrive_cluster(&tm_empty[q], 0);
-          else tc::mbar_arrive(&tm_empty[q]);
-        }
+        if (lane == 0) tc::mbar_arrive_cluster(&tm_empty[q], 0);
       }
     }
   }
   tc::tc_fence_before();
   __syncthreads();
-  if constexpr (PAIR) {
-    tc::cluster_sync();
-    if (warp == 9) tc::tmem_dealloc2(tmem_base, p.tmem_cols);
-  } else {
-    if (warp == 9) tc::tmem_dealloc(tmem_base, p.tmem_cols);
-  }
+  tc::cluster_sync();
+  if (warp == 9) tc::tmem_dealloc2(tmem_base, p.tmem_cols);
 }
 
 // T[dy][n = dx*8 + dz][ci] = w(dx,dy,dz,ci) for dx, dz < 7, else 0 (same flip convention as toeplitz_a_kernel), stored as
@@ -800,20 +729,13 @@ expand_z_kernel(const bf16 *__restrict__ q, bf16 *__restrict__ e, long long line
 }
 
 // ---------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFnT)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-void *tc_encode_fn_ptr();  // conv_tc.cu
-CUtensorMapL2promotion tc_l2_promo();  // conv_tc.cu
-
 static int encode_map(CUtensorMap *tm, const void *ptr, int rank, const cuuint64_t *gdim, const cuuint64_t *gstr,
                       const cuuint32_t *box, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_NONE) {
-  EncodeTiledFnT enc = reinterpret_cast<EncodeTiledFnT>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, tc_l2_promo(),
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (thin conv) failed with %d", (int)r);
   return 0;
 }
@@ -821,11 +743,11 @@ static int encode_map(CUtensorMap *tm, const void *ptr, int rank, const cuuint64
 // un-swizzled map of an arbitrary element type (weight tiles viewed as rows of 256 bytes)
 static int encode_map_raw(CUtensorMap *tm, const void *ptr, CUtensorMapDataType dt, int rank, const cuuint64_t *gdim, const cuuint64_t *gstr,
                           const cuuint32_t *box) {
-  EncodeTiledFnT enc = reinterpret_cast<EncodeTiledFnT>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
   CUresult r = enc(tm, dt, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_NONE, tc_l2_promo(), CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (weight tiles) failed with %d", (int)r);
   return 0;
 }
@@ -846,20 +768,11 @@ static bool plan_thin_a(const cgan3d_conv_geom &g, int op, ThinAPlan &best) {
   p.B = g.B;
   if (op == 0) { p.Xi = g.Xb; p.Yi = g.Yb; p.Zi = g.Zb; p.Xo = g.Xs; p.Yo = g.Ys; p.Zo = g.Zs; p.P = g.pad; }
   else         { p.Xi = g.Xs; p.Yi = g.Ys; p.Zi = g.Zs; p.Xo = g.Xb; p.Yo = g.Yb; p.Zo = g.Zb; p.P = 6 - g.pad; }
-  p.zshift[0] = ((0 - p.P) % 8 + 8) % 8;
-  p.zshift[1] = ((4 - p.P) % 8 + 8) % 8;
+  p.zshift = ((0 - p.P) % 8 + 8) % 8;
   p.Zc = round_up(p.Zi + 16, 8);
-  {
-    static int off = -1, zb4 = -1;
-    if (off < 0) off = getenv("CGAN3D_NO_PAIR") ? 1 : 0;
-    if (zb4 < 0) zb4 = getenv("CGAN3D_THIN_ZB4") ? 1 : 0;  // A/B timing: four output z per item (N = 64)
-    p.pair = off ? 0 : 1;
-    p.zb = (p.pair && !zb4) ? 8 : 4;
-  }
-  p.nzb = (p.Zo + p.zb - 1) / p.zb;
-  const uint32_t tile_full = p.zb == 8 ? kTileBytesAMax : kTileBytesA;
-  const int max_mt = p.zb == 8 ? 2 : 4;  // the accumulator ring needs at least two buffers of mtiles * N columns
-  const uint32_t fixed = kTapTilesA * tile_full / (p.pair ? 2 : 1) + 16384 + 512;  // Toeplitz tiles, store staging, barriers
+  p.nzb = (p.Zo + kZbA - 1) / kZbA;
+  const int max_mt = 2;  // the accumulator ring needs at least two buffers of mtiles * N columns
+  const uint32_t fixed = kTapTilesA * kTileBytesA / 2 + 16384 + 512;  // this CTA's Toeplitz half tiles, store staging, barriers
   double best_score = 0;
   bool found = false;
   for (int nyt = 1; nyt <= p.Yo; ++nyt) {
@@ -877,9 +790,7 @@ static bool plan_thin_a(const cgan3d_conv_geom &g, int op, ThinAPlan &best) {
       const int nxt = (p.Xo + Xt - 1) / Xt;
       const double eff = (double)p.Xo * p.Yo / ((double)nxt * nyt * mt * 128);
       const double halo = (double)(Xh * Yh) / (Xt * Yt);
-      static double halo_w = -1;
-      if (halo_w < 0) { const char *e = getenv("CGAN3D_THIN_HALO_W"); halo_w = e ? atof(e) : 0.02; }
-      const double score = eff / (1.0 + halo_w * halo) * (nslots >= 3 ? 1.0 : 0.8);
+      const double score = eff / (1.0 + kHaloWeightA * halo) * (nslots >= 3 ? 1.0 : 0.8);
       if (score > best_score + 1e-9) {
         best_score = score; found = true;
         best = p;
@@ -891,14 +802,13 @@ static bool plan_thin_a(const cgan3d_conv_geom &g, int op, ThinAPlan &best) {
   }
   if (!found) return false;
   best.box_bytes = 32u * best.Yh * best.Xh;
-  best.tmem_cols = 512;  // a ring of 512 / (mtiles * 64) accumulator buffers
+  best.tmem_cols = 512;  // a ring of 512 / (mtiles * 128) accumulator buffers
   best.smem_bytes = fixed + best.nslots * best.slot_bytes;
   return true;
 }
 
 static bool plan_thin_c(const cgan3d_conv_geom &g, ThinCPlan &p);
 static size_t thin_c_workspace(const ThinCPlan &p);
-bool thin_w2_supported(const cgan3d_conv_geom &g);  // wgrad7_v2.cu
 
 // op 0: gather with Cb == 16, Cs == 1;  op 1: scatter with Cb == 1, Cs == 16
 static bool thin_b_shape(const cgan3d_conv_geom &g, int op) {
@@ -947,12 +857,13 @@ bool thin_supported(const cgan3d_conv_geom &g, int dtype, int op) {
   return false;
 }
 
+// room for two shifted copies of the input (the workspace size callers allocate); the 8-z items read only the first
 static size_t thin_a_repitch_bytes(const ThinAPlan &p) { return (size_t)2 * p.B * p.Xi * p.Yi * p.Zc * 2; }
 
 size_t thin_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
   if (dtype != CGAN3D_BF16) return 0;
   ThinAPlan p;
-  if ((op == 0 || op == 1) && plan_thin_a(g, op, p)) return (size_t)kTapTilesA * kTileBytesAMax + 256 + thin_a_repitch_bytes(p) + 256;
+  if ((op == 0 || op == 1) && plan_thin_a(g, op, p)) return (size_t)kTapTilesA * kTileBytesA + 256 + thin_a_repitch_bytes(p) + 256;
   ThinBPlan pb;
   if ((op == 0 || op == 1) && plan_thin_b(g, op, pb)) return (size_t)kTapTilesB * kTileBytesB + 256;
   ThinCPlan pc;
@@ -965,20 +876,17 @@ static int run_thin_a(const cgan3d_conv_geom &g, int op, const void *in, const v
                       cudaStream_t st, double *bn_sums) {
   ThinAPlan p;
   if (!plan_thin_a(g, op, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: shape not supported");
-  if (const char *dbg = getenv("CGAN3D_THIN_DEBUG")) p.debug = atoi(dbg);
   const size_t need = thin_workspace_bytes(g, CGAN3D_BF16, op);
   if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 thin conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 15) || (reinterpret_cast<uintptr_t>(ws) & 255))
     return fail(CGAN3D_E_ARG, "tcgen05 thin conv: pointers must be 16-byte aligned (workspace 256)");
   bf16 *wt = reinterpret_cast<bf16 *>(ws);
-  const uint32_t tile_full = p.zb == 8 ? kTileBytesAMax : kTileBytesA;
-  toeplitz_a_kernel<<<49, 256, 0, st>>>(reinterpret_cast<const bf16 *>(wp), wt, op, p.pair, p.zb * 16);
+  toeplitz_a_kernel<<<49, 256, 0, st>>>(reinterpret_cast<const bf16 *>(wp), wt, op);
   CG_LAUNCH_CHECK("toeplitz_a");
-  bf16 *rp = reinterpret_cast<bf16 *>(reinterpret_cast<uint8_t *>(ws) + (size_t)kTapTilesA * kTileBytesAMax + 256);
+  bf16 *rp = reinterpret_cast<bf16 *>(reinterpret_cast<uint8_t *>(ws) + (size_t)kTapTilesA * kTileBytesA + 256);
   const long long rows = (long long)p.B * p.Xi * p.Yi;
-  // 8 output z per item: every window starts on a 16-byte boundary of copy 0, the second copy is not needed
   shifted_copies_kernel<<<(unsigned)((rows + 7) / 8), 256, (size_t)8 * ((p.Zc + 24 + 7) & ~7) * 2, st>>>(
-      reinterpret_cast<const bf16 *>(in), rp, rows, p.Zi, p.Zc, p.zshift[0], p.zshift[1], p.zb == 8 ? 1 : 2);
+      reinterpret_cast<const bf16 *>(in), rp, rows, p.Zi, p.Zc, p.zshift);
   CG_LAUNCH_CHECK("shifted_copies");
   CUtensorMap tm;
   const cuuint64_t zc = (cuuint64_t)p.Zc;
@@ -987,50 +895,21 @@ static int run_thin_a(const cgan3d_conv_geom &g, int op, const void *in, const v
   const cuuint32_t box[5] = {16, (cuuint32_t)p.Yh, (cuuint32_t)p.Xh, 1, 1};
   int r = encode_map(&tm, rp, 5, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_32B);
   if (r) return r;
-  CUtensorMap tmw{};
-  if (p.pair) {  // the Toeplitz tiles as rows of 256 bytes: 196 rows per CTA half
-    const cuuint64_t wdim[2] = {64, (cuuint64_t)(kTapTilesA * tile_full / 256)};
-    const cuuint64_t wstr[1] = {256};
-    const cuuint32_t wbox[2] = {64, 196};  // 49 KB per box: one per CTA at N = 64, two at N = 128
-    r = encode_map_raw(&tmw, wt, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wdim, wstr, wbox);
-    if (r) return r;
-  }
+  CUtensorMap tmw;  // the Toeplitz tiles as rows of 256 bytes: 392 rows per CTA half, loaded as two boxes of 49 KB
+  const cuuint64_t wdim[2] = {64, (cuuint64_t)(kTapTilesA * kTileBytesA / 256)};
+  const cuuint64_t wstr[1] = {256};
+  const cuuint32_t wbox[2] = {64, 196};
+  r = encode_map_raw(&tmw, wt, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wdim, wstr, wbox);
+  if (r) return r;
   const long long total = (long long)p.B * p.nxt * p.nyt * p.nzb;
-  const int grid = p.pair ? 2 * (int)mn<long long>((total + 1) / 2, (long long)(num_sms() / 2)) : (int)mn<long long>(total, (long long)num_sms());
-  auto launch_s = [&](auto mt_tag, auto st_tag, auto pair_tag) -> int {
+  const int grid = 2 * (int)mn<long long>((total + 1) / 2, (long long)(num_sms() / 2));
+  auto launch = [&](auto mt_tag, auto st_tag) -> int {
     constexpr int MT = decltype(mt_tag)::value;
     constexpr bool ST = decltype(st_tag)::value;
-    constexpr bool PR = decltype(pair_tag)::value;
     static bool attr_set = false;
     if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv7_c1_tc_kernel<MT, ST, PR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
+      cudaError_t e = cudaFuncSetAttribute(conv7_c1_tc_kernel<MT, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
       if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv7_c1_tc_kernel)");
-      attr_set = true;
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(192);
-    cfg.dynamicSmemBytes = p.smem_bytes + 1024;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = PR ? 2 : 1;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_c1_tc_kernel<MT, ST, PR>, tm, tmw, (const bf16 *)wt, reinterpret_cast<bf16 *>(outp), p, bn_sums);
-    if (e != cudaSuccess) return cuda_fail(e, "conv7_c1_tc_kernel launch");
-    CG_LAUNCH_CHECK("conv7_c1_tc_kernel");
-    return 0;
-  };
-  auto launch_z8 = [&](auto mt_tag, auto st_tag) -> int {  // CTA pairs, 8 output z per item
-    constexpr int MT = decltype(mt_tag)::value;
-    constexpr bool ST = decltype(st_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv7_c1_tc_kernel<MT, ST, true, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv7_c1_tc_kernel, 8 z)");
       attr_set = true;
     }
     cudaLaunchConfig_t cfg{};
@@ -1045,37 +924,20 @@ static int run_thin_a(const cgan3d_conv_geom &g, int op, const void *in, const v
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_c1_tc_kernel<MT, ST, true, 8>, tm, tmw, (const bf16 *)wt, reinterpret_cast<bf16 *>(outp), p, bn_sums);
-    if (e != cudaSuccess) return cuda_fail(e, "conv7_c1_tc_kernel (8 z) launch");
+    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_c1_tc_kernel<MT, ST>, tm, tmw, reinterpret_cast<bf16 *>(outp), p, bn_sums);
+    if (e != cudaSuccess) return cuda_fail(e, "conv7_c1_tc_kernel launch");
     CG_LAUNCH_CHECK("conv7_c1_tc_kernel");
     return 0;
   };
-  if (p.zb == 8) {
-    if (p.mtiles == 1) return bn_sums ? launch_z8(std::integral_constant<int, 1>{}, std::true_type{}) : launch_z8(std::integral_constant<int, 1>{}, std::false_type{});
-    if (p.mtiles == 2) return bn_sums ? launch_z8(std::integral_constant<int, 2>{}, std::true_type{}) : launch_z8(std::integral_constant<int, 2>{}, std::false_type{});
-    return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv (8 z): mtiles %d not built", p.mtiles);
-  }
-  auto launch = [&](auto mt_tag) -> int {
-    if (p.pair) return bn_sums ? launch_s(mt_tag, std::true_type{}, std::true_type{}) : launch_s(mt_tag, std::false_type{}, std::true_type{});
-    return bn_sums ? launch_s(mt_tag, std::true_type{}, std::false_type{}) : launch_s(mt_tag, std::false_type{}, std::false_type{});
-  };
-  switch (p.mtiles) {
-    case 1: return launch(std::integral_constant<int, 1>{});
-    case 2: return launch(std::integral_constant<int, 2>{});
-    case 3: return launch(std::integral_constant<int, 3>{});
-    case 4: return launch(std::integral_constant<int, 4>{});
-    default: return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: mtiles %d not built", p.mtiles);
-  }
+  if (p.mtiles == 1) return bn_sums ? launch(std::integral_constant<int, 1>{}, std::true_type{}) : launch(std::integral_constant<int, 1>{}, std::false_type{});
+  if (p.mtiles == 2) return bn_sums ? launch(std::integral_constant<int, 2>{}, std::true_type{}) : launch(std::integral_constant<int, 2>{}, std::false_type{});
+  return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: mtiles %d not built", p.mtiles);
 }
 
 static int run_thin_b(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
                       cudaStream_t st) {
   ThinBPlan p;
   if (!plan_thin_b(g, op, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv (16->1): shape not supported");
-  if (const char *dbg = getenv("CGAN3D_THIN_DEBUG")) p.debug = atoi(dbg);
-  if (getenv("CGAN3D_THIN_VERBOSE"))
-    fprintf(stderr, "thinB plan: Zt %d nzt %d Yt %d nyt %d mt %d rows_alloc %d nslots %d smem %u\n", p.Zt, p.nzt, p.Yt, p.nyt, p.mtiles,
-            p.rows_alloc, p.nslots, p.smem_bytes);
   const size_t need = (size_t)kTapTilesB * kTileBytesB;
   if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 thin conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
@@ -1089,26 +951,20 @@ static int run_thin_b(const cgan3d_conv_geom &g, int op, const void *in, const v
   const cuuint32_t box[5] = {16, (cuuint32_t)p.Zh, (cuuint32_t)p.Yh, 1, 1};
   int r = encode_map(&tm, in, 5, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_32B);
   if (r) return r;
-  static int pair_off = -1;
-  if (pair_off < 0) pair_off = getenv("CGAN3D_NO_PAIR") ? 1 : 0;
-  const bool pair = !pair_off;
-  CUtensorMap tmw{};
-  if (pair) {  // the 7 filter tiles as rows of 256 bytes (8 rows per tile, 4 per CTA half)
-    const cuuint64_t wdim[2] = {64, (cuuint64_t)(kTapTilesB * kTileBytesB / 256)};
-    const cuuint64_t wstr[1] = {256};
-    const cuuint32_t wbox[2] = {64, 4};
-    r = encode_map_raw(&tmw, wt, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wdim, wstr, wbox);
-    if (r) return r;
-  }
+  CUtensorMap tmw;  // the 7 filter tiles as rows of 256 bytes (8 rows per tile, 4 per CTA half)
+  const cuuint64_t wdim[2] = {64, (cuuint64_t)(kTapTilesB * kTileBytesB / 256)};
+  const cuuint64_t wstr[1] = {256};
+  const cuuint32_t wbox[2] = {64, 4};
+  r = encode_map_raw(&tmw, wt, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wdim, wstr, wbox);
+  if (r) return r;
   const long long ncols = (long long)p.B * p.nyt * p.nzt;
-  const long long total = (pair ? (ncols + 1) / 2 : ncols) * p.Xo;
-  const int grid = pair ? 2 * (int)mn<long long>(total, (long long)(num_sms() / 2)) : (int)mn<long long>(total, (long long)num_sms());
-  auto launch_p = [&](auto mt_tag, auto pair_tag) -> int {
+  const long long total = (ncols + 1) / 2 * p.Xo;
+  const int grid = 2 * (int)mn<long long>(total, (long long)(num_sms() / 2));
+  auto launch = [&](auto mt_tag) -> int {
     constexpr int MT = decltype(mt_tag)::value;
-    constexpr bool PR = decltype(pair_tag)::value;
     static bool attr_set = false;
     if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv7_to1_tc_kernel<MT, PR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
+      cudaError_t e = cudaFuncSetAttribute(conv7_to1_tc_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
       if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv7_to1_tc_kernel)");
       attr_set = true;
     }
@@ -1119,18 +975,15 @@ static int run_thin_b(const cgan3d_conv_geom &g, int op, const void *in, const v
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = PR ? 2 : 1;
+    attr[0].val.clusterDim.x = 2;
     attr[0].val.clusterDim.y = 1;
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_to1_tc_kernel<MT, PR>, tm, tmw, (const bf16 *)wt, reinterpret_cast<bf16 *>(outp), p);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_to1_tc_kernel<MT>, tm, tmw, reinterpret_cast<bf16 *>(outp), p);
     if (e != cudaSuccess) return cuda_fail(e, "conv7_to1_tc_kernel launch");
     CG_LAUNCH_CHECK("conv7_to1_tc_kernel");
     return 0;
-  };
-  auto launch = [&](auto mt_tag) -> int {
-    return pair ? launch_p(mt_tag, std::true_type{}) : launch_p(mt_tag, std::false_type{});
   };
   switch (p.mtiles) {
     case 1: return launch(std::integral_constant<int, 1>{});
@@ -1172,10 +1025,6 @@ static bool plan_thin_c(const cgan3d_conv_geom &g, ThinCPlan &p) {
 }
 
 static size_t thin_c_workspace(const ThinCPlan &p) { return (size_t)p.B * p.Xe * p.Ye * p.Zs * 16 + 256; }
-
-// wgrad7_v2.cu: the z-expansion is built in shared memory (no workspace), M = 128 x N = 128 MMAs
-bool thin_w2_supported(const cgan3d_conv_geom &g);
-int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
 
 int thin_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
                    cudaStream_t st) {

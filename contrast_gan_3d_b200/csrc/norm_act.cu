@@ -4,8 +4,6 @@
 // (reference model/blocks.py:45,50,52-53,87-88; generator.py:85; trainer/Trainer.py:171).
 #include <type_traits>
 
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace cg {
@@ -262,8 +260,7 @@ static ColGrid col_grid8(int64_t n_rows, int C, int ns) {
   g.rows_per_block = 0;  // rows are walked grid-strided
   // two blocks per SM = one resident wave (measured at 16x128^3x16 / 16x64^3x32 / 16x32^3x64 bf16: 2 -> 90 / 81 / 56 % of the HBM
   // peak, 4 -> 89 / 75 / 52 %, 8 -> 87 / 71 / 39 %; eight row pairs in flight per thread instead of four: slower)
-  static int per_sm = getenv("CGAN3D_RED_BLOCKS") ? atoi(getenv("CGAN3D_RED_BLOCKS")) : 2;
-  g.blocks = (int)mx<int64_t>(1, mn<int64_t>((n_rows + lanes - 1) / lanes, (int64_t)num_sms() * per_sm));
+  g.blocks = (int)mx<int64_t>(1, mn<int64_t>((n_rows + lanes - 1) / lanes, (int64_t)num_sms() * 2));
   g.smem = (size_t)ns * lanes * C * sizeof(double);
   return g;
 }

@@ -27,21 +27,20 @@
 #include "common.cuh"
 #include "conv_internal.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace cg {
 
 using bf16 = __nv_bfloat16;
 constexpr uint32_t kSmemLimitW2 = 232448 - 1024;
-constexpr int kMaxRingW2 = 14;  // default logical S16 plane slots: 8 live + 4 or 6 in flight (TMA runs 2 - 3 steps ahead of the MMAs)
-constexpr int kRingCapW2 = 20;  // barrier slots (CGAN3D_W2_RING experiments: deeper ring, fewer mirrors)
+constexpr int kMaxRingW2 = 14;  // logical S16 plane slots: 8 live + 4 or 6 in flight (TMA runs 2 - 3 steps ahead of the MMAs)
 constexpr int kMaxPrefW2 = 11;     // staged 32-bit words per fetch thread and step
 constexpr int kBuildWarpsW2 = 10;  // warps 0-3 (also the epilogue) and 6-11 expand the operand
 constexpr int kFetchWarp0W2 = 12;  // warps 12-15 fetch and stage the raw Q1 words
 constexpr int kFetchersW2 = 128;
 constexpr int kThreadsW2 = 512;
-constexpr int kMaxStagesW2 = 4;
-constexpr int kMaxStageBufsW2 = 4;  // raw-line staging buffers (named barriers 1.. = full, 1 + kMaxStageBufsW2.. = empty)
+constexpr int kStagesW2 = 2;     // stages of the expanded operand
+constexpr int kStageBufsW2 = 3;  // raw-line staging buffers (named barriers 1.. = full, 1 + kStageBufsW2.. = empty): the fetch
+                                 // warps run two steps ahead of the builders
 constexpr int kBuildersW2 = (kBuildWarpsW2 + kFetchersW2 / 32) * 32;  // threads on the named barrier shared by the build and fetch warps (see bar_sync_builders)
 
 struct ThinW2Plan {
@@ -57,10 +56,6 @@ struct ThinW2Plan {
   uint32_t slot_bytes, e2_bytes, box_bytes, stage_words, smem_bytes;
   int zp;     // z-pair variant: K rows are pairs of voxels (zr = Zt / 2 rows per line), else single voxels (zr = Zt)
   int zr;
-  int nst;     // stages of the expanded operand (2..4)
-  int nsb;     // raw-line staging buffers (2..4): the fetch warps run nsb - 1 steps ahead of the builders
-  int cfence;  // 1: the MMA-issuing thread runs the generic->async proxy fence after its wait (DESIGN fact 12), 0: every builder before its arrive
-  int debug;  // CGAN3D_W2_DEBUG (profiling aid, results are wrong): 1 = skip the operand build, 2 = skip the MMAs, 4 = skip the plane loads, 8 = skip the Q1 loads
 };
 
 // Work = ncols columns (b, y-tile) x npairs plane pairs.  Columns are dealt to the CTAs ROUND-ROBIN (CTA c takes columns
@@ -97,8 +92,9 @@ struct SegIterW2 {
   }
 };
 
-// Hand-off of the two staging buffers between the fetch warps (producers) and the build warps (consumers): named barriers
-// 1 + buf ("full": 128 fetch threads arrive, 320 builders wait) and 3 + buf ("empty": the builders arrive, the fetchers wait).
+// Hand-off of the staging buffers between the fetch warps (producers) and the build warps (consumers): named barriers
+// 1 + buf ("full": 128 fetch threads arrive, 320 builders wait) and 1 + kStageBufsW2 + buf ("empty": the builders arrive, the
+// fetchers wait).
 __device__ __forceinline__ void bar_sync_id(uint32_t id) { static_assert(kBuildersW2 == 448, "barrier count"); asm volatile("bar.sync %0, 448;" ::"r"(id) : "memory"); }
 __device__ __forceinline__ void bar_arrive_id(uint32_t id) { asm volatile("bar.arrive %0, 448;" ::"r"(id) : "memory"); }
 
@@ -132,45 +128,24 @@ struct StepWalkW2 {
   }
 };
 
-// Built with -DCGAN3D_W2_PROF: CGAN3D_W2_DEBUG bit 16 makes CTA 0 print where each role's leading thread spends its cycles
-// (waits vs work; a named-barrier wait is charged to the NEXT lap because BAR.SYNC blocks at its first dependent
-// instruction).  Compiled out by default (the printf costs registers and stack).
-#ifdef CGAN3D_W2_PROF
-struct ProfW2 {
-  long long t0, acc[6];
-  bool on;
-  __device__ __forceinline__ ProfW2(bool on_) : on(on_) { for (int i = 0; i < 6; ++i) acc[i] = 0; t0 = on ? clock64() : 0; }
-  __device__ __forceinline__ void lap(int i) { if (on) { const long long t = clock64(); acc[i] += t - t0; t0 = t; } }
-};
-#define W2_PROF_PRINT(...) printf(__VA_ARGS__)
-#else
-struct ProfW2 {
-  static constexpr bool on = false;
-  long long acc[6];
-  __device__ __forceinline__ ProfW2(bool) {}
-  __device__ __forceinline__ void lap(int) {}
-};
-#define W2_PROF_PRINT(...) ((void)0)
-#endif
-
 template <bool ZP>
 __global__ void __launch_bounds__(kThreadsW2, 1)
 wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__restrict__ q1, float *__restrict__ dw,
                  const __grid_constant__ ThinW2Plan p) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t *ring = reinterpret_cast<uint8_t *>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);  // nphys S16 plane slots, [rows][16 ch], SWIZZLE_32B (TMA)
-  uint8_t *e2 = ring + (size_t)p.nphys * p.slot_bytes;          // 2 stages of the expanded operand, [L * Zt rows][2][8], SWIZZLE_32B
-  uint32_t *stage = reinterpret_cast<uint32_t *>(e2 + (size_t)p.nst * p.e2_bytes);  // nsb buffers of raw Q1 line segments [2][L][LW]
-  uint64_t *bars = reinterpret_cast<uint64_t *>(stage + (size_t)p.nsb * p.stage_words);
-  uint64_t *s_full = bars, *s_empty = bars + kRingCapW2, *e_full = s_empty + kRingCapW2, *e_empty = e_full + kMaxStagesW2, *done = e_empty + kMaxStagesW2;
+  uint8_t *e2 = ring + (size_t)p.nphys * p.slot_bytes;          // stages of the expanded operand, [L * Zt rows][2][8], SWIZZLE_32B
+  uint32_t *stage = reinterpret_cast<uint32_t *>(e2 + (size_t)kStagesW2 * p.e2_bytes);  // raw Q1 line segments [2][L][LW]
+  uint64_t *bars = reinterpret_cast<uint64_t *>(stage + (size_t)kStageBufsW2 * p.stage_words);
+  uint64_t *s_full = bars, *s_empty = bars + kMaxRingW2, *e_full = s_empty + kMaxRingW2, *e_empty = e_full + kStagesW2, *done = e_empty + kStagesW2;
   uint32_t *tmem_ptr = reinterpret_cast<uint32_t *>(done + 1);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   constexpr uint32_t kCols = ZP ? 256 : 128;  // accumulator columns: 8 planes x (32 | 16)
   constexpr uint32_t kNper = ZP ? 32 : 16;    // N elements per plane
 
   if (threadIdx.x == 0) {
-    for (int i = 0; i < kRingCapW2; ++i) { tc::mbar_init(&s_full[i], 1); tc::mbar_init(&s_empty[i], 1); }
-    for (int i = 0; i < kMaxStagesW2; ++i) { tc::mbar_init(&e_full[i], kBuildWarpsW2); tc::mbar_init(&e_empty[i], 1); }
+    for (int i = 0; i < kMaxRingW2; ++i) { tc::mbar_init(&s_full[i], 1); tc::mbar_init(&s_empty[i], 1); }
+    for (int i = 0; i < kStagesW2; ++i) { tc::mbar_init(&e_full[i], kBuildWarpsW2); tc::mbar_init(&e_empty[i], 1); }
     tc::mbar_init(done, 1);
     tc::fence_barrier_init();
   }
@@ -195,7 +170,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
   if (warp == 4) {
     // ------------------------------------------------ S16 plane producer (TMA).  A swizzled tensor map moves one inner row
     // (32 B of one voxel, or 64 B of a z pair) per request at ~3 cycles each, so the z-pair rows halve the engine's work
-    // per plane; with everything else disabled the plane loads add 0.08 ms to the kernel.  A 16-byte cp.async producer
+    // per plane; with everything else disabled the plane loads added 0.08 ms to the kernel.  A 16-byte cp.async producer
     // warp with the swizzle applied by hand was tried and is slower (5400 cycles per step).  Planes are numbered by the
     // order in which this CTA loads them: slot q % ring, mirrored at ring + slot when that exists.  A segment loads its 6
     // warm-up planes and then two planes per step, (ring - 8) / 2 steps ahead of the MMAs.
@@ -206,19 +181,12 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
       uint32_t slot = 0, use = 0;
       const uint32_t mirrored = (uint32_t)(p.nphys - p.ring);
       uint8_t *slot_ptr = ring;
-      ProfW2 prof((p.debug & 16) && blockIdx.x == 0);
       auto load_plane = [&](int xs, int b, int y0) {
-        prof.lap(0);
         if (use > 0) tc::mbar_wait(&s_empty[slot], (use - 1) & 1);
-        prof.lap(1);
-        if (p.debug & 4) {  // profiling aid: no plane loads at all
-          tc::mbar_arrive(&s_full[slot]);
-        } else {
-          const bool mirror = slot < mirrored;
-          tc::mbar_expect_tx(&s_full[slot], mirror ? 2 * p.box_bytes : p.box_bytes);
-          tc::tma_load_5d(slot_ptr, &tmS, &s_full[slot], 0, 0, y0, xs, b);
-          if (mirror) tc::tma_load_5d(slot_ptr + (size_t)p.ring * p.slot_bytes, &tmS, &s_full[slot], 0, 0, y0, xs, b);
-        }
+        const bool mirror = slot < mirrored;
+        tc::mbar_expect_tx(&s_full[slot], mirror ? 2 * p.box_bytes : p.box_bytes);
+        tc::tma_load_5d(slot_ptr, &tmS, &s_full[slot], 0, 0, y0, xs, b);
+        if (mirror) tc::tma_load_5d(slot_ptr + (size_t)p.ring * p.slot_bytes, &tmS, &s_full[slot], 0, 0, y0, xs, b);
         slot_ptr += p.slot_bytes;
         if (++slot == (uint32_t)p.ring) { slot = 0; ++use; slot_ptr = ring; }
       };
@@ -231,8 +199,6 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
           load_plane(2 * (p0 + i) + 1, b, y0);
         }
       }
-      prof.lap(0);
-      if (prof.on) W2_PROF_PRINT("w2 prof TMA : work %lld  wait s_empty %lld\n", prof.acc[0], prof.acc[1]);
     }
   } else if (warp == 5) {
     // ------------------------------------------------ MMA issuer
@@ -247,22 +213,17 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
     // of waited / ring, w0s = w0 % ring (all incremental: no runtime divisions on this warp's critical path)
     uint32_t waited = 0, w0 = 0, ws = 0, wph = 0, w0s = 0, st = 0, eph = 0;  // st, eph: operand stage of the step and its parity
     const uint32_t ringn = (uint32_t)p.ring;
-    ProfW2 prof((p.debug & 16) && blockIdx.x == 0 && lane == 0);
     int col, p0, plen;
     for (SegIterW2 it(ncols, p.npairs); it.next(col, p0, plen);) {
       w0 = waited;  // the segment's first window starts at its first warm-up plane
       w0s = ws;
-      prof.lap(0);
       for (int i = 0; i < plen; ++i, w0 += 2) {
         while (waited < w0 + 8) {
           tc::mbar_wait(&s_full[ws], wph);
           ++waited;
           if (++ws == ringn) { ws = 0; wph ^= 1u; }
         }
-        prof.lap(1);
-        tc::mbar_wait(&e_full[st], eph);
-        prof.lap(2);
-        if (p.cfence) tc::fence_proxy_async();  // the builders' plain stores -> visible to the MMAs issued below
+        tc::mbar_wait(&e_full[st], eph);  // the builders fenced their plain stores into the async proxy before arriving
         tc::tc_fence_after();
         const uint32_t a0 = (e2_u32 + st * p.e2_bytes) >> 4;
         uint32_t j = 0;
@@ -273,7 +234,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
           const uint32_t idesc = tc::make_idesc_bf16(128, (int)(kNper * run), 1, 1);
           const uint32_t b0 = (ring_u32 + slot * p.slot_bytes) >> 4;
           const uint32_t d = tmem_base + kNper * j;
-          if (leader && !(p.debug & 2)) {
+          if (leader) {
             uint64_t a_desc = a_hi | (uint64_t)(a0 & 0x3FFF), b_desc = b_hi | (uint64_t)(b0 & 0x3FFF);
 #pragma unroll 4
             for (int kb = 0; kb < p.kblocks; ++kb) {
@@ -285,7 +246,6 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
           __syncwarp();
           j += run;
         }
-        prof.lap(3);
         if (leader) {
           tc::umma_commit(&e_empty[st]);
           tc::umma_commit(&s_empty[w0s]);  // the two oldest planes leave the window (w0s is even, so is the ring)
@@ -294,8 +254,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
         __syncwarp();
         w0s += 2;
         if (w0s >= ringn) w0s -= ringn;
-        if (++st == (uint32_t)p.nst) { st = 0; eph ^= 1u; }
-        prof.lap(4);
+        if (++st == (uint32_t)kStagesW2) { st = 0; eph ^= 1u; }
       }
       // the six planes still resident belong to this segment only
       if (leader)
@@ -304,20 +263,18 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
     }
     if (leader) tc::umma_commit(done);
     __syncwarp();
-    if (prof.on) W2_PROF_PRINT("w2 prof MMA : other %lld  wait s_full %lld  wait e_full %lld  issue %lld  commit %lld (leader %d)\n", prof.acc[0], prof.acc[1],
-             prof.acc[2], prof.acc[3], prof.acc[4], (int)leader);
   } else {
     // ------------------------------------------------ warps 0..3, 6..11: build the expanded operand (0..3 then run the
     // epilogue); warps 12..15: bring the raw Q1 words of the next steps into the staging buffers.  The roles are split
     // because the generic->async proxy fence that publishes the operand compiles to MEMBAR.ALL.CTA, which waits for every
     // outstanding global load of the executing thread: a warp that prefetches AND builds exposes the full load latency
-    // (~1 us under load) in every step.  The staging area has nsb buffers handed over with arrive / wait named barriers,
-    // so the fetch warps run nsb - 1 steps ahead of the builders.
-    // Where the time goes now (per-role cycle counters, -DCGAN3D_W2_PROF; `first` at C3, ~1590 cycles per step): the 8
-    // N = 256 MMAs of a step read 96 KB of shared memory, the TMA fills write 23 KB (mirrors included), the builders move
-    // 36 KB, the staging 10 KB: ~165 KB per step against 128 B/clk = 1290 cycles.  Shared-memory bandwidth, not the tensor
-    // pipe (8 x 128 cycles), bounds the step (DESIGN fact 13); deeper rings, more operand stages and a consumer-side fence
-    // (CGAN3D_W2_RING / _STAGES / _CFENCE) change nothing.
+    // (~1 us under load) in every step.  The staging area has kStageBufsW2 buffers handed over with arrive / wait named
+    // barriers, so the fetch warps run two steps ahead of the builders.
+    // Where the time went when measured with per-role cycle counters (`first` at C3, ~1590 cycles per step): the 8 N = 256
+    // MMAs of a step read 96 KB of shared memory, the TMA fills write 23 KB (mirrors included), the builders move 36 KB, the
+    // staging 10 KB: ~165 KB per step against 128 B/clk = 1290 cycles.  Shared-memory bandwidth, not the tensor pipe
+    // (8 x 128 cycles), bounds the step (DESIGN fact 13); deeper rings, more operand stages and a fence on the MMA side
+    // instead of the builders' changed nothing (DESIGN §4.2).
     const int ZqW = p.Zq >> 1;
     const SegIterW2 range(ncols, p.npairs);
     const uint32_t total = (uint32_t)range.steps();
@@ -328,7 +285,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
       // word i of this thread: staging index tid + 128 i = (h, l, w); rel = its offset from the step's base pointer.  Validity
       // is a bit mask over i: z range (fixed), line in [0, Yq) (changes with the column), plane in [0, Xq) (changes with the
       // step, one mask per plane h).  The words travel global -> shared as 4-byte zero-filling cp.async (src-size 0 for an
-      // invalid word): no branches, no registers, and the load latency is covered by nsb - 1 steps of lookahead instead of
+      // invalid word): no branches, no registers, and the load latency is covered by two steps of lookahead instead of
       // being exposed in this warp (first form: 11 branchy __ldg + st.shared per thread and step = 1700 cycles per step with
       // the warps never idle — the kernel's bottleneck).
       int rel[kMaxPrefW2];
@@ -347,7 +304,6 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
           rel[i] = (h * p.Yq + l) * ZqW + w;
         }
       }
-      ProfW2 prof((p.debug & 16) && blockIdx.x == 0 && tid == 0);
       StepWalkW2 walk(range);
       int cur_col = -1;
       uint32_t ymask = 0;
@@ -369,8 +325,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
         walk.advance();
         // base may point outside the tensor (halo): it is only dereferenced for in-range (plane, line)
         const uint32_t *base = col_base + (long long)xb * plane_words;
-        uint32_t valid = zmask & ymask & (((unsigned)xb < (unsigned)p.Xq ? mh[0] : 0u) | ((unsigned)(xb + 1) < (unsigned)p.Xq ? mh[1] : 0u));
-        if (p.debug & 8) valid = 0;
+        const uint32_t valid = zmask & ymask & (((unsigned)xb < (unsigned)p.Xq ? mh[0] : 0u) | ((unsigned)(xb + 1) < (unsigned)p.Xq ? mh[1] : 0u));
         const uint32_t dst = stage_u32 + buf * stage_stride;
 #pragma unroll
         for (int i = 0; i < kMaxPrefW2; ++i) {
@@ -382,32 +337,26 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
         }
         asm volatile("cp.async.commit_group;" ::: "memory");
       };
-      // steps k .. k + nsb - 2 are in flight while step k is handed over; buffer (k + nsb - 1) % nsb was read by step k - 1
-      const uint32_t nsb = (uint32_t)p.nsb, ahead = nsb - 1;
+      // steps k .. k + 1 are in flight while step k is handed over; buffer (k + 2) % 3 was read by step k - 1
+      const uint32_t nsb = (uint32_t)kStageBufsW2, ahead = nsb - 1;
       uint32_t issued = 0, ibuf = 0, buf = 0;
       for (; issued < ahead && issued < total; ++issued) {
         issue(ibuf);
         if (++ibuf == nsb) ibuf = 0;
       }
       for (; n < total; ++n) {
-        prof.lap(0);
-        // the group of step n is the oldest of (issued - n) pending ones
-        if (issued - n >= 3) asm volatile("cp.async.wait_group 2;" ::: "memory");
-        else if (issued - n == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
+        // the group of step n is the oldest of (issued - n) <= 2 pending ones
+        if (issued - n == 2) asm volatile("cp.async.wait_group 1;" ::: "memory");
         else asm volatile("cp.async.wait_group 0;" ::: "memory");
-        prof.lap(2);
         bar_arrive_id(1 + buf);
         if (++buf == nsb) buf = 0;
         if (issued < total) {
-          if (issued >= nsb) bar_sync_id(1 + kMaxStageBufsW2 + ibuf);  // the builders have finished reading step issued - nsb
-          prof.lap(1);
+          if (issued >= nsb) bar_sync_id(1 + kStageBufsW2 + ibuf);  // the builders have finished reading step issued - nsb
           issue(ibuf);
           ++issued;
           if (++ibuf == nsb) ibuf = 0;
         }
       }
-      prof.lap(0);
-      if (prof.on) W2_PROF_PRINT("w2 prof FETCH: issue %lld  wait empty %lld  wait loads %lld  steps %u\n", prof.acc[0], prof.acc[1], prof.acc[2], total);
     } else {
       const int bw = warp < 4 ? warp : warp - 2;  // builder warp 0..9
       // E2[l * Zt + r][h][j] = line(h, l)[r + j], j = 0..7.  A warp iteration = 32 rows of one staged line (h, l): 5
@@ -428,7 +377,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
       // and all loads of a step are issued before the first store (the looped form below exposes the LDS -> STS latency of
       // every iteration: 240 cycles each while the tensor core is reading shared memory).
       constexpr int kFastPerW2 = 6;
-      const bool fast = ZP && per <= kFastPerW2 && !(p.debug & 32);  // debug bit 32: looped form
+      const bool fast = ZP && per <= kFastPerW2;
       uint32_t f_src[kFastPerW2], f_dst[kFastPerW2], f_ok = 0;
 #pragma unroll
       for (int q = 0; q < kFastPerW2; ++q) {
@@ -441,14 +390,10 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
           f_dst[q] = (uint32_t)(l * p.zr + rb * 32 + lane) * 32u + (((uint32_t)h ^ swz) << 4);
         }
       }
-      ProfW2 prof((p.debug & 16) && blockIdx.x == 0 && threadIdx.x == 0);
       for (; n < total; ++n) {
-        prof.lap(0);
         bar_sync_id(1 + sb);  // the fetch warps have written this step's staging buffer
-        prof.lap(1);
         if (use > 0) tc::mbar_wait(&e_empty[st], (use - 1) & 1);
-        prof.lap(2);
-        if (fast && !(p.debug & 1)) {
+        if (fast) {
           const uint32_t sbase = tc::smem_u32(stage) + sb * stage_stride, dbase = tc::smem_u32(e2) + st * p.e2_bytes;
           uint32_t a[kFastPerW2][4];
 #pragma unroll
@@ -464,7 +409,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
           for (int q = 0; q < kFastPerW2; ++q)
             if ((f_ok >> q) & 1u)
               asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(dbase + f_dst[q]), "r"(a[q][0]), "r"(a[q][1]), "r"(a[q][2]), "r"(a[q][3]) : "memory");
-        } else if (!(p.debug & 1)) {
+        } else {
           const uint32_t dst_u32 = tc::smem_u32(e2) + st * p.e2_bytes + lane_dst;
           int it = it0, hl = hl0, rb = rb0;
           while (it < it1) {
@@ -494,17 +439,13 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
             ++hl;
           }
         }
-        prof.lap(3);
-        if (n + (uint32_t)p.nsb < total) bar_arrive_id(1 + kMaxStageBufsW2 + sb);  // this warp has read the staging buffer: the fetch warps may refill it
-        if (++sb == (uint32_t)p.nsb) sb = 0;
-        if (!p.cfence) tc::fence_proxy_async();  // generic-proxy writes -> visible to the tensor core's async-proxy reads
+        if (n + (uint32_t)kStageBufsW2 < total) bar_arrive_id(1 + kStageBufsW2 + sb);  // this warp has read the staging buffer: the fetch warps may refill it
+        if (++sb == (uint32_t)kStageBufsW2) sb = 0;
+        tc::fence_proxy_async();  // generic-proxy writes -> visible to the tensor core's async-proxy reads
         __syncwarp();
         if (lane == 0) tc::mbar_arrive(&e_full[st]);
-        if (++st == (uint32_t)p.nst) { st = 0; ++use; }
-        prof.lap(4);
+        if (++st == (uint32_t)kStagesW2) { st = 0; ++use; }
       }
-      if (prof.on) W2_PROF_PRINT("w2 prof BUILD: other %lld  wait full %lld  wait e_empty %lld  build %lld  fence+arrive %lld\n", prof.acc[0], prof.acc[1],
-               prof.acc[2], prof.acc[3], prof.acc[4]);
     }
     // epilogue: TMEM lane m = (dy = m >> 4, dx_lo = (m >> 3) & 1, dz = m & 7); column = 16 * j + c, dx = 6 - j + dx_lo
     if (n > 0 && warp < 4) {
@@ -541,16 +482,7 @@ wgrad7_v2_kernel(const __grid_constant__ CUtensorMap tmS, const uint32_t *__rest
 }
 
 // ---------------------------------------------------------------- host side
-typedef CUresult (*EncodeTiledFnW2)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                    const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-void *tc_encode_fn_ptr();              // conv_tc.cu
-CUtensorMapL2promotion tc_l2_promo();  // conv_tc.cu
-
 static bool plan_w2(const cgan3d_conv_geom &g, ThinW2Plan &p) {
-  static int off = -1;
-  if (off < 0) off = getenv("CGAN3D_WGRAD7_V1") ? 1 : 0;
-  if (off) return false;
   if (g.k != 7 || g.stride != 1) return false;
   const bool first = g.Cb == 1 && g.Cs == 16, last = g.Cb == 16 && g.Cs == 1;
   if (!first && !last) return false;
@@ -566,16 +498,8 @@ static bool plan_w2(const cgan3d_conv_geom &g, ThinW2Plan &p) {
   p.LW = (p.Zt + 8) / 2 + 1;
   p.nb16 = p.Zt / 16;
   p.inv_nb16 = (65536 + p.nb16 - 1) / p.nb16;
-  static int v2_single = -1;  // CGAN3D_WGRAD7_V2_SINGLE: one voxel per K row (the first form of this kernel), for A/B timing
-  if (v2_single < 0) v2_single = getenv("CGAN3D_WGRAD7_V2_SINGLE") ? 1 : 0;
-  p.zp = (v2_single || (p.Zs & 1)) ? 0 : 1;
+  p.zp = (p.Zs & 1) ? 0 : 1;  // an odd extent keeps one voxel per K row
   p.zr = p.zp ? p.Zt / 2 : p.Zt;
-  p.nst = 2;
-  if (const char *e = getenv("CGAN3D_W2_STAGES")) p.nst = mx(2, mn(kMaxStagesW2, atoi(e)));
-  p.nsb = 3;
-  if (const char *e = getenv("CGAN3D_W2_STAGEBUFS")) p.nsb = mx(2, mn(kMaxStageBufsW2, atoi(e)));
-  p.cfence = 0;
-  if (const char *e = getenv("CGAN3D_W2_CFENCE")) p.cfence = atoi(e) ? 1 : 0;
   // pass 0 only takes a tile whose ring is the deep one (14 logical slots, >= 4 mirrored); pass 1 takes what fits
   for (int pass = p.zp ? 0 : 1; pass < 2 && p.Yt == 0; ++pass)
   for (int Yt = mn(p.Ys, 8); Yt >= 1; --Yt) {
@@ -585,23 +509,17 @@ static bool plan_w2(const cgan3d_conv_geom &g, ThinW2Plan &p) {
     const uint32_t slot = (uint32_t)Yt * p.Zt * 32u;
     const uint32_t e2b = ((uint32_t)L * p.zr * 32u + 1023u) / 1024u * 1024u;
     const uint32_t stage_words = ((uint32_t)(2 * L * p.LW) + 3u) & ~3u;
-    const uint32_t fixed = (uint32_t)p.nst * e2b + (uint32_t)p.nsb * stage_words * 4 + 512;
+    const uint32_t fixed = (uint32_t)kStagesW2 * e2b + (uint32_t)kStageBufsW2 * stage_words * 4 + 512;
     if (slot % 1024) continue;
     int nphys = (int)((kSmemLimitW2 - mn(kSmemLimitW2, fixed)) / slot);
-    const int nphys_fit = nphys;
     if (nphys > kMaxRingW2 + 6) nphys = kMaxRingW2 + 6;
     // ring of 14 (TMA three steps ahead) when at least four of its slots can be mirrored, else 12; a mirrored slot keeps the
     // window of 8 planes contiguous, so most steps need ONE N = 128 MMA per K block
-    int ring = nphys >= kMaxRingW2 + 4 ? kMaxRingW2 : 12;
-    if (const char *e = getenv("CGAN3D_W2_RING")) {  // experiment: ring depth / mirror split
-      const int want = mx(10, mn(kRingCapW2, atoi(e))) & ~1;
-      if (nphys_fit >= want) { ring = want; nphys = mn(nphys_fit, ring + 6); }
-    }
+    const int ring = nphys >= kMaxRingW2 + 4 ? kMaxRingW2 : 12;
     if (nphys < ring + 2 && Yt > 1) continue;
     if (nphys < ring) continue;
     if (pass == 0 && ring < kMaxRingW2) continue;
     if (nphys > ring + 6) nphys = ring + 6;  // windows start at even slots <= ring - 2: six mirrors make every window contiguous
-    if (const char *e = getenv("CGAN3D_W2_NPHYS")) nphys = mx(ring, mn(nphys, atoi(e)));  // experiment: fewer mirrored slots
     p.Yt = Yt; p.L = L; p.nphys = nphys; p.ring = ring;
     p.slot_bytes = slot; p.e2_bytes = e2b; p.stage_words = stage_words;
     p.smem_bytes = fixed + (uint32_t)nphys * slot;
@@ -623,7 +541,6 @@ bool thin_w2_supported(const cgan3d_conv_geom &g) {
 int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {
   ThinW2Plan p;
   if (!plan_w2(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin wgrad v2: shape not supported");
-  if (const char *e = getenv("CGAN3D_W2_DEBUG")) p.debug = atoi(e);
   const bool first = p.flip == 0;
   const void *s16 = first ? small : big, *q1 = first ? big : small;
   if ((reinterpret_cast<uintptr_t>(s16) & 15) || (reinterpret_cast<uintptr_t>(q1) & 3))
@@ -632,7 +549,7 @@ int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, f
     cudaError_t e = cudaMemsetAsync(dw, 0, (size_t)16 * 343 * sizeof(float), st);
     if (e != cudaSuccess) return cuda_fail(e, "tcgen05 thin wgrad v2 memset");
   }
-  EncodeTiledFnW2 enc = reinterpret_cast<EncodeTiledFnW2>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   CUtensorMap tmS;
   {
@@ -643,8 +560,8 @@ int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, f
     const cuuint32_t box[5] = {(cuuint32_t)(16 * vox), (cuuint32_t)p.zr, (cuuint32_t)p.Yt, 1, 1};
     const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
     CUresult r = enc(&tmS, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(s16), gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, p.zp ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B, tc_l2_promo(),
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, p.zp ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (thin wgrad v2) failed with %d", (int)r);
   }
   static bool attr_set = false;

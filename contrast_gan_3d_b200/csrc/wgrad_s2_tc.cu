@@ -13,14 +13,14 @@
 //     taps per MMA.
 //   * The 4 parity-class sub-slabs of X are adjacent N blocks: ONE MMA with N = 4*Cb covers every class at a row shift.
 //     2 (Cs = 32) or 4 (Cs = 64) MMAs per K block and dx instead of 6-9.
-//   * Stride 1 (the generator's ResNet layers, Cs = 64): the N blocks are the SAME X halo slab one / two voxels later
-//     (LBO = one row), so one MMA with N = 3*Cb yields the three dz taps of a (dx, dy) pair: 3 MMAs per K block and dx
-//     instead of 9.
+//   * Cs == 64 runs M = 128 the same way: block 0 = dY[z-1], block 1 = dY[z].
+//   * Stride 1 (the generator's ResNet layers, Cs = 64): the N blocks are the SAME X halo slab zero and two voxels later
+//     (LBO = two rows), so one M = 128 MMA with N = 2*Cb yields the three dz taps of a (dx, dy) pair: 3 MMAs per K block
+//     and dx instead of 9.
 //   * A CTA owns one dx (filter x-offset) and a contiguous range of (b, y-slab, x) steps; split-K over CTAs, fp32 atomics.
 #include "common.cuh"
 #include "conv_internal.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace cg {
 
@@ -33,7 +33,6 @@ struct WsPlan {
   int Cb, Cs, k, taps;
   int Zh, Yt, Yh, nslabs;
   int kpad, rowsA, rowsB;
-  int nblkA;       // M blocks: 1 (Cs == 64) or 2 (Cs == 32: block 1 = the slab one row later)
   int stride;      // 2: N blocks = the 4 parity-class sub-slabs; 1: N blocks = 3 row-shifted views of one halo slab
   int nsrc, nblkB; // TMA sub-slabs of X per step / N blocks per MMA
   uint32_t lboB;   // bytes between N blocks
@@ -41,8 +40,7 @@ struct WsPlan {
   uint16_t row_shift[kMaxWsMma];
   int8_t acc_tap[kMaxWsMma][2][4];  // (dy*k+dz) of [MMA][M block][N block]; -1 = discard
   uint32_t rowbytesA, rowbytesB, a_bytes, srcB_bytes, stage_bytes, boxA_bytes, boxB_bytes, smem_bytes, tmem_cols;
-  int debug;
-  int m128;  // stride-1, Cs == 64: M = 128 = dY[z-1] | dY[z] (two z-adjacent taps per MMA), N = 2 views (shift 0 and 2)
+  int m128;  // Cs == 64: M = 128 = dY[z-1] | dY[z] (two z-adjacent taps per MMA); Cs == 32: M = 64, the same two M blocks
 };
 
 __global__ void __launch_bounds__(192, 1)
@@ -95,8 +93,8 @@ wgrad_s2_sw_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constan
         if (use > 0) tc::mbar_wait(&empty[s], (use - 1) & 1);
         tc::mbar_expect_tx(&full[s], p.boxA_bytes + p.nsrc * p.boxB_bytes);
         uint8_t *a = stage_mem + (size_t)s * p.stage_bytes, *bb = a + p.a_bytes;
-        // dY slab; with two M blocks it starts one voxel early so that block 0 = dY[z-1] and block 1 (next row) = dY[z]
-        tc::tma_load_5d(a, &tmY, &full[s], 0, p.nblkA == 2 ? -1 : 0, y0, x, b);
+        // dY slab, one voxel early so that M block 0 = dY[z-1] and block 1 (next row) = dY[z]
+        tc::tma_load_5d(a, &tmY, &full[s], 0, -1, y0, x, b);
         if (p.stride == 2) {
           for (int src = 0; src < 4; ++src)  // parity class (q, r) = (src >> 1, src & 1): sub-slab starts at 2*o - class
             tc::tma_load_5d(bb + (size_t)src * p.srcB_bytes, &tmX, &full[s], 0, -(src & 1), 2 * y0 - (src >> 1), 2 * x + dx - 1, b);
@@ -141,6 +139,7 @@ wgrad_s2_sw_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constan
     // epilogue: TMEM lane 32*warp + l: l < 16 -> accumulator 2g row 16*warp + l, l >= 16 -> accumulator 2g + 1
     tc::mbar_wait(done, 0);
     tc::tc_fence_after();
+    float *dw_dx = dw + dx * p.k * p.k;  // this CTA's filter x-offset
     if (p.m128) {  // M = 128: TMEM lane 32*warp + l is accumulator row 32*warp + l = (block, channel)
       const int m = warp * 32 + lane;
       const int cs = m & 63, blk = m >> 6;
@@ -154,7 +153,7 @@ wgrad_s2_sw_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constan
             const int nn = c0 + c;
             const int src = nn / p.Cb, cb = nn - src * p.Cb;
             const int t2 = p.acc_tap[j][blk][src];
-            if (t2 >= 0 && !p.debug) atomicAdd(&dw[((size_t)cs * p.Cb + cb) * p.taps + dx * p.k * p.k + t2], __uint_as_float(v[c]));
+            if (t2 >= 0) atomicAdd(&dw_dx[((size_t)cs * p.Cb + cb) * p.taps + t2], __uint_as_float(v[c]));
           }
         }
     } else {
@@ -173,7 +172,7 @@ wgrad_s2_sw_kernel(const __grid_constant__ CUtensorMap tmY, const __grid_constan
             const int nn = c0 + c;
             const int src = nn / p.Cb, cb = nn - src * p.Cb;
             const int t2 = p.acc_tap[j][blk][src];
-            if (t2 >= 0 && !p.debug) atomicAdd(&dw[((size_t)cs * p.Cb + cb) * p.taps + dx * p.k * p.k + t2], __uint_as_float(v[c]));
+            if (t2 >= 0) atomicAdd(&dw_dx[((size_t)cs * p.Cb + cb) * p.taps + t2], __uint_as_float(v[c]));
           }
         }
       }
@@ -205,42 +204,36 @@ static bool plan_ws(const cgan3d_conv_geom &g, WsPlan &p) {
   const int halo = s == 1 ? 2 : 1;
   p.Zh = p.Z + halo;
   if (s * (p.Zh - 1) + 1 > 256) return false;
-  p.nblkA = 64 / g.Cs;
+  p.m128 = g.Cs == 64 ? 1 : 0;
   p.rowbytesA = 2u * g.Cs;
   p.rowbytesB = 2u * g.Cb;
   p.stages = 2;
   int nm = 0;
   if (s == 2) {
     p.nsrc = 4; p.nblkB = 4;
-    if (g.Cs == 64 && !getenv("CGAN3D_WS_M64")) { p.nblkA = 2; p.m128 = 1; }  // M = 128: dY[z-1] | dY[z], as for Cs == 32 at M = 64
-    // MMA program: sub-grid shift (sy, sz) in {0,1}^2; tap d has parity class (d-1)&1 and shift (d - 1 + class) / 2
+    // MMA program: sub-grid shift (sy, sz) in {0,1}^2; tap d has parity class (d-1)&1 and shift (d - 1 + class) / 2.  The two
+    // M blocks cover both z shifts: block 0 holds dY[z-1] (z shift 1), block 1 holds dY[z] (z shift 0).
     auto cls = [](int d) { return (d - 1) & 1; };
     auto shf = [&](int d) { return (d - 1 + cls(d)) / 2; };
     auto find = [&](int c, int sh) { for (int d = 0; d < k; ++d) if (cls(d) == c && shf(d) == sh) return d; return -1; };
-    for (int by = 0; by < 2; ++by)
-      for (int bz = 0; bz < 2; bz += p.nblkA) {
-        bool any = false;
-        for (int blk = 0; blk < 2; ++blk)
-          for (int src = 0; src < 4; ++src) {
-            int tap = -1;
-            if (blk < p.nblkA) {
-              // two M blocks: block 0 holds dY[z-1] (z shift bz + 1), block 1 holds dY[z] (z shift bz)
-              const int sz = p.nblkA == 2 ? bz + 1 - blk : bz;
-              const int dy = find(src >> 1, by), dz = find(src & 1, sz);
-              if (dy >= 0 && dz >= 0) tap = dy * k + dz;
-            }
-            p.acc_tap[nm][blk][src] = (int8_t)tap;
-            any = any || tap >= 0;
-          }
-        if (!any) continue;
-        p.row_shift[nm] = (uint16_t)(by * p.Zh + bz);
-        ++nm;
-      }
-  } else if (g.Cs == 64 && !getenv("CGAN3D_WS_M64")) {
+    for (int by = 0; by < 2; ++by) {
+      bool any = false;
+      for (int blk = 0; blk < 2; ++blk)
+        for (int src = 0; src < 4; ++src) {
+          int tap = -1;
+          const int dy = find(src >> 1, by), dz = find(src & 1, 1 - blk);
+          if (dy >= 0 && dz >= 0) tap = dy * k + dz;
+          p.acc_tap[nm][blk][src] = (int8_t)tap;
+          any = any || tap >= 0;
+        }
+      if (!any) continue;
+      p.row_shift[nm] = (uint16_t)(by * p.Zh);
+      ++nm;
+    }
+  } else {
     // M = 128: block 0 = dY[z-1], block 1 = dY[z] (the slab one row later); N blocks = the X halo slab 0 and 2 voxels later.
     // (block 1, shift s) is tap dz = s, (block 0, shift s) is tap dz = s + 1: dz = 0, 1, 2 from one MMA of N = 2*Cb, which
     // costs 84.5 cycles instead of the 96.9 of an M = 64, N = 3*Cb MMA that leaves half of the tensor rows idle.
-    p.m128 = 1; p.nblkA = 2;
     p.nsrc = 1; p.nblkB = 2;
     for (int dy = 0; dy < 3; ++dy) {
       for (int blk = 0; blk < 2; ++blk)
@@ -248,14 +241,6 @@ static bool plan_ws(const cgan3d_conv_geom &g, WsPlan &p) {
           const int dz = nb < 2 ? (blk == 1 ? 2 * nb : 2 * nb + 1) : -1;
           p.acc_tap[nm][blk][nb] = (int8_t)((dz >= 0 && dz < 3) ? dy * 3 + dz : -1);
         }
-      p.row_shift[nm] = (uint16_t)(dy * p.Zh);
-      ++nm;
-    }
-  } else {
-    p.nsrc = 1; p.nblkB = 3;
-    for (int dy = 0; dy < 3; ++dy) {  // N block dz = the halo slab dz voxels later
-      for (int blk = 0; blk < 2; ++blk)
-        for (int nb = 0; nb < 4; ++nb) p.acc_tap[nm][blk][nb] = (int8_t)((blk == 0 && nb < 3) ? dy * 3 + nb : -1);
       p.row_shift[nm] = (uint16_t)(dy * p.Zh);
       ++nm;
     }
@@ -289,7 +274,7 @@ static bool plan_ws(const cgan3d_conv_geom &g, WsPlan &p) {
   sizes(p.Yt, p.kpad, p.rowsA, p.rowsB);
   p.a_bytes = ((uint32_t)p.rowsA * p.rowbytesA + 1023) / 1024 * 1024;
   p.srcB_bytes = ((uint32_t)p.rowsB * p.rowbytesB + 1023) / 1024 * 1024;
-  p.lboB = s == 2 ? p.srcB_bytes : (p.m128 ? 2 * p.rowbytesB : p.rowbytesB);
+  p.lboB = s == 2 ? p.srcB_bytes : 2 * p.rowbytesB;
   p.stage_bytes = p.a_bytes + p.nsrc * p.srcB_bytes;
   p.boxA_bytes = p.rowbytesA * p.Zh * p.Yt;
   p.boxB_bytes = p.rowbytesB * p.Zh * p.Yh;
@@ -301,14 +286,8 @@ static bool plan_ws(const cgan3d_conv_geom &g, WsPlan &p) {
   return true;
 }
 
-typedef CUresult (*EncodeTiledFnW)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-void *tc_encode_fn_ptr();               // conv_tc.cu
-CUtensorMapL2promotion tc_l2_promo();   // conv_tc.cu
-
 static int encode_voxel_map(CUtensorMap *tm, const void *ptr, int C, int Z, int Y, int X, int B, int nz, int ny, int es) {
-  EncodeTiledFnW enc = reinterpret_cast<EncodeTiledFnW>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   const cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)B};
   const cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2, (cuuint64_t)X * Y * Z * C * 2};
@@ -316,7 +295,7 @@ static int encode_voxel_map(CUtensorMap *tm, const void *ptr, int C, int Z, int 
   const cuuint32_t estr[5] = {1, (cuuint32_t)es, (cuuint32_t)es, 1, 1};
   const CUtensorMapSwizzle swz = C * 2 == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (C * 2 == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, tc_l2_promo(), CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (strided wgrad) failed with %d", (int)r);
   return 0;
 }
@@ -329,7 +308,6 @@ bool tc_wgrad_s2_supported(const cgan3d_conv_geom &g) {
 int tc_wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {
   WsPlan p;
   if (!plan_ws(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 strided wgrad: shape not supported");
-  if (const char *e = getenv("CGAN3D_WS_DEBUG")) p.debug = atoi(e);
   if ((reinterpret_cast<uintptr_t>(big) & 15) || (reinterpret_cast<uintptr_t>(small) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 strided wgrad: pointers must be 16-byte aligned");
   if (beta == 0.f) {

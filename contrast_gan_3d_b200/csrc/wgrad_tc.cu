@@ -278,21 +278,15 @@ static bool plan_wgrad(const cgan3d_conv_geom &g, WgPlan &p) {
   return true;
 }
 
-typedef CUresult (*EncodeTiledFn3)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
-                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-void *tc_encode_fn_ptr();  // conv_tc.cu
-CUtensorMapL2promotion tc_l2_promo();  // conv_tc.cu
-
 static int encode_act_map(CUtensorMap *tm, const void *ptr, int C, int Z, int Y, int X, int B, int nz, int ny, int es) {
-  EncodeTiledFn3 enc = reinterpret_cast<EncodeTiledFn3>(tc_encode_fn_ptr());
+  EncodeTiledFn enc = tc_encode_fn();
   if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   const cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)B};
   const cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2, (cuuint64_t)X * Y * Z * C * 2};
   const cuuint32_t box[5] = {8, (cuuint32_t)(es * (nz - 1) + 1), (cuuint32_t)(es * (ny - 1) + 1), 1, 1};
   const cuuint32_t estr[5] = {1, (cuuint32_t)es, (cuuint32_t)es, 1, 1};
   CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, tc_l2_promo(),
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled failed with %d", (int)r);
   return 0;

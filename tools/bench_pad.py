@@ -1,6 +1,6 @@
 """Device time of the reflection-pad kernels at the generator's C3 shapes (CUDA events, L2 flushed between iterations).
 
-    python tools/bench_pad.py            # CGAN3D_PADBWD_LPB=1 reproduces the one-line-per-block adjoint
+    python tools/bench_pad.py
 """
 import json
 import sys
