@@ -9,6 +9,8 @@
 
 namespace cg {
 
+using bf16 = __nv_bfloat16;
+
 // thread-local last error text (cgan3d_last_error)
 char *err_buf();
 int fail(int code, const char *fmt, ...);
@@ -92,5 +94,6 @@ template <typename T>
 __host__ __device__ __forceinline__ T mn(T a, T b) { return a < b ? a : b; }
 template <typename T>
 __host__ __device__ __forceinline__ T mx(T a, T b) { return a > b ? a : b; }
+static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
 }  // namespace cg

@@ -19,20 +19,7 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-constexpr uint32_t kSmemLimitD1 = 232448 - 1024;
-
-static int encode_map_d1(CUtensorMap *tm, const void *ptr, int rank, const cuuint64_t *gdim, const cuuint64_t *gstr,
-                         const cuuint32_t *box, const cuuint32_t *estr) {
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (critic first layer) failed with %d", (int)r);
-  return 0;
-}
-static inline int round_up_d1(int v, int m) { return (v + m - 1) / m * m; }
+constexpr uint32_t kSmemLimitD1 = kMaxDynSmem - 1024;
 
 static bool d1_shape(const cgan3d_conv_geom &g) {
   return g.k == 4 && g.stride == 2 && g.pad == 1 && g.Cb == 1 && g.Cs == 8;
@@ -230,7 +217,7 @@ static bool plan_d1_gather(const cgan3d_conv_geom &g, D1GatherPlan &best) {
   if (!d1_shape(g)) return false;
   D1GatherPlan p{};
   p.B = g.B; p.Xi = g.Xb; p.Yi = g.Yb; p.Zi = g.Zb; p.Xo = g.Xs; p.Yo = g.Ys; p.Zo = g.Zs;
-  p.Zc = round_up_d1(p.Zi + 17, 8);
+  p.Zc = round_up(p.Zi + 17, 8);
   p.nzb = (p.Zo + 3) / 4;
   const uint32_t fixed = kD1Tiles * kD1TileBytes + 512;
   double best_score = 0;
@@ -242,7 +229,7 @@ static bool plan_d1_gather(const cgan3d_conv_geom &g, D1GatherPlan &best) {
       if (Yt > mt * 128) continue;
       const int Xt = mn(p.Xo, (mt * 128 - Yt) / Yh + 1), Xh = Xt + 1;
       if (2 * (Xh - 1) + 1 > 256) continue;
-      const int rows_alloc = round_up_d1(mx(Xh * Yh, mt * 128 + Yh + 1), 8);
+      const int rows_alloc = round_up(mx(Xh * Yh, mt * 128 + Yh + 1), 8);
       const uint32_t slot = 2u * rows_alloc * 16;
       const int nslots = (int)mn<uint32_t>(8, (kSmemLimitD1 - fixed) / slot);
       if (nslots < 4) continue;
@@ -290,21 +277,14 @@ static int run_d1_gather(const cgan3d_conv_geom &g, const void *in, const void *
   const cuuint64_t gstr[3] = {zc * 2, (cuuint64_t)p.Yi * zc * 2, (cuuint64_t)p.Xi * p.Yi * zc * 2};
   const cuuint32_t box[4] = {8, (cuuint32_t)(2 * (p.Yh - 1) + 1), (cuuint32_t)(2 * (p.Xh - 1) + 1), 1};
   const cuuint32_t estr[4] = {1, 2, 2, 1};
-  int r = encode_map_d1(&tm, cp, 4, gdim, gstr, box, estr);
+  int r = encode_tiled(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, cp, gdim, gstr, box, estr, CU_TENSOR_MAP_SWIZZLE_NONE, "critic first layer");
   if (r) return r;
   const long long total = (long long)p.B * p.nxt * p.nyt * p.nzb;
   const int grid = (int)mn<long long>(total, (long long)num_sms());
   auto launch = [&](auto mt_tag) -> int {
     constexpr int MT = decltype(mt_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(d1_gather_tc_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitD1 + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(d1_gather_tc_kernel)");
-      attr_set = true;
-    }
-    d1_gather_tc_kernel<MT><<<grid, 192, p.smem_bytes + 1024, st>>>(tm, wt, reinterpret_cast<bf16 *>(outp), p);
-    CG_LAUNCH_CHECK("d1_gather_tc_kernel");
-    return 0;
+    return tc_launch<d1_gather_tc_kernel<MT>>("d1_gather_tc_kernel", grid, 192, p.smem_bytes + 1024, 1, st, tm, wt,
+                                              reinterpret_cast<bf16 *>(outp), p);
   };
   switch (p.mtiles) {
     case 1: return launch(std::integral_constant<int, 1>{});
@@ -450,8 +430,8 @@ static bool plan_d1_wgrad(const cgan3d_conv_geom &g, D1WgradPlan &p) {
   p.B = g.B; p.Xi = g.Xb; p.Yi = g.Yb; p.Zi = g.Zb; p.Xs = g.Xs; p.Ys = g.Ys; p.Zs = g.Zs;
   p.Ye = p.Ys + 1;
   p.nzt = (p.Zs + 255) / 256;
-  p.Zt = round_up_d1((p.Zs + p.nzt - 1) / p.nzt, 16);
-  if (p.Zt > 256) { p.nzt += 1; p.Zt = round_up_d1((p.Zs + p.nzt - 1) / p.nzt, 16); }
+  p.Zt = round_up((p.Zs + p.nzt - 1) / p.nzt, 16);
+  if (p.Zt > 256) { p.nzt += 1; p.Zt = round_up((p.Zs + p.nzt - 1) / p.nzt, 16); }
   p.Yt = mx(1, mn(p.Ys, 512 / p.Zt));
   p.nyt = (p.Ys + p.Yt - 1) / p.Yt;
   p.rows = p.Yt * p.Zt;
@@ -483,32 +463,13 @@ int d1_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, 
       reinterpret_cast<const bf16 *>(big), E, elines, p.Xi, p.Yi, p.Zi, p.Ye, p.Zs);
   CG_LAUNCH_CHECK("d1_expand");
   CUtensorMap tmE, tmS;
-  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  {
-    const cuuint64_t gdim[5] = {8, (cuuint64_t)p.Zs, (cuuint64_t)p.Ye, (cuuint64_t)p.Xi, (cuuint64_t)p.B};
-    const cuuint64_t gstr[4] = {16, (cuuint64_t)p.Zs * 16, (cuuint64_t)p.Ye * p.Zs * 16, (cuuint64_t)p.Xi * p.Ye * p.Zs * 16};
-    const cuuint32_t box[5] = {8, (cuuint32_t)p.Zt, (cuuint32_t)p.Yt, 1, 1};
-    int r = encode_map_d1(&tmE, E, 5, gdim, gstr, box, estr);
-    if (r) return r;
-  }
-  {
-    const cuuint64_t gdim[5] = {8, (cuuint64_t)p.Zs, (cuuint64_t)p.Ys, (cuuint64_t)p.Xs, (cuuint64_t)p.B};
-    const cuuint64_t gstr[4] = {16, (cuuint64_t)p.Zs * 16, (cuuint64_t)p.Ys * p.Zs * 16, (cuuint64_t)p.Xs * p.Ys * p.Zs * 16};
-    const cuuint32_t box[5] = {8, (cuuint32_t)p.Zt, (cuuint32_t)p.Yt, 1, 1};
-    int r = encode_map_d1(&tmS, small, 5, gdim, gstr, box, estr);
-    if (r) return r;
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(d1_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitD1 + 1024);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(d1_wgrad_tc_kernel)");
-    attr_set = true;
-  }
+  int r = encode_act_map(&tmE, E, 8, p.Zs, p.Ye, p.Xi, p.B, 8, p.Zt, p.Yt, 1, 1, 0, "critic first layer, expanded input");
+  if (r) return r;
+  r = encode_act_map(&tmS, small, 8, p.Zs, p.Ys, p.Xs, p.B, 8, p.Zt, p.Yt, 1, 1, 0, "critic first layer, 8 channels");
+  if (r) return r;
   const long long total = (long long)p.B * p.Xs * p.nyt * p.nzt;
   const int grid = (int)mn<long long>(total, (long long)num_sms());
-  d1_wgrad_tc_kernel<<<grid, 192, p.smem_bytes + 1024, st>>>(tmE, tmS, dw, p);
-  CG_LAUNCH_CHECK("d1_wgrad_tc_kernel");
-  return 0;
+  return tc_launch<d1_wgrad_tc_kernel>("d1_wgrad_tc_kernel", grid, 192, p.smem_bytes + 1024, 1, st, tmE, tmS, dw, p);
 }
 
 // ============================================================================================================== scatter
@@ -679,7 +640,7 @@ static bool plan_d1_scatter(const cgan3d_conv_geom &g, D1ScatterPlan &best) {
       const int Yh = Yt + 1;
       const int mt = ((Yt - 1) * Zh + Zt + 127) / 128;
       if (mt > 4) break;
-      const int rows_alloc = round_up_d1(mx(Yh * Zh, mt * 128 + Zh + 2), 8);
+      const int rows_alloc = round_up(mx(Yh * Zh, mt * 128 + Zh + 2), 8);
       const uint32_t slot = (uint32_t)rows_alloc * 16;
       const int nslots = (int)mn<uint32_t>(8, (kSmemLimitD1 - 2048 - 512) / slot);
       if (nslots < 4) break;
@@ -713,25 +674,14 @@ static int run_d1_scatter(const cgan3d_conv_geom &g, const void *small, const vo
   d1_scatter_tiles_kernel<<<4, 256, 0, st>>>(reinterpret_cast<const bf16 *>(wp), wt);
   CG_LAUNCH_CHECK("d1_scatter_tiles");
   CUtensorMap tm;
-  const cuuint64_t gdim[5] = {8, (cuuint64_t)p.Zs, (cuuint64_t)p.Ys, (cuuint64_t)p.Xs, (cuuint64_t)p.B};
-  const cuuint64_t gstr[4] = {16, (cuuint64_t)p.Zs * 16, (cuuint64_t)p.Ys * p.Zs * 16, (cuuint64_t)p.Xs * p.Ys * p.Zs * 16};
-  const cuuint32_t box[5] = {8, (cuuint32_t)p.Zh, (cuuint32_t)p.Yh, 1, 1};
-  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  int r = encode_map_d1(&tm, small, 5, gdim, gstr, box, estr);
+  int r = encode_act_map(&tm, small, 8, p.Zs, p.Ys, p.Xs, p.B, 8, p.Zh, p.Yh, 1, 1, 0, "critic first layer");
   if (r) return r;
   const long long total = (long long)p.B * p.Xg * p.nyt * p.nzt;
   const int grid = (int)mn<long long>(total, (long long)num_sms());
   auto launch = [&](auto mt_tag) -> int {
     constexpr int MT = decltype(mt_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(d1_scatter_tc_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitD1 + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(d1_scatter_tc_kernel)");
-      attr_set = true;
-    }
-    d1_scatter_tc_kernel<MT><<<grid, 192, p.smem_bytes + 1024, st>>>(tm, wt, reinterpret_cast<bf16 *>(outp), p);
-    CG_LAUNCH_CHECK("d1_scatter_tc_kernel");
-    return 0;
+    return tc_launch<d1_scatter_tc_kernel<MT>>("d1_scatter_tc_kernel", grid, 192, p.smem_bytes + 1024, 1, st, tm, wt,
+                                               reinterpret_cast<bf16 *>(outp), p);
   };
   switch (p.mtiles) {
     case 1: return launch(std::integral_constant<int, 1>{});

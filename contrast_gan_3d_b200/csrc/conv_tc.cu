@@ -24,8 +24,6 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-
 struct TcPlan {
   int B, X, Y, Z, Cin, N;
   int Zt, nzt, Zh;
@@ -40,7 +38,7 @@ struct TcPlan {
 
 constexpr int kPlaneSlots = 3;
 constexpr int kThreads = 224;
-constexpr uint32_t kSmemLimit = 232448 - 1024;
+constexpr uint32_t kSmemLimit = kMaxDynSmem - 1024;
 
 // Work = ncols columns (b, z-tile, y-slab) x X output planes, flattened as idx = col * X + x.  CTA c owns the contiguous
 // range [c*total/grid, (c+1)*total/grid): at most one plane of imbalance; a range that crosses a column boundary is
@@ -691,17 +689,49 @@ __global__ void repack_b_kernel(const bf16 *__restrict__ wp, bf16 *__restrict__ 
 
 // ---------------------------------------------------------------- host side
 EncodeTiledFn tc_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  static bool tried = false;
-  if (!tried) {
-    tried = true;
+  static const EncodeTiledFn fn = [] {
     void *p = nullptr;
     cudaDriverEntryPointQueryResult qres;
     if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
         qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
+      return reinterpret_cast<EncodeTiledFn>(p);
+    return EncodeTiledFn{nullptr};
+  }();
   return fn;
+}
+
+int encode_tiled(CUtensorMap *tm, CUtensorMapDataType dtype, int rank, const void *ptr, const cuuint64_t *gdim,
+                 const cuuint64_t *gstr, const cuuint32_t *box, const cuuint32_t *estr, CUtensorMapSwizzle swizzle,
+                 const char *what) {
+  EncodeTiledFn enc = tc_encode_fn();
+  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
+  const cuuint32_t ones[5] = {1, 1, 1, 1, 1};
+  CUresult r = enc(tm, dtype, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr ? estr : ones,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (%s) failed with %d", what, (int)r);
+  return 0;
+}
+
+int encode_weight_rows(CUtensorMap *tm, const void *ptr, int nrows, int box_rows) {
+  const cuuint64_t gdim[2] = {64, (cuuint64_t)nrows};
+  const cuuint64_t gstr[1] = {256};
+  const cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
+  return encode_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, ptr, gdim, gstr, box, nullptr, CU_TENSOR_MAP_SWIZZLE_NONE,
+                      "weight rows");
+}
+
+int encode_act_map(CUtensorMap *tm, const void *ptr, int C, int Z, int Y, int X, int B, int box_c, int nz, int ny, int ez,
+                   int ey, int swizzle_bytes, const char *what) {
+  const cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)B};
+  const cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2, (cuuint64_t)X * Y * Z * C * 2};
+  // a box spans ez * (nz - 1) + 1 voxels along z, of which TMA loads every ez-th (likewise along y)
+  const cuuint32_t box[5] = {(cuuint32_t)box_c, (cuuint32_t)(ez * (nz - 1) + 1), (cuuint32_t)(ey * (ny - 1) + 1), 1, 1};
+  const cuuint32_t estr[5] = {1, (cuuint32_t)ez, (cuuint32_t)ey, 1, 1};
+  const CUtensorMapSwizzle swz = swizzle_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
+                                 : swizzle_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B
+                                 : swizzle_bytes == 32 ? CU_TENSOR_MAP_SWIZZLE_32B
+                                                       : CU_TENSOR_MAP_SWIZZLE_NONE;
+  return encode_tiled(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, ptr, gdim, gstr, box, estr, swz, what);
 }
 
 // CTA pairs need whole-voxel swizzled planes (one TMA box per plane), N/2 a multiple of 16 and 256-byte weight-map rows.
@@ -841,8 +871,6 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
   if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 31) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 conv: input / workspace must be 16-byte aligned, the output 32-byte aligned (256-bit stores)");
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   bf16 *wb = reinterpret_cast<bf16 *>(ws);
   TcPlan ps;
   const bool stack = plan_s1_stack(g.B, g.Xb, g.Yb, g.Zb, Cin, N, ps) && !(bn_sums && N > 64);
@@ -855,24 +883,12 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
     CG_LAUNCH_CHECK("repack_b");
   }
   CUtensorMap tm;
-  const cuuint64_t gdim[5] = {(cuuint64_t)Cin, (cuuint64_t)p.Z, (cuuint64_t)p.Y, (cuuint64_t)p.X, (cuuint64_t)p.B};
-  const cuuint64_t gstr[4] = {(cuuint64_t)Cin * 2, (cuuint64_t)p.Z * Cin * 2, (cuuint64_t)p.Y * p.Z * Cin * 2,
-                              (cuuint64_t)p.X * p.Y * p.Z * Cin * 2};
-  const cuuint32_t box[5] = {(cuuint32_t)(p.a_swz ? Cin : 8), (cuuint32_t)p.Zh, (cuuint32_t)p.Yh, 1, 1};
-  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  const CUtensorMapSwizzle swz = p.a_swz == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                 : (p.a_swz == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : (p.a_swz == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE));
-  CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(in), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled failed with %d", (int)r);
+  int r = encode_act_map(&tm, in, Cin, p.Z, p.Y, p.X, p.B, p.a_swz ? Cin : 8, p.Zh, p.Yh, 1, 1, p.a_swz, "stride-1 conv");
+  if (r) return r;
   CUtensorMap tmw{};
-  if (p.pair) {  // the repacked weights as rows of 256 bytes: one (tap, half) tile is btile_bytes / 256 rows
-    const cuuint64_t wdim[2] = {64, (cuuint64_t)(27 * 2) * (p.btile_bytes >> 8)};
-    const cuuint64_t wstr[1] = {256};
-    const cuuint32_t wbox[2] = {64, (cuuint32_t)(p.btile_bytes >> 8)};
-    r = enc(&tmw, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wb, wdim, wstr, wbox, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (weights) failed with %d", (int)r);
+  if (p.pair) {  // one (tap, half) tile is btile_bytes / 256 weight rows
+    r = encode_weight_rows(&tmw, wb, 27 * 2 * (int)(p.btile_bytes >> 8), (int)(p.btile_bytes >> 8));
+    if (r) return r;
   }
   const long long work = (long long)(p.pair ? (p.nitems + 1) / 2 : p.nitems) * p.X;
   const int grid = p.pair ? 2 * (int)mn<long long>(work, (long long)(num_sms() / 2)) : (int)mn<long long>(work, (long long)num_sms());
@@ -882,28 +898,8 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
       constexpr int KS = decltype(ks_tag)::value;
       constexpr int MT = decltype(mt_tag)::value;
       constexpr bool ST = decltype(st_tag)::value;
-      static bool attr_set = false;
-      if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(conv_s1_stack_kernel<KS, MT, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimit + 1024);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv_s1_stack_kernel)");
-        attr_set = true;
-      }
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3((unsigned)grid);
-      cfg.blockDim = dim3(kStackThreads);
-      cfg.dynamicSmemBytes = p.smem_bytes + 1024;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 2;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      cudaError_t e = cudaLaunchKernelEx(&cfg, conv_s1_stack_kernel<KS, MT, ST>, tm, tmw, reinterpret_cast<bf16 *>(outp), p, bn_sums);
-      if (e != cudaSuccess) return cuda_fail(e, "conv_s1_stack_kernel launch");
-      CG_LAUNCH_CHECK("conv_s1_stack_kernel");
-      return 0;
+      return tc_launch<conv_s1_stack_kernel<KS, MT, ST>>("conv_s1_stack_kernel", grid, kStackThreads, p.smem_bytes + 1024, 2, st, tm,
+                                                         tmw, reinterpret_cast<bf16 *>(outp), p, bn_sums);
     };
     auto by_st = [&](auto ks_tag, auto mt_tag) -> int {
       return bn_sums ? launch_k(ks_tag, mt_tag, std::true_type{}) : launch_k(ks_tag, mt_tag, std::false_type{});
@@ -923,30 +919,8 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
     constexpr int MT = decltype(mt_tag)::value;
     constexpr bool ST = decltype(st_tag)::value;
     constexpr bool PR = decltype(pair_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv_s1_tc_kernel<KS, MT, ST, PR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)kSmemLimit + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv_s1_tc_kernel)");
-      attr_set = true;
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = p.smem_bytes + 1024;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = PR ? 2 : 1;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, conv_s1_tc_kernel<KS, MT, ST, PR>, tm, tmw, (const bf16 *)wb, reinterpret_cast<bf16 *>(outp), p,
-                                       bn_sums);
-    if (e != cudaSuccess) return cuda_fail(e, "conv_s1_tc_kernel launch");
-    CG_LAUNCH_CHECK("conv_s1_tc_kernel");
-    return 0;
+    return tc_launch<conv_s1_tc_kernel<KS, MT, ST, PR>>("conv_s1_tc_kernel", grid, kThreads, p.smem_bytes + 1024, PR ? 2 : 1, st, tm, tmw,
+                                                        (const bf16 *)wb, reinterpret_cast<bf16 *>(outp), p, bn_sums);
   };
   auto launch = [&](auto ks_tag, auto mt_tag) -> int {
     if (p.pair) {

@@ -354,32 +354,22 @@ int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const vo
   if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 strided conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 strided conv: pointers must be 16-byte aligned");
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
   // input tensor: gather reads the big side with element strides 2 on z and y; scatter reads the small side densely
   const int Xi = scatter ? g.Xs : g.Xb, Yi = scatter ? g.Ys : g.Yb, Zi = scatter ? g.Zs : g.Zb, Ci = p.Cin;
   if ((reinterpret_cast<uintptr_t>(outp) & 15) || (p.Nout * 2) % 16 || (p.out_pitch * 2) % 16) return fail(CGAN3D_E_ARG, "tcgen05 strided conv: output rows must be 16-byte aligned");
   const int es = p.in_scale;
   CUtensorMap tm;
   // z-pair gather: the innermost dimension is a PAIR of z-adjacent voxels (dense along z, element stride 2 only on y)
-  const cuuint64_t zp = p.zpair ? 2 : 1;
-  const cuuint64_t gdim[5] = {(cuuint64_t)Ci * zp, (cuuint64_t)Zi / zp, (cuuint64_t)Yi, (cuuint64_t)Xi, (cuuint64_t)g.B};
-  const cuuint64_t gstr[4] = {(cuuint64_t)Ci * 2 * zp, (cuuint64_t)Zi * Ci * 2, (cuuint64_t)Yi * Zi * Ci * 2,
-                              (cuuint64_t)Xi * Yi * Zi * Ci * 2};
-  const cuuint32_t box[5] = {(cuuint32_t)(p.a_swz ? Ci * (int)zp : 8), (cuuint32_t)(p.zpair ? p.Zh : es * (p.Zh - 1) + 1),
-                             (cuuint32_t)(es * (p.Yh - 1) + 1), 1, 1};
-  const cuuint32_t estr[5] = {1, (cuuint32_t)(p.zpair ? 1 : es), (cuuint32_t)es, 1, 1};
-  const CUtensorMapSwizzle swz = p.a_swz == 128 ? CU_TENSOR_MAP_SWIZZLE_128B
-                                 : (p.a_swz == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : (p.a_swz == 32 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_NONE));
-  CUresult r = enc(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(in), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (strided) failed with %d", (int)r);
+  const int zp = p.zpair ? 2 : 1;
+  int r = encode_act_map(&tm, in, Ci * zp, Zi / zp, Yi, Xi, g.B, p.a_swz ? Ci * zp : 8, p.Zh, p.Yh, p.zpair ? 1 : es, es, p.a_swz,
+                         "strided conv");
+  if (r) return r;
   const long long total = (long long)p.B * p.nzt * p.nslabs * p.Xg;
   const int grid = p.pair ? 2 * (int)mn<long long>((total + 1) / 2, (long long)(num_sms() / 2)) : (int)mn<long long>(total, (long long)num_sms());
   if (bn_sums && p.Nout > 64) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 strided conv: fused BatchNorm statistics need <= 64 channels per launch");
   ProgLaunchArgs la{};
   la.tm = tm; la.g = g; la.scatter = scatter; la.nsplit = nsplit; la.grid = grid; la.wp = wp; la.outp = outp; la.ws = ws;
-  la.part_bytes = part_bytes; la.bn_sums = bn_sums; la.st = st; la.enc = enc;
+  la.part_bytes = part_bytes; la.bn_sums = bn_sums; la.st = st;
   switch (p.paired ? 1 : (p.Cin >> 4)) {
     case 1: return prog_launch_ks<1>(p, la);
     case 2: return prog_launch_ks<2>(p, la);

@@ -30,10 +30,8 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-
 constexpr int kMaxEntries = 16, kMaxTaps = 64;
-constexpr uint32_t kSmemLimitProg = 232448 - 1024;
+constexpr uint32_t kSmemLimitProg = kMaxDynSmem - 1024;
 
 struct ProgTap {
   uint16_t row_shift;  // rows (16 B units) added to the A descriptor start
@@ -390,7 +388,6 @@ struct ProgLaunchArgs {
   size_t part_bytes;
   double *bn_sums;
   cudaStream_t st;
-  EncodeTiledFn enc;
 };
 
 template <int KS_>
@@ -403,49 +400,22 @@ int prog_launch_ks(ProgPlan &p, const ProgLaunchArgs &a) {
   const size_t part_bytes = a.part_bytes;
   double *bn_sums = a.bn_sums;
   cudaStream_t st = a.st;
-  EncodeTiledFn enc = a.enc;
   auto launch_s = [&](auto ks_tag, auto mt_tag, auto st_tag, auto pair_tag) -> int {
     constexpr int KS = decltype(ks_tag)::value;
     constexpr int MT = decltype(mt_tag)::value;
     constexpr int ST = decltype(st_tag)::value;
     constexpr bool PR = decltype(pair_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv_prog_tc_kernel<KS, MT, ST, PR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)kSmemLimitProg + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv_prog_tc_kernel)");
-      attr_set = true;
-    }
     for (int part = 0; part < nsplit; ++part) {  // output-channel parts (1 unless the filters exceed shared memory)
       p.out_c0 = part * p.Nout;
       bf16 *wb = reinterpret_cast<bf16 *>(reinterpret_cast<uint8_t *>(ws) + part * part_bytes);
       if (int rr = repack_prog_launch(reinterpret_cast<const bf16 *>(wp), wb, g.Cb, g.Cs, scatter, p, st)) return rr;
       CUtensorMap tmw{};
       if (PR) {  // the repacked half tiles as rows of 256 bytes
-        const cuuint64_t wdim[2] = {64, (cuuint64_t)2 * p.nbt * (p.btile_bytes >> 8)};
-        const cuuint64_t wstr[1] = {256};
-        const cuuint32_t wbox[2] = {64, (cuuint32_t)(p.btile_bytes >> 8)};
-        const cuuint32_t we[2] = {1, 1};
-        CUresult rw = enc(&tmw, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wb, wdim, wstr, wbox, we, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (rw != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (strided, filters) failed with %d", (int)rw);
+        if (int rw = encode_weight_rows(&tmw, wb, 2 * p.nbt * (int)(p.btile_bytes >> 8), (int)(p.btile_bytes >> 8))) return rw;
       }
-      cudaLaunchConfig_t cfg{};
-      cfg.gridDim = dim3((unsigned)grid);
-      cfg.blockDim = dim3(192);
-      cfg.dynamicSmemBytes = p.smem_bytes + 1024;
-      cfg.stream = st;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = PR ? 2 : 1;
-      attr[0].val.clusterDim.y = 1;
-      attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      cudaError_t e = cudaLaunchKernelEx(&cfg, conv_prog_tc_kernel<KS, MT, ST, PR>, tm, tmw, (const bf16 *)wb, reinterpret_cast<bf16 *>(outp), p,
-                                         bn_sums);
-      if (e != cudaSuccess) return cuda_fail(e, "conv_prog_tc_kernel launch");
-      CG_LAUNCH_CHECK("conv_prog_tc_kernel");
+      if (int rl = tc_launch<conv_prog_tc_kernel<KS, MT, ST, PR>>("conv_prog_tc_kernel", grid, 192, p.smem_bytes + 1024, PR ? 2 : 1, st,
+                                                                 tm, tmw, (const bf16 *)wb, reinterpret_cast<bf16 *>(outp), p, bn_sums))
+        return rl;
     }
     return 0;
   };

@@ -20,9 +20,7 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-
-constexpr uint32_t kSmemLimitThin = 232448 - 1024;
+constexpr uint32_t kSmemLimitThin = kMaxDynSmem - 1024;
 constexpr int kTapTilesA = 49;
 constexpr int kZbA = 8;                  // output z per work item
 constexpr uint32_t kTileBytesA = 4096;  // [2 z-chunks][128 n = 8 z x 16 ch][8 z] bf16
@@ -729,31 +727,6 @@ expand_z_kernel(const bf16 *__restrict__ q, bf16 *__restrict__ e, long long line
 }
 
 // ---------------------------------------------------------------- host side
-static int encode_map(CUtensorMap *tm, const void *ptr, int rank, const cuuint64_t *gdim, const cuuint64_t *gstr,
-                      const cuuint32_t *box, CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_NONE) {
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
-  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (thin conv) failed with %d", (int)r);
-  return 0;
-}
-
-// un-swizzled map of an arbitrary element type (weight tiles viewed as rows of 256 bytes)
-static int encode_map_raw(CUtensorMap *tm, const void *ptr, CUtensorMapDataType dt, int rank, const cuuint64_t *gdim, const cuuint64_t *gstr,
-                          const cuuint32_t *box) {
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
-  const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = enc(tm, dt, (cuuint32_t)rank, const_cast<void *>(ptr), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (weight tiles) failed with %d", (int)r);
-  return 0;
-}
-
-static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
-
 // op 0: gather with Cb == 1, Cs == 16 (valid conv, P = pad);  op 1: scatter with Cb == 16, Cs == 1 (P = 6 - pad)
 static bool thin_a_shape(const cgan3d_conv_geom &g, int op) {
   if (g.k != 7 || g.stride != 1) return false;
@@ -888,46 +861,23 @@ static int run_thin_a(const cgan3d_conv_geom &g, int op, const void *in, const v
   shifted_copies_kernel<<<(unsigned)((rows + 7) / 8), 256, (size_t)8 * ((p.Zc + 24 + 7) & ~7) * 2, st>>>(
       reinterpret_cast<const bf16 *>(in), rp, rows, p.Zi, p.Zc, p.zshift);
   CG_LAUNCH_CHECK("shifted_copies");
-  CUtensorMap tm;
+  CUtensorMap tm;  // the two shifted copies [2][B][Xi][Yi][Zc]
   const cuuint64_t zc = (cuuint64_t)p.Zc;
   const cuuint64_t gdim[5] = {zc, (cuuint64_t)p.Yi, (cuuint64_t)p.Xi, (cuuint64_t)p.B, 2};
   const cuuint64_t gstr[4] = {zc * 2, (cuuint64_t)p.Yi * zc * 2, (cuuint64_t)p.Xi * p.Yi * zc * 2, (cuuint64_t)rows * zc * 2};
   const cuuint32_t box[5] = {16, (cuuint32_t)p.Yh, (cuuint32_t)p.Xh, 1, 1};
-  int r = encode_map(&tm, rp, 5, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_32B);
+  int r = encode_tiled(&tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, rp, gdim, gstr, box, nullptr, CU_TENSOR_MAP_SWIZZLE_32B, "thin conv");
   if (r) return r;
-  CUtensorMap tmw;  // the Toeplitz tiles as rows of 256 bytes: 392 rows per CTA half, loaded as two boxes of 49 KB
-  const cuuint64_t wdim[2] = {64, (cuuint64_t)(kTapTilesA * kTileBytesA / 256)};
-  const cuuint64_t wstr[1] = {256};
-  const cuuint32_t wbox[2] = {64, 196};
-  r = encode_map_raw(&tmw, wt, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wdim, wstr, wbox);
+  CUtensorMap tmw;  // the Toeplitz tiles: 392 weight rows per CTA half, loaded as two boxes of 49 KB
+  r = encode_weight_rows(&tmw, wt, kTapTilesA * kTileBytesA / 256, 196);
   if (r) return r;
   const long long total = (long long)p.B * p.nxt * p.nyt * p.nzb;
   const int grid = 2 * (int)mn<long long>((total + 1) / 2, (long long)(num_sms() / 2));
   auto launch = [&](auto mt_tag, auto st_tag) -> int {
     constexpr int MT = decltype(mt_tag)::value;
     constexpr bool ST = decltype(st_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv7_c1_tc_kernel<MT, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv7_c1_tc_kernel)");
-      attr_set = true;
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(192);
-    cfg.dynamicSmemBytes = p.smem_bytes + 1024;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_c1_tc_kernel<MT, ST>, tm, tmw, reinterpret_cast<bf16 *>(outp), p, bn_sums);
-    if (e != cudaSuccess) return cuda_fail(e, "conv7_c1_tc_kernel launch");
-    CG_LAUNCH_CHECK("conv7_c1_tc_kernel");
-    return 0;
+    return tc_launch<conv7_c1_tc_kernel<MT, ST>>("conv7_c1_tc_kernel", grid, 192, p.smem_bytes + 1024, 2, st, tm, tmw,
+                                                 reinterpret_cast<bf16 *>(outp), p, bn_sums);
   };
   if (p.mtiles == 1) return bn_sums ? launch(std::integral_constant<int, 1>{}, std::true_type{}) : launch(std::integral_constant<int, 1>{}, std::false_type{});
   if (p.mtiles == 2) return bn_sums ? launch(std::integral_constant<int, 2>{}, std::true_type{}) : launch(std::integral_constant<int, 2>{}, std::false_type{});
@@ -946,44 +896,18 @@ static int run_thin_b(const cgan3d_conv_geom &g, int op, const void *in, const v
   stack_b_kernel<<<28, 256, 0, st>>>(reinterpret_cast<const bf16 *>(wp), wt, op);
   CG_LAUNCH_CHECK("stack_b");
   CUtensorMap tm;
-  const cuuint64_t gdim[5] = {16, (cuuint64_t)p.Zi, (cuuint64_t)p.Yi, (cuuint64_t)p.Xi, (cuuint64_t)p.B};
-  const cuuint64_t gstr[4] = {32, (cuuint64_t)p.Zi * 32, (cuuint64_t)p.Yi * p.Zi * 32, (cuuint64_t)p.Xi * p.Yi * p.Zi * 32};
-  const cuuint32_t box[5] = {16, (cuuint32_t)p.Zh, (cuuint32_t)p.Yh, 1, 1};
-  int r = encode_map(&tm, in, 5, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_32B);
+  int r = encode_act_map(&tm, in, 16, p.Zi, p.Yi, p.Xi, p.B, 16, p.Zh, p.Yh, 1, 1, 32, "thin conv");
   if (r) return r;
-  CUtensorMap tmw;  // the 7 filter tiles as rows of 256 bytes (8 rows per tile, 4 per CTA half)
-  const cuuint64_t wdim[2] = {64, (cuuint64_t)(kTapTilesB * kTileBytesB / 256)};
-  const cuuint64_t wstr[1] = {256};
-  const cuuint32_t wbox[2] = {64, 4};
-  r = encode_map_raw(&tmw, wt, CU_TENSOR_MAP_DATA_TYPE_INT32, 2, wdim, wstr, wbox);
+  CUtensorMap tmw;  // the 7 filter tiles: 8 weight rows per tile, 4 per CTA half
+  r = encode_weight_rows(&tmw, wt, kTapTilesB * kTileBytesB / 256, 4);
   if (r) return r;
   const long long ncols = (long long)p.B * p.nyt * p.nzt;
   const long long total = (ncols + 1) / 2 * p.Xo;
   const int grid = 2 * (int)mn<long long>(total, (long long)(num_sms() / 2));
   auto launch = [&](auto mt_tag) -> int {
     constexpr int MT = decltype(mt_tag)::value;
-    static bool attr_set = false;
-    if (!attr_set) {
-      cudaError_t e = cudaFuncSetAttribute(conv7_to1_tc_kernel<MT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
-      if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(conv7_to1_tc_kernel)");
-      attr_set = true;
-    }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(320);
-    cfg.dynamicSmemBytes = p.smem_bytes + 1024;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, conv7_to1_tc_kernel<MT>, tm, tmw, reinterpret_cast<bf16 *>(outp), p);
-    if (e != cudaSuccess) return cuda_fail(e, "conv7_to1_tc_kernel launch");
-    CG_LAUNCH_CHECK("conv7_to1_tc_kernel");
-    return 0;
+    return tc_launch<conv7_to1_tc_kernel<MT>>("conv7_to1_tc_kernel", grid, 320, p.smem_bytes + 1024, 2, st, tm, tmw,
+                                              reinterpret_cast<bf16 *>(outp), p);
   };
   switch (p.mtiles) {
     case 1: return launch(std::integral_constant<int, 1>{});
@@ -1048,31 +972,13 @@ int thin_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small
       reinterpret_cast<const bf16 *>(q1), E, elines, Xq, Yq, Zq, p.Xe, p.Ye, p.Zs, p.P);
   CG_LAUNCH_CHECK("expand_z");
   CUtensorMap tmE, tmS;
-  {
-    const cuuint64_t gdim[5] = {8, (cuuint64_t)p.Zs, (cuuint64_t)p.Ye, (cuuint64_t)p.Xe, (cuuint64_t)p.B};
-    const cuuint64_t gstr[4] = {16, (cuuint64_t)p.Zs * 16, (cuuint64_t)p.Ye * p.Zs * 16, (cuuint64_t)p.Xe * p.Ye * p.Zs * 16};
-    const cuuint32_t box[5] = {8, (cuuint32_t)p.Zt, (cuuint32_t)(p.Yt + 7), 1, 1};
-    int r = encode_map(&tmE, E, 5, gdim, gstr, box);
-    if (r) return r;
-  }
-  {
-    const cuuint64_t gdim[5] = {16, (cuuint64_t)p.Zs, (cuuint64_t)p.Ys, (cuuint64_t)p.Xs, (cuuint64_t)p.B};
-    const cuuint64_t gstr[4] = {32, (cuuint64_t)p.Zs * 32, (cuuint64_t)p.Ys * p.Zs * 32, (cuuint64_t)p.Xs * p.Ys * p.Zs * 32};
-    const cuuint32_t box[5] = {16, (cuuint32_t)p.Zt, (cuuint32_t)p.Yt, 1, 1};
-    int r = encode_map(&tmS, s16, 5, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_32B);
-    if (r) return r;
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad7_thin_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitThin + 1024);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(wgrad7_thin_tc_kernel)");
-    attr_set = true;
-  }
+  int r = encode_act_map(&tmE, E, 8, p.Zs, p.Ye, p.Xe, p.B, 8, p.Zt, p.Yt + 7, 1, 1, 0, "thin wgrad, expanded input");
+  if (r) return r;
+  r = encode_act_map(&tmS, s16, 16, p.Zs, p.Ys, p.Xs, p.B, 16, p.Zt, p.Yt, 1, 1, 32, "thin wgrad, 16 channels");
+  if (r) return r;
   const long long total = (long long)p.B * p.nyt * p.nzt * p.Xe;
   const int grid = (int)mn<long long>(total, (long long)num_sms());
-  wgrad7_thin_tc_kernel<<<grid, 192, p.smem_bytes + 1024, st>>>(tmE, tmS, dw, p);
-  CG_LAUNCH_CHECK("wgrad7_thin_tc_kernel");
-  return 0;
+  return tc_launch<wgrad7_thin_tc_kernel>("wgrad7_thin_tc_kernel", grid, 192, p.smem_bytes + 1024, 1, st, tmE, tmS, dw, p);
 }
 
 bool thin_fuses_bnstats(const cgan3d_conv_geom &g, int op) { return op == 0 && thin_a_shape(g, 0); }

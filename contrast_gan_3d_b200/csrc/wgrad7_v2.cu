@@ -30,8 +30,7 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-constexpr uint32_t kSmemLimitW2 = 232448 - 1024;
+constexpr uint32_t kSmemLimitW2 = kMaxDynSmem - 1024;
 constexpr int kMaxRingW2 = 14;  // logical S16 plane slots: 8 live + 4 or 6 in flight (TMA runs 2 - 3 steps ahead of the MMAs)
 constexpr int kMaxPrefW2 = 11;     // staged 32-bit words per fetch thread and step
 constexpr int kBuildWarpsW2 = 10;  // warps 0-3 (also the epilogue) and 6-11 expand the operand
@@ -549,37 +548,17 @@ int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, f
     cudaError_t e = cudaMemsetAsync(dw, 0, (size_t)16 * 343 * sizeof(float), st);
     if (e != cudaSuccess) return cuda_fail(e, "tcgen05 thin wgrad v2 memset");
   }
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
-  CUtensorMap tmS;
-  {
-    // rows of one voxel (16 channels, 32 B) or of a z-adjacent voxel pair (64 B)
-    const cuuint64_t vox = p.zp ? 2 : 1;
-    const cuuint64_t gdim[5] = {16 * vox, (cuuint64_t)p.Zs / vox, (cuuint64_t)p.Ys, (cuuint64_t)p.Xs, (cuuint64_t)p.B};
-    const cuuint64_t gstr[4] = {32 * vox, (cuuint64_t)p.Zs * 32, (cuuint64_t)p.Ys * p.Zs * 32, (cuuint64_t)p.Xs * p.Ys * p.Zs * 32};
-    const cuuint32_t box[5] = {(cuuint32_t)(16 * vox), (cuuint32_t)p.zr, (cuuint32_t)p.Yt, 1, 1};
-    const cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-    CUresult r = enc(&tmS, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(s16), gdim, gstr, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, p.zp ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B,
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (thin wgrad v2) failed with %d", (int)r);
-  }
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad7_v2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitW2 + 1024);
-    if (e == cudaSuccess)
-      e = cudaFuncSetAttribute(wgrad7_v2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitW2 + 1024);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(wgrad7_v2_kernel)");
-    attr_set = true;
-  }
+  CUtensorMap tmS;  // rows of one voxel (16 channels, 32 B) or of a z-adjacent voxel pair (64 B)
+  const int vox = p.zp ? 2 : 1;
+  const int r = encode_act_map(&tmS, s16, 16 * vox, p.Zs / vox, p.Ys, p.Xs, p.B, 16 * vox, p.zr, p.Yt, 1, 1, 32 * vox, "thin wgrad v2");
+  if (r) return r;
   const long long total = (long long)p.B * p.nyt * p.npairs;
   const int grid = (int)mn<long long>(total, (long long)num_sms());
   if (p.zp)
-    wgrad7_v2_kernel<true><<<grid, kThreadsW2, p.smem_bytes + 1024, st>>>(tmS, reinterpret_cast<const uint32_t *>(q1), dw, p);
-  else
-    wgrad7_v2_kernel<false><<<grid, kThreadsW2, p.smem_bytes + 1024, st>>>(tmS, reinterpret_cast<const uint32_t *>(q1), dw, p);
-  CG_LAUNCH_CHECK("wgrad7_v2_kernel");
-  return 0;
+    return tc_launch<wgrad7_v2_kernel<true>>("wgrad7_v2_kernel", grid, kThreadsW2, p.smem_bytes + 1024, 1, st, tmS,
+                                             reinterpret_cast<const uint32_t *>(q1), dw, p);
+  return tc_launch<wgrad7_v2_kernel<false>>("wgrad7_v2_kernel", grid, kThreadsW2, p.smem_bytes + 1024, 1, st, tmS,
+                                            reinterpret_cast<const uint32_t *>(q1), dw, p);
 }
 
 }  // namespace cg

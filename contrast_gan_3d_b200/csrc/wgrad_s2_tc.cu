@@ -24,8 +24,7 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-constexpr uint32_t kSmemLimitWs = 232448 - 2048;
+constexpr uint32_t kSmemLimitWs = kMaxDynSmem - 2048;
 constexpr int kMaxWsMma = 4;
 
 struct WsPlan {
@@ -286,20 +285,6 @@ static bool plan_ws(const cgan3d_conv_geom &g, WsPlan &p) {
   return true;
 }
 
-static int encode_voxel_map(CUtensorMap *tm, const void *ptr, int C, int Z, int Y, int X, int B, int nz, int ny, int es) {
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
-  const cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)B};
-  const cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2, (cuuint64_t)X * Y * Z * C * 2};
-  const cuuint32_t box[5] = {(cuuint32_t)C, (cuuint32_t)(es * (nz - 1) + 1), (cuuint32_t)(es * (ny - 1) + 1), 1, 1};
-  const cuuint32_t estr[5] = {1, (cuuint32_t)es, (cuuint32_t)es, 1, 1};
-  const CUtensorMapSwizzle swz = C * 2 == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : (C * 2 == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B);
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled (strided wgrad) failed with %d", (int)r);
-  return 0;
-}
-
 bool tc_wgrad_s2_supported(const cgan3d_conv_geom &g) {
   WsPlan p;
   return plan_ws(g, p);
@@ -314,21 +299,13 @@ int tc_wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *smal
     cudaError_t e = cudaMemsetAsync(dw, 0, (size_t)g.Cs * g.Cb * p.taps * sizeof(float), st);
     if (e != cudaSuccess) return cuda_fail(e, "tcgen05 strided wgrad memset");
   }
-  CUtensorMap tmY, tmX;
-  int r = encode_voxel_map(&tmY, small, g.Cs, g.Zs, g.Ys, g.Xs, g.B, p.Zh, p.Yt, 1);
+  CUtensorMap tmY, tmX;  // whole voxels, swizzled by the row width
+  int r = encode_act_map(&tmY, small, g.Cs, g.Zs, g.Ys, g.Xs, g.B, g.Cs, p.Zh, p.Yt, 1, 1, 2 * g.Cs, "strided wgrad, small side");
   if (r) return r;
-  r = encode_voxel_map(&tmX, big, g.Cb, g.Zb, g.Yb, g.Xb, g.B, p.Zh, p.Yh, g.stride);
+  r = encode_act_map(&tmX, big, g.Cb, g.Zb, g.Yb, g.Xb, g.B, g.Cb, p.Zh, p.Yh, g.stride, g.stride, 2 * g.Cb, "strided wgrad, big side");
   if (r) return r;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad_s2_sw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitWs + 2048);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(wgrad_s2_sw_kernel)");
-    attr_set = true;
-  }
   const int grid = (int)mn<long long>((long long)p.k * p.steps_per_dx, (long long)(num_sms() / p.k) * p.k);
-  wgrad_s2_sw_kernel<<<grid, 192, p.smem_bytes, st>>>(tmY, tmX, dw, p);
-  CG_LAUNCH_CHECK("wgrad_s2_sw_kernel");
-  return 0;
+  return tc_launch<wgrad_s2_sw_kernel>("wgrad_s2_sw_kernel", grid, 192, p.smem_bytes, 1, st, tmY, tmX, dw, p);
 }
 
 }  // namespace cg

@@ -20,8 +20,7 @@
 
 namespace cg {
 
-using bf16 = __nv_bfloat16;
-constexpr uint32_t kSmemLimitWg = 232448 - 1024;
+constexpr uint32_t kSmemLimitWg = kMaxDynSmem - 1024;
 constexpr int kMaxWgMma = 16, kMaxWgSrc = 4;
 
 struct WgMma {
@@ -278,20 +277,6 @@ static bool plan_wgrad(const cgan3d_conv_geom &g, WgPlan &p) {
   return true;
 }
 
-static int encode_act_map(CUtensorMap *tm, const void *ptr, int C, int Z, int Y, int X, int B, int nz, int ny, int es) {
-  EncodeTiledFn enc = tc_encode_fn();
-  if (!enc) return fail(CGAN3D_E_UNSUPPORTED, "cuTensorMapEncodeTiled not available");
-  const cuuint64_t gdim[5] = {(cuuint64_t)C, (cuuint64_t)Z, (cuuint64_t)Y, (cuuint64_t)X, (cuuint64_t)B};
-  const cuuint64_t gstr[4] = {(cuuint64_t)C * 2, (cuuint64_t)Z * C * 2, (cuuint64_t)Y * Z * C * 2, (cuuint64_t)X * Y * Z * C * 2};
-  const cuuint32_t box[5] = {8, (cuuint32_t)(es * (nz - 1) + 1), (cuuint32_t)(es * (ny - 1) + 1), 1, 1};
-  const cuuint32_t estr[5] = {1, (cuuint32_t)es, (cuuint32_t)es, 1, 1};
-  CUresult r = enc(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, const_cast<void *>(ptr), gdim, gstr, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return fail(CGAN3D_E_SHAPE, "cuTensorMapEncodeTiled failed with %d", (int)r);
-  return 0;
-}
-
 bool tc_wgrad_supported(const cgan3d_conv_geom &g) {
   WgPlan p;
   return plan_wgrad(g, p);
@@ -307,20 +292,12 @@ int tc_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, 
     if (e != cudaSuccess) return cuda_fail(e, "tcgen05 wgrad memset");
   }
   CUtensorMap tmY, tmX;
-  int r = encode_act_map(&tmY, small, g.Cs, g.Zs, g.Ys, g.Xs, g.B, p.Zh, p.Yt, 1);
+  int r = encode_act_map(&tmY, small, g.Cs, g.Zs, g.Ys, g.Xs, g.B, 8, p.Zh, p.Yt, 1, 1, 0, "wgrad, small side");
   if (r) return r;
-  r = encode_act_map(&tmX, big, g.Cb, g.Zb, g.Yb, g.Xb, g.B, p.Zh, p.Yh, g.stride);
+  r = encode_act_map(&tmX, big, g.Cb, g.Zb, g.Yb, g.Xb, g.B, 8, p.Zh, p.Yh, g.stride, g.stride, 0, "wgrad, big side");
   if (r) return r;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad_prog_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemLimitWg + 1024);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(wgrad_prog_tc_kernel)");
-    attr_set = true;
-  }
   const int grid = (int)mn<long long>((long long)p.k * p.steps_per_dx, (long long)(num_sms() / p.k) * p.k);
-  wgrad_prog_tc_kernel<<<grid, 192, p.smem_bytes + 1024, st>>>(tmY, tmX, dw, p);
-  CG_LAUNCH_CHECK("wgrad_prog_tc_kernel");
-  return 0;
+  return tc_launch<wgrad_prog_tc_kernel>("wgrad_prog_tc_kernel", grid, 192, p.smem_bytes + 1024, 1, st, tmY, tmX, dw, p);
 }
 
 }  // namespace cg
