@@ -25,6 +25,16 @@ class ConvGeom(C.Structure):
         return tuple(getattr(self, n) for n, _ in self._fields_)
 
 
+BORDER_CONSTANT, BORDER_NEAREST = 0, 1
+SPATIAL_TRANSFORM, SPATIAL_ELASTIC = 1, 2
+
+
+class SpatialParams(C.Structure):
+    """cgan3d_spatial_params_t: per-sample record of cgan3d_spatial_resample."""
+    _fields_ = [("flags", C.c_int32), ("coef_slot", C.c_int32), ("field_slot", C.c_int32), ("shift", C.c_int32 * 3),
+                ("A", C.c_float * 9), ("ctr", C.c_float * 3)]
+
+
 class Cgan3dError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"libcgan3d error {code}: {msg}")
@@ -81,6 +91,12 @@ SIGNATURES = {
     "cgan3d_tile_accumulate": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "cgan3d_tile_finalize": (_i, [_vp, _vp, _vp, _i64, _f, _f, _vp]),
     "cgan3d_sub_resized": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
+    "cgan3d_elastic_noise": (_i, [_i, _i, _i, _i, _vp, _vp, _vp]),
+    "cgan3d_elastic_workspace_bytes": (_sz, [_i, _i, _i, _i]),
+    "cgan3d_elastic_field": (_i, [_i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "cgan3d_spline_workspace_bytes": (_sz, [_i, _i, _i, _i, _i]),
+    "cgan3d_spline_prefilter": (_i, [_vp, _i, _i, _i, _i, _vp, _i, _vp, _sz, _vp]),
+    "cgan3d_spatial_resample": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _f, _i, _vp, _vp, _vp]),
 }
 
 _lib = None

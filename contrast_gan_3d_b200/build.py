@@ -14,7 +14,7 @@ ROOT = PKG.parent
 CSRC = PKG / "csrc"
 OBJ = PKG / "build"
 LIB = PKG / "libcgan3d.so"
-SOURCES = ["api_misc.cu", "conv_api.cu", "conv_generic.cu", "conv_tc.cu", "conv_tc_prog.cu", "conv_tc_prog_ks1.cu", "conv_tc_prog_ks2.cu", "conv_tc_prog_ks4.cu", "conv_tc_prog_ks8.cu", "conv_thin_tc.cu", "wgrad7_v2.cu", "conv_d1_tc.cu", "wgrad_tc.cu", "wgrad_s2_tc.cu", "norm_act.cu", "loss_optim.cu"]
+SOURCES = ["api_misc.cu", "conv_api.cu", "conv_generic.cu", "conv_tc.cu", "conv_tc_prog.cu", "conv_tc_prog_ks1.cu", "conv_tc_prog_ks2.cu", "conv_tc_prog_ks4.cu", "conv_tc_prog_ks8.cu", "conv_thin_tc.cu", "wgrad7_v2.cu", "conv_d1_tc.cu", "wgrad_tc.cu", "wgrad_s2_tc.cu", "norm_act.cu", "loss_optim.cu", "augment.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr", "--expt-extended-lambda", "-I", str(ROOT / "include"), "-I", str(CSRC)]
 

@@ -1,6 +1,7 @@
 """Patch sampler: the crop / pad index law of reference data/CCTADataLoader.py:76-108 (which delegates to
 batchgenerators `pad_nd_image` + `crop(crop_type="random")`), with the pad + crop + int16->f32 + HU scaling
-done by one device kernel per patch instead of a whole-volume float copy on CPU workers.
+done by one device kernel per patch instead of a whole-volume float copy on CPU workers.  An optional `transform`
+(data.augment.SpatialTransform2, the reference's SpatialTransform_2) is applied to each batch after its crops.
 
 The integer index math is host-side Python and bit-exact with the oracle restatement; volumes are int16
 [W, H, D, 2] (HU, centerline mask)."""
@@ -36,10 +37,11 @@ def random_crop_lower_bounds(padded_shape: Sequence[int], patch: Sequence[int], 
 
 class DevicePatchSampler:
     """Samples batches {"data": f32 [B,1,*patch], "seg": bool [B,1,*patch], "name", "path"} like
-    CCTADataLoader.generate_train_batch, from device-resident int16 volumes."""
+    CCTADataLoader.generate_train_batch, from device-resident int16 volumes.  With a `transform`, the batch passes
+    through it after all its crops are drawn (the reference's loader-then-augmenter order), drawing from the same `rs`."""
 
     def __init__(self, volumes: List[torch.Tensor], patch_shape: Sequence[int], batch_size: int,
-                 scaler: FactorZeroCenterScaler = None, names: List[str] = None, rs=np.random):
+                 scaler: FactorZeroCenterScaler = None, names: List[str] = None, rs=np.random, transform=None):
         for v in volumes:
             if v.dtype != torch.int16 or v.dim() != 4 or v.shape[-1] != 2 or not v.is_cuda:
                 raise ValueError("volumes must be CUDA int16 tensors [W, H, D, 2]")
@@ -49,6 +51,7 @@ class DevicePatchSampler:
         self.scaler = scaler or FactorZeroCenterScaler(-1024, 1500, 600)
         self.names = names or [f"vol{i}" for i in range(len(volumes))]
         self.rs = rs
+        self.transform = transform
 
     def get_indices(self) -> np.ndarray:
         # batchgenerators DataLoader.get_indices with infinite=True
@@ -70,7 +73,8 @@ class DevicePatchSampler:
         for i, idx in enumerate(self.get_indices()):
             lbs.append(self.sample_one(self.volumes[idx], data[i], seg[i]))
             names.append(self.names[idx])
-        return {"data": data, "seg": seg.view(torch.bool), "name": names, "path": names, "lbs": lbs}
+        batch = {"data": data, "seg": seg.view(torch.bool), "name": names, "path": names, "lbs": lbs}
+        return batch if self.transform is None else self.transform(batch, rs=self.rs)
 
     def __next__(self):
         return self.generate_train_batch()

@@ -3,9 +3,11 @@ train.py:97-107): pass it to `--conf-overwrites` to rebind the generator / criti
 B200-native implementations.  Values mirror basic_conf.py:22-68."""
 from functools import partial
 
+import numpy as np
 import torch
 from torch.optim.lr_scheduler import MultiStepLR
 
+from ..data.augment import SpatialTransform2
 from ..data.Scaler import FactorZeroCenterScaler
 from ..model.discriminator import PatchGANDiscriminator
 from ..model.generator import ResnetGenerator
@@ -32,3 +34,14 @@ critic_args = {"channels_in": 1, "init_channels_out": 8, "discriminator_depth": 
 critic_class = partial(PatchGANDiscriminator, **critic_args, compute_dtype=compute_dtype)
 critic_optim_class = partial(FusedAdam, lr=lr, betas=betas)
 critic_lr_scheduler_class = partial(MultiStepLR, milestones=milestones, gamma=lr_gamma)
+
+# Training augmentation: batchgenerators SpatialTransform_2 of basic_conf.py:88-106 on the device, with the values
+# SURVEY §3.4 records (elastic p=0.1, scale 0.7-1.4 p=0.2, rotation ±30° p=0.2, taken here as all three axes).  The
+# arguments it does not record (patch_center_dist_from_border, deformation_scale, border modes and orders, random_crop)
+# stay at upstream's defaults.  Pass it as DevicePatchSampler(..., transform=train_transform); validation sampling stays
+# untransformed.
+patch_size = (128, 128, 128)
+train_transform = SpatialTransform2(
+    patch_size, do_elastic_deform=True, p_el_per_sample=0.1, do_scale=True, scale=(0.7, 1.4), p_scale_per_sample=0.2,
+    do_rotation=True, angle_x=(-np.pi / 6, np.pi / 6), angle_y=(-np.pi / 6, np.pi / 6), angle_z=(-np.pi / 6, np.pi / 6),
+    p_rot_per_sample=0.2)

@@ -232,6 +232,48 @@ int cgan3d_tile_finalize(const float *acc, const float *cnt, float *out, int64_t
 int cgan3d_sub_resized(const float *x, const float *att, float *out, int B, int X, int Y, int Z, int Xa, int Ya, int Za,
                        void *stream);
 
+/* ---- spatial augmentation (batchgenerators SpatialTransform_2, reference experiments/basic_conf.py:88-106) ------
+ * Three stages per batch: elastic offset fields for the samples that drew elastic deformation, cubic B-spline
+ * coefficients for the samples that drew any transform, and one resampling launch for the whole batch.  Data order 3
+ * with border mode constant or nearest, seg order 0 constant, 3-D only; anything else is CGAN3D_E_UNSUPPORTED.
+ * Extents are 4..256 per axis.  Every parameter array is a device pointer.                                          */
+#define CGAN3D_BORDER_CONSTANT 0
+#define CGAN3D_BORDER_NEAREST 1
+#define CGAN3D_SPATIAL_TRANSFORM 1 /* sample drew elastic, rotation or scaling: resample, else shifted copy */
+#define CGAN3D_SPATIAL_ELASTIC 2   /* sample adds field[field_slot] to the mesh */
+
+/* per-sample record of the resampling stage (72 bytes) */
+typedef struct {
+  int32_t flags;      /* CGAN3D_SPATIAL_* */
+  int32_t coef_slot;  /* index of the sample's coefficient volume (TRANSFORM) */
+  int32_t field_slot; /* index of the sample's offset field and sums (ELASTIC) */
+  int32_t shift[3];   /* lower bounds of the zero-filled copy (no TRANSFORM): out[x] = in[x + shift] */
+  float A[9];         /* row-major linear map: diag(scale) * rotation^T */
+  float ctr[3];       /* centre of the patch in input voxels */
+} cgan3d_spatial_params_t;
+
+/* uniform [-1, 1) noise [n][3][PX][PY][PZ] fp32 of the elastic stage: Philox4x32-10 keyed by seeds[i], counter = the
+ * element's linear index within its sample.  The elastic field generates exactly these values internally.          */
+int cgan3d_elastic_noise(int n, int PX, int PY, int PZ, const uint64_t *seeds, float *noise, void *stream);
+size_t cgan3d_elastic_workspace_bytes(int n, int PX, int PY, int PZ);
+/* field[i][d] = g / (max|g| / (mags[i][d] + 1e-8)), g = circular convolution of the noise with taps[i] (per sample:
+ * PX x-taps, PY y-taps, PZ z-taps, fp64, the real inverse FFT of fourier_gaussian's kernel) along z, y and x;
+ * sums[i][d] = sum of field[i][d] (fp64).  Fixed-order reductions: the output depends on the seeds only.           */
+int cgan3d_elastic_field(int n, int PX, int PY, int PZ, const uint64_t *seeds, const double *mags, const double *taps,
+                         float *field, double *sums, void *ws, size_t ws_bytes, void *stream);
+/* coefficient volumes of scipy.ndimage.spline_filter(order=3) of data[samples[j]] (fp32 [B][SX][SY][SZ]); for
+ * CGAN3D_BORDER_NEAREST of the input edge-padded by 12 voxels, as map_coordinates does.                            */
+size_t cgan3d_spline_workspace_bytes(int n, int SX, int SY, int SZ, int mode);
+int cgan3d_spline_prefilter(const float *data, int SX, int SY, int SZ, int n, const int32_t *samples, int mode,
+                            float *coef, size_t coef_bytes, void *stream);
+/* out[b] (fp32 [B][PX][PY][PZ]) and out_seg[b] (uint8) from data / seg [B][SX][SY][SZ]: per sample either
+ * map_coordinates at c = A (mesh + field) - A mean(field) + ctr (data order 3 in `mode`, cval outside; seg order 0,
+ * seg_fill outside [0, S-1]) or the zero-filled copy at params[b].shift.                                           */
+int cgan3d_spatial_resample(const float *data, const uint8_t *seg, int B, int SX, int SY, int SZ, int PX, int PY, int PZ,
+                            const cgan3d_spatial_params_t *params, const float *field, const double *sums,
+                            const float *coef, int mode, float cval, int seg_fill, float *out, uint8_t *out_seg,
+                            void *stream);
+
 #ifdef __cplusplus
 }
 #endif
