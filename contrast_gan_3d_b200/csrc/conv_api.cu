@@ -22,11 +22,75 @@ static int check_geom(const cgan3d_conv_geom *g, int dtype) {
   return 0;
 }
 
-static int pick(const cgan3d_conv_geom &g, int dtype, int op, int impl, bool *use_tc) {
-  const bool can = tc_supported(g, dtype, op);
+enum class TcFamily { None, ThinA, ThinB, D1Gather, D1Scatter, S1, Prog, ThinW2, ThinC, D1Wgrad, WgradS2, WgradProg };
+
+struct TcRoute {
+  TcFamily family = TcFamily::None;
+  TcQuery q{};
+};
+
+// The tcgen05 kernel family that runs (g, dtype, op), with what its planner reports: the first family in the op's list
+// whose planner accepts the shape, or None (the generic CUDA-core kernels then run; every family is bf16 only).  The
+// families' shape domains overlap in two places, and there the order decides: the v2 thin weight gradient before the
+// round-1 one (even padding and extents), wgrad_s2 before wgrad_prog.
+static TcRoute tc_route(const cgan3d_conv_geom &g, int dtype, int op) {
+  using F = TcFamily;
+  struct Entry {
+    F family;
+    bool (*query)(const cgan3d_conv_geom &, int, TcQuery &);
+  };
+  static const Entry kOrder[3][5] = {
+      {{F::ThinA, thin_a_query}, {F::ThinB, thin_b_query}, {F::D1Gather, d1_gather_query}, {F::S1, s1_query}, {F::Prog, prog_query}},
+      {{F::ThinA, thin_a_query}, {F::ThinB, thin_b_query}, {F::D1Scatter, d1_scatter_query}, {F::S1, s1_query}, {F::Prog, prog_query}},
+      {{F::ThinW2, thin_w2_query}, {F::ThinC, thin_c_query}, {F::D1Wgrad, d1_wgrad_query}, {F::WgradS2, wgrad_s2_query},
+       {F::WgradProg, wgrad_prog_query}}};
+  TcRoute r;
+  if (!cgan3d_device_supports_tc() || tc_encode_fn() == nullptr || dtype != CGAN3D_BF16 || op < 0 || op > 2) return r;
+  for (const Entry &e : kOrder[op])
+    if (e.query(g, op, r.q)) {
+      r.family = e.family;
+      break;
+    }
+  return r;
+}
+
+static int pick(const TcRoute &r, int impl, bool *use_tc) {
+  const bool can = r.family != TcFamily::None;
   if (impl == 2 && !can) return fail(CGAN3D_E_UNSUPPORTED, "conv: tcgen05 path does not support this shape/op");
   *use_tc = (impl == 2) || (impl == 0 && can);
   return 0;
+}
+
+static int check_workspace(const TcRoute &r, const void *ws, size_t ws_bytes) {
+  const size_t need = r.q.workspace_bytes;
+  if (need && (ws == nullptr || ws_bytes < need))
+    return fail(CGAN3D_E_WORKSPACE, "tcgen05 conv: workspace %zu < %zu", ws_bytes, need);
+  return 0;
+}
+
+// gather (op 0: in = big side, out = small side) or scatter (op 1: the other way round) on the routed family
+static int tc_conv(const TcRoute &r, const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *out, void *ws,
+                   size_t ws_bytes, cudaStream_t st, double *bn_sums) {
+  if (int e = check_workspace(r, ws, ws_bytes)) return e;
+  switch (r.family) {
+    case TcFamily::ThinA: return thin_a_run(g, op, in, wp, out, ws, st, bn_sums);
+    case TcFamily::ThinB: return thin_b_run(g, op, in, wp, out, ws, st);
+    case TcFamily::D1Gather: return d1_gather_run(g, in, wp, out, ws, st);
+    case TcFamily::D1Scatter: return d1_scatter_run(g, in, wp, out, ws, st);
+    case TcFamily::S1: return s1_run(g, op, in, wp, out, ws, st, bn_sums);
+    case TcFamily::Prog: return prog_run(g, op, in, wp, out, ws, st, bn_sums);
+    default: return fail(CGAN3D_E_UNSUPPORTED, "conv: tcgen05 path does not support this shape/op");
+  }
+}
+
+static int run_conv(const cgan3d_conv_geom &g, int dtype, int op, const void *in, const void *wp, const float *bias, void *out,
+                    void *ws, size_t ws_bytes, int impl, cudaStream_t st) {
+  const TcRoute r = tc_route(g, dtype, op);
+  bool tc = false;
+  if (int e = pick(r, impl, &tc)) return e;
+  if (!tc) return op == 0 ? generic_gather(g, dtype, in, wp, bias, out, st) : generic_scatter(g, dtype, in, wp, bias, out, ws, ws_bytes, st);
+  if (bias) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: bias is applied by the bias_act pass");
+  return tc_conv(r, g, op, in, wp, out, ws, ws_bytes, st, nullptr);
 }
 
 }  // namespace cg
@@ -44,14 +108,14 @@ int cgan3d_pack_weights(const float *w, void *packed, int dtype, int Cs, int Cb,
 
 size_t cgan3d_conv_workspace_bytes(const cgan3d_conv_geom *g, int dtype, int op) {
   if (!g || check_geom(g, dtype) != 0) return 0;
-  const size_t a = tc_supported(*g, dtype, op) ? tc_workspace_bytes(*g, dtype, op) : 0, b = generic_workspace_bytes(*g, dtype, op);
+  const size_t a = tc_route(*g, dtype, op).q.workspace_bytes, b = generic_workspace_bytes(*g, dtype, op);
   return a > b ? a : b;
 }
 
 int cgan3d_conv_select(const cgan3d_conv_geom *g, int dtype, int op) {
   int r = check_geom(g, dtype);
   if (r) return r;
-  return tc_supported(*g, dtype, op) ? 2 : 1;
+  return tc_route(*g, dtype, op).family != TcFamily::None ? 2 : 1;
 }
 
 int cgan3d_conv_gather(const cgan3d_conv_geom *g, int dtype, const void *big, const void *wpacked, const float *bias,
@@ -60,15 +124,12 @@ int cgan3d_conv_gather(const cgan3d_conv_geom *g, int dtype, const void *big, co
   if (r) return r;
   CG_CHECK_ARG(big && wpacked && small, "conv_gather: NULL pointer");
   if (g->B == 0) return 0;
-  bool tc = false;
-  if ((r = pick(*g, dtype, 0, impl, &tc))) return r;
-  if (tc) return tc_gather(*g, big, wpacked, bias, small, workspace, workspace_bytes, as_stream(stream));
-  return generic_gather(*g, dtype, big, wpacked, bias, small, as_stream(stream));
+  return run_conv(*g, dtype, 0, big, wpacked, bias, small, workspace, workspace_bytes, impl, as_stream(stream));
 }
 
 int cgan3d_conv_fuses_bnstats(const cgan3d_conv_geom *g, int dtype, int op) {
   if (!g || check_geom(g, dtype) != 0) return 0;
-  return tc_fuses_bnstats(*g, dtype, op) ? 1 : 0;
+  return tc_route(*g, dtype, op).q.fuses_bnstats ? 1 : 0;
 }
 
 int cgan3d_conv_bnstats(const cgan3d_conv_geom *g, int dtype, int op, const void *in, const void *wpacked, void *out,
@@ -77,13 +138,13 @@ int cgan3d_conv_bnstats(const cgan3d_conv_geom *g, int dtype, int op, const void
   if (r) return r;
   CG_CHECK_ARG(in && wpacked && out && sums, "conv_bnstats: NULL pointer");
   CG_CHECK_ARG(op == 0 || op == 1, "conv_bnstats: op must be 0 (gather) or 1 (scatter)");
-  if (!tc_fuses_bnstats(*g, dtype, op)) return fail(CGAN3D_E_UNSUPPORTED, "conv_bnstats: this layer / device cannot fuse the statistics");
+  const TcRoute rt = tc_route(*g, dtype, op);
+  if (!rt.q.fuses_bnstats) return fail(CGAN3D_E_UNSUPPORTED, "conv_bnstats: this layer / device cannot fuse the statistics");
   const int C = op == 0 ? g->Cs : g->Cb;
   cudaError_t e = cudaMemsetAsync(sums, 0, (size_t)2 * C * sizeof(double), as_stream(stream));
   if (e != cudaSuccess) return cuda_fail(e, "conv_bnstats memset");
   if (g->B == 0) return 0;
-  if (op == 0) return tc_gather(*g, in, wpacked, nullptr, out, workspace, workspace_bytes, as_stream(stream), sums);
-  return tc_scatter(*g, in, wpacked, nullptr, out, workspace, workspace_bytes, as_stream(stream), sums);
+  return tc_conv(rt, *g, op, in, wpacked, out, workspace, workspace_bytes, as_stream(stream), sums);
 }
 
 int cgan3d_conv_scatter(const cgan3d_conv_geom *g, int dtype, const void *small, const void *wpacked,
@@ -93,10 +154,7 @@ int cgan3d_conv_scatter(const cgan3d_conv_geom *g, int dtype, const void *small,
   if (r) return r;
   CG_CHECK_ARG(big && wpacked && small, "conv_scatter: NULL pointer");
   if (g->B == 0) return 0;
-  bool tc = false;
-  if ((r = pick(*g, dtype, 1, impl, &tc))) return r;
-  if (tc) return tc_scatter(*g, small, wpacked, bias, big, workspace, workspace_bytes, as_stream(stream));
-  return generic_scatter(*g, dtype, small, wpacked, bias, big, workspace, workspace_bytes, as_stream(stream));
+  return run_conv(*g, dtype, 1, small, wpacked, bias, big, workspace, workspace_bytes, impl, as_stream(stream));
 }
 
 int cgan3d_conv_wgrad(const cgan3d_conv_geom *g, int dtype, const void *big, const void *small, float *dw, float beta,
@@ -105,10 +163,20 @@ int cgan3d_conv_wgrad(const cgan3d_conv_geom *g, int dtype, const void *big, con
   if (r) return r;
   CG_CHECK_ARG(big && small && dw, "conv_wgrad: NULL pointer");
   CG_CHECK_ARG(beta == 0.f || beta == 1.f, "conv_wgrad: beta must be 0 or 1");
+  const TcRoute rt = tc_route(*g, dtype, 2);
   bool tc = false;
-  if ((r = pick(*g, dtype, 2, impl, &tc))) return r;
-  if (tc) return tc_wgrad(*g, big, small, dw, beta, workspace, workspace_bytes, as_stream(stream));
-  return generic_wgrad(*g, dtype, big, small, dw, beta, as_stream(stream));
+  if ((r = pick(rt, impl, &tc))) return r;
+  if (!tc) return generic_wgrad(*g, dtype, big, small, dw, beta, as_stream(stream));
+  if ((r = check_workspace(rt, workspace, workspace_bytes))) return r;
+  const cudaStream_t st = as_stream(stream);
+  switch (rt.family) {
+    case TcFamily::ThinW2: return thin_w2_run(*g, big, small, dw, beta, st);
+    case TcFamily::ThinC: return thin_c_run(*g, big, small, dw, beta, workspace, st);
+    case TcFamily::D1Wgrad: return d1_wgrad_run(*g, big, small, dw, beta, workspace, st);
+    case TcFamily::WgradS2: return wgrad_s2_run(*g, big, small, dw, beta, st);
+    case TcFamily::WgradProg: return wgrad_prog_run(*g, big, small, dw, beta, st);
+    default: return fail(CGAN3D_E_UNSUPPORTED, "conv: tcgen05 path does not support this shape/op");
+  }
 }
 
 int cgan3d_reflect_pad(const void *in, void *out, int dtype, int B, int X, int Y, int Z, int C, int pad,

@@ -254,13 +254,16 @@ static bool plan_d1_gather(const cgan3d_conv_geom &g, D1GatherPlan &best) {
   return true;
 }
 
-static size_t d1_gather_ws(const D1GatherPlan &p) { return (size_t)kD1Tiles * kD1TileBytes + 256 + (size_t)p.B * p.Xi * p.Yi * p.Zc * 2 + 256; }
+bool d1_gather_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
+  D1GatherPlan p;
+  if (!plan_d1_gather(g, p)) return false;
+  q = {(size_t)kD1Tiles * kD1TileBytes + 256 + (size_t)p.B * p.Xi * p.Yi * p.Zc * 2 + 256, false};
+  return true;
+}
 
-static int run_d1_gather(const cgan3d_conv_geom &g, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                         cudaStream_t st) {
+int d1_gather_run(const cgan3d_conv_geom &g, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st) {
   D1GatherPlan p;
   if (!plan_d1_gather(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 critic-first conv: shape not supported");
-  if (ws == nullptr || ws_bytes < d1_gather_ws(p)) return fail(CGAN3D_E_WORKSPACE, "tcgen05 critic-first conv: workspace too small");
   if ((reinterpret_cast<uintptr_t>(outp) & 15) || (reinterpret_cast<uintptr_t>(ws) & 255))
     return fail(CGAN3D_E_ARG, "tcgen05 critic-first conv: pointers must be 16-byte aligned (workspace 256)");
   bf16 *wt = reinterpret_cast<bf16 *>(ws);
@@ -444,13 +447,16 @@ static bool plan_d1_wgrad(const cgan3d_conv_geom &g, D1WgradPlan &p) {
   return true;
 }
 
-static size_t d1_wgrad_ws(const D1WgradPlan &p) { return (size_t)p.B * p.Xi * p.Ye * p.Zs * 16 + 256; }
+bool d1_wgrad_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
+  D1WgradPlan p;
+  if (!plan_d1_wgrad(g, p)) return false;
+  q = {(size_t)p.B * p.Xi * p.Ye * p.Zs * 16 + 256, false};
+  return true;
+}
 
-int d1_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-                 cudaStream_t st) {
+int d1_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, cudaStream_t st) {
   D1WgradPlan p;
   if (!plan_d1_wgrad(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 critic-first wgrad: shape not supported");
-  if (ws == nullptr || ws_bytes < d1_wgrad_ws(p)) return fail(CGAN3D_E_WORKSPACE, "tcgen05 critic-first wgrad: workspace too small");
   if ((reinterpret_cast<uintptr_t>(small) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 critic-first wgrad: pointers must be 16-byte aligned");
   if (beta == 0.f) {
@@ -663,11 +669,16 @@ static bool plan_d1_scatter(const cgan3d_conv_geom &g, D1ScatterPlan &best) {
   return true;
 }
 
-static int run_d1_scatter(const cgan3d_conv_geom &g, const void *small, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                          cudaStream_t st) {
+bool d1_scatter_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
+  D1ScatterPlan p;
+  if (!plan_d1_scatter(g, p)) return false;
+  q = {4 * kD1STileBytes + 256, false};
+  return true;
+}
+
+int d1_scatter_run(const cgan3d_conv_geom &g, const void *small, const void *wp, void *outp, void *ws, cudaStream_t st) {
   D1ScatterPlan p;
   if (!plan_d1_scatter(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 critic-first dgrad: shape not supported");
-  if (ws == nullptr || ws_bytes < 4 * kD1STileBytes) return fail(CGAN3D_E_WORKSPACE, "tcgen05 critic-first dgrad: workspace too small");
   if ((reinterpret_cast<uintptr_t>(small) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 critic-first dgrad: pointers must be 16-byte aligned");
   bf16 *wt = reinterpret_cast<bf16 *>(ws);
@@ -690,30 +701,6 @@ static int run_d1_scatter(const cgan3d_conv_geom &g, const void *small, const vo
     case 4: return launch(std::integral_constant<int, 4>{});
     default: return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 critic-first dgrad: mtiles %d not built", p.mtiles);
   }
-}
-
-// ============================================================================================================== dispatch
-bool d1_supported(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16 || !d1_shape(g)) return false;
-  if (op == 0) { D1GatherPlan p; return plan_d1_gather(g, p); }
-  if (op == 1) { D1ScatterPlan p; return plan_d1_scatter(g, p); }
-  if (op == 2) { D1WgradPlan p; return plan_d1_wgrad(g, p); }
-  return false;
-}
-
-size_t d1_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (!d1_supported(g, dtype, op)) return 0;
-  if (op == 0) { D1GatherPlan p; plan_d1_gather(g, p); return d1_gather_ws(p); }
-  if (op == 1) return 4 * kD1STileBytes + 256;
-  D1WgradPlan p;
-  plan_d1_wgrad(g, p);
-  return d1_wgrad_ws(p);
-}
-
-int d1_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes, cudaStream_t st) {
-  if (op == 0) return run_d1_gather(g, in, wp, outp, ws, ws_bytes, st);
-  if (op == 1) return run_d1_scatter(g, in, wp, outp, ws, ws_bytes, st);
-  return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 critic-first conv: op %d", op);
 }
 
 }  // namespace cg

@@ -19,21 +19,8 @@ int reflect_pad(const void *in, void *out, int dtype, int B, int X, int Y, int Z
 int reflect_pad_backward(const void *gp, void *gi, int dtype, int B, int X, int Y, int Z, int C, int pad,
                          cudaStream_t st);
 
-// tcgen05 implicit-GEMM path (conv_tc.cu). op: 0 gather, 1 scatter, 2 wgrad.
-bool tc_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t tc_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-// bn_sums (optional, fp64 [2*Cout], zeroed by the caller): the epilogue adds the per-channel sum / sum of squares of the
-// fp32 accumulators (BatchNorm batch statistics fused into the convolution); see tc_fuses_bnstats.
-int tc_gather(const cgan3d_conv_geom &g, const void *big, const void *wp, const float *bias, void *small,
-              void *ws, size_t ws_bytes, cudaStream_t st, double *bn_sums = nullptr);
-int tc_scatter(const cgan3d_conv_geom &g, const void *small, const void *wp, const float *bias, void *big,
-               void *ws, size_t ws_bytes, cudaStream_t st, double *bn_sums = nullptr);
-bool tc_fuses_bnstats(const cgan3d_conv_geom &g, int dtype, int op);
-int tc_wgrad(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws,
-             size_t ws_bytes, cudaStream_t st);
-
 // cuTensorMapEncodeTiled, looked up once through the runtime's driver entry point (conv_tc.cu); nullptr when the driver
-// does not export it.  Only encode_tiled calls it; tc_supported uses it to test availability.
+// does not export it.  Only encode_tiled calls it; the tcgen05 route (conv_api.cu) uses it to test availability.
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *, const cuuint64_t *,
                                   const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -86,39 +73,56 @@ int tc_launch(const char *name, int grid, int block, size_t smem, int cluster, c
   return 0;
 }
 
-// conv_tc_prog.cu (strided convolutions)
-bool tc_prog_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t tc_prog_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                cudaStream_t st, double *bn_sums = nullptr);
-bool tc_prog_fuses_bnstats(const cgan3d_conv_geom &g, int scatter);
+// ---------------------------------------------------------------- tcgen05 kernel families (bf16 only)
+// Each family exports a query and a launcher.  tc_route (conv_api.cu) picks the family, and the entry points there check
+// the rules the families share.  A query returns true when the family's planner accepts the shape and then fills TcQuery;
+// op: 0 gather, 1 scatter, 2 wgrad (families that serve one op ignore it).  A launcher takes a shape its query accepted, a
+// workspace of at least the reported size and, where the family fuses them, bn_sums (fp64 [2*Cout], zeroed by the
+// caller): the epilogue adds the per-channel sum / sum of squares of the fp32 accumulators.  The launchers check the
+// pointer alignment their kernels need.
+struct TcQuery {
+  size_t workspace_bytes;  // what cgan3d_conv_workspace_bytes reports for the family; 0: none used
+  bool fuses_bnstats;      // the launcher takes bn_sums
+};
 
-// conv_thin_tc.cu (7x7x7 thin-channel layers)
-bool thin_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t thin_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-int thin_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-             cudaStream_t st, double *bn_sums = nullptr);
-bool thin_fuses_bnstats(const cgan3d_conv_geom &g, int op);
-int thin_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-                   cudaStream_t st);
+// conv_thin_tc.cu (7x7x7 thin-channel layers).  A: 1 -> 16 channels (gather of Cb == 1, scatter of Cs == 1);
+// B: 16 -> 1 channels (the other two); C: round-1 weight gradient of both, for the shapes wgrad7_v2.cu does not plan
+bool thin_a_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int thin_a_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st,
+               double *bn_sums);
+bool thin_b_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int thin_b_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st);
+bool thin_c_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int thin_c_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, cudaStream_t st);
 
 // wgrad7_v2.cu: weight gradient of the thin layers, the z-expansion built in shared memory (no workspace)
-bool thin_w2_supported(const cgan3d_conv_geom &g);
+bool thin_w2_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
 int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
 
 // conv_d1_tc.cu (first critic layer: 1 -> 8 channels, k4 s2)
-bool d1_supported(const cgan3d_conv_geom &g, int dtype, int op);
-size_t d1_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op);
-int d1_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes, cudaStream_t st);
-int d1_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-                 cudaStream_t st);
+bool d1_gather_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int d1_gather_run(const cgan3d_conv_geom &g, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st);
+bool d1_scatter_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int d1_scatter_run(const cgan3d_conv_geom &g, const void *small, const void *wp, void *outp, void *ws, cudaStream_t st);
+bool d1_wgrad_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int d1_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, cudaStream_t st);
+
+// conv_tc.cu (3x3x3 stride-1 convolutions, Cin in {16, 32, 64, 128})
+bool s1_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int s1_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st,
+           double *bn_sums);
+
+// conv_tc_prog.cu (strided convolutions)
+bool prog_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int prog_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st,
+             double *bn_sums);
 
 // wgrad_s2_tc.cu (stride-2 layers with Cs in {32, 64}, Cb in {16, 32}, and the stride-1 ResNet layers with Cs == 64)
-bool tc_wgrad_s2_supported(const cgan3d_conv_geom &g);
-int tc_wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
+bool wgrad_s2_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
 
 // wgrad_tc.cu (the weight-gradient shapes wgrad_s2_tc.cu does not plan)
-bool tc_wgrad_supported(const cgan3d_conv_geom &g);
-int tc_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
+bool wgrad_prog_query(const cgan3d_conv_geom &g, int op, TcQuery &q);
+int wgrad_prog_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st);
 
 }  // namespace cg

@@ -837,43 +837,26 @@ static bool plan_s1_stack(int B, int X, int Y, int Z, int Cin, int N, TcPlan &be
   return true;
 }
 
-static bool s1_shape_ok(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16 || op < 0 || op > 1) return false;
-  if (g.k != 3 || g.stride != 1 || g.pad != 1) return false;
+bool s1_query(const cgan3d_conv_geom &g, int op, TcQuery &q) {
+  if (op < 0 || op > 1 || g.k != 3 || g.stride != 1 || g.pad != 1) return false;
   if (g.Xb != g.Xs || g.Yb != g.Ys || g.Zb != g.Zs) return false;
+  const int Cin = op == 0 ? g.Cb : g.Cs, N = op == 0 ? g.Cs : g.Cb;
+  TcPlan p;
+  if (!plan_s1(g.B, g.Xb, g.Yb, g.Zb, Cin, N, p)) return false;
+  q = {(size_t)27 * g.Cb * g.Cs * 2 + 256, N <= 64};
   return true;
 }
 
-bool tc_supported(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (!cgan3d_device_supports_tc() || tc_encode_fn() == nullptr) return false;
-  if (thin_supported(g, dtype, op) || d1_supported(g, dtype, op)) return true;
-  if (op == 2) return dtype == CGAN3D_BF16 && (tc_wgrad_s2_supported(g) || tc_wgrad_supported(g));
-  if (!s1_shape_ok(g, dtype, op)) return tc_prog_supported(g, dtype, op);
-  TcPlan p;
-  const int Cin = op == 0 ? g.Cb : g.Cs, N = op == 0 ? g.Cs : g.Cb;
-  return plan_s1(g.B, g.Xb, g.Yb, g.Zb, Cin, N, p);
-}
-
-size_t tc_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (thin_supported(g, dtype, op)) return thin_workspace_bytes(g, dtype, op);
-  if (d1_supported(g, dtype, op)) return d1_workspace_bytes(g, dtype, op);
-  if (op == 2) return 0;
-  if (!s1_shape_ok(g, dtype, op)) return tc_prog_workspace_bytes(g, dtype, op);
-  return (size_t)27 * g.Cb * g.Cs * 2 + 256;
-}
-
-static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                  cudaStream_t st, double *bn_sums) {
-  const int Cin = flip ? g.Cs : g.Cb, N = flip ? g.Cb : g.Cs;
+int s1_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st,
+           double *bn_sums) {
+  const int flip = op, Cin = flip ? g.Cs : g.Cb, N = flip ? g.Cb : g.Cs;
   TcPlan p;
   if (!plan_s1(g.B, g.Xb, g.Yb, g.Zb, Cin, N, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: no tiling for this shape");
-  const size_t need = (size_t)27 * Cin * N * 2;
-  if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 31) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 conv: input / workspace must be 16-byte aligned, the output 32-byte aligned (256-bit stores)");
   bf16 *wb = reinterpret_cast<bf16 *>(ws);
   TcPlan ps;
-  const bool stack = plan_s1_stack(g.B, g.Xb, g.Yb, g.Zb, Cin, N, ps) && !(bn_sums && N > 64);
+  const bool stack = plan_s1_stack(g.B, g.Xb, g.Yb, g.Zb, Cin, N, ps);
   if (stack) {
     p = ps;
     repack_b_stack_kernel<<<64, 256, 0, st>>>(reinterpret_cast<const bf16 *>(wp), wb, g.Cb, g.Cs, flip);
@@ -892,7 +875,6 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
   }
   const long long work = (long long)(p.pair ? (p.nitems + 1) / 2 : p.nitems) * p.X;
   const int grid = p.pair ? 2 * (int)mn<long long>(work, (long long)(num_sms() / 2)) : (int)mn<long long>(work, (long long)num_sms());
-  if (bn_sums && N > 64) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: fused BatchNorm statistics need Cout <= 64");
   if (stack) {
     auto launch_k = [&](auto ks_tag, auto mt_tag, auto st_tag) -> int {
       constexpr int KS = decltype(ks_tag)::value;
@@ -947,44 +929,6 @@ static int run_s1(const cgan3d_conv_geom &g, int flip, const void *in, const voi
     case 8: return by_mt(std::integral_constant<int, 8>{});
     default: return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: Cin must be 16, 32, 64 or 128");
   }
-}
-
-bool tc_fuses_bnstats(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16 || (op != 0 && op != 1) || !tc_supported(g, dtype, op)) return false;
-  if (thin_supported(g, dtype, op)) return thin_fuses_bnstats(g, op);
-  if (d1_supported(g, dtype, op)) return false;
-  const int N = op == 0 ? g.Cs : g.Cb;
-  if (N > 64) return false;
-  if (!s1_shape_ok(g, dtype, op)) return tc_prog_fuses_bnstats(g, op);
-  return true;
-}
-
-int tc_gather(const cgan3d_conv_geom &g, const void *big, const void *wp, const float *bias, void *small, void *ws,
-              size_t ws_bytes, cudaStream_t st, double *bn_sums) {
-  if (bias) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: bias is applied by the bias_act pass");
-  if (bn_sums && !tc_fuses_bnstats(g, CGAN3D_BF16, 0)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: this layer cannot fuse the BatchNorm statistics");
-  if (thin_supported(g, CGAN3D_BF16, 0)) return thin_run(g, 0, big, wp, small, ws, ws_bytes, st, bn_sums);
-  if (d1_supported(g, CGAN3D_BF16, 0)) return d1_run(g, 0, big, wp, small, ws, ws_bytes, st);
-  if (!s1_shape_ok(g, CGAN3D_BF16, 0)) return tc_prog_run(g, 0, big, wp, small, ws, ws_bytes, st, bn_sums);
-  return run_s1(g, 0, big, wp, small, ws, ws_bytes, st, bn_sums);
-}
-
-int tc_scatter(const cgan3d_conv_geom &g, const void *small, const void *wp, const float *bias, void *big, void *ws,
-               size_t ws_bytes, cudaStream_t st, double *bn_sums) {
-  if (bias) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: bias is applied by the bias_act pass");
-  if (bn_sums && !tc_fuses_bnstats(g, CGAN3D_BF16, 1)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 conv: this layer cannot fuse the BatchNorm statistics");
-  if (thin_supported(g, CGAN3D_BF16, 1)) return thin_run(g, 1, small, wp, big, ws, ws_bytes, st);
-  if (d1_supported(g, CGAN3D_BF16, 1)) return d1_run(g, 1, small, wp, big, ws, ws_bytes, st);
-  if (!s1_shape_ok(g, CGAN3D_BF16, 1)) return tc_prog_run(g, 1, small, wp, big, ws, ws_bytes, st, bn_sums);
-  return run_s1(g, 1, small, wp, big, ws, ws_bytes, st, bn_sums);
-}
-
-int tc_wgrad(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-             cudaStream_t st) {
-  if (thin_supported(g, CGAN3D_BF16, 2)) return thin_wgrad_run(g, big, small, dw, beta, ws, ws_bytes, st);
-  if (d1_supported(g, CGAN3D_BF16, 2)) return d1_wgrad_run(g, big, small, dw, beta, ws, ws_bytes, st);
-  if (tc_wgrad_s2_supported(g)) return tc_wgrad_s2_run(g, big, small, dw, beta, st);
-  return tc_wgrad_run(g, big, small, dw, beta, st);
 }
 
 }  // namespace cg

@@ -325,33 +325,25 @@ static bool plan_prog_split(const cgan3d_conv_geom &g, int scatter, ProgPlan &be
   return true;
 }
 
-bool tc_prog_supported(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16 || (op != 0 && op != 1)) return false;
-  ProgPlan p;
-  return plan_prog(g, op, p);
-}
+// bytes of one output-channel part's repacked filter tiles in the workspace
+static size_t prog_part_bytes(const ProgPlan &p) { return ((size_t)p.nbt * p.btile_bytes * (p.pair ? 2 : 1) + 255) / 256 * 256; }
 
-size_t tc_prog_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16 || (op != 0 && op != 1)) return 0;
+bool prog_query(const cgan3d_conv_geom &g, int op, TcQuery &q) {
+  if (op != 0 && op != 1) return false;
   ProgPlan p;
   int nsplit = 1;
-  if (!plan_prog(g, op, p, &nsplit)) return 0;
-  return (((size_t)p.nbt * p.btile_bytes * (p.pair ? 2 : 1) + 255) / 256 * 256) * nsplit + 256;
+  if (!plan_prog(g, op, p, &nsplit)) return false;
+  q = {prog_part_bytes(p) * nsplit + 256, (op == 0 ? g.Cs : g.Cb) <= 64};
+  return true;
 }
 
-bool tc_prog_fuses_bnstats(const cgan3d_conv_geom &g, int scatter) {
-  ProgPlan p;
-  return plan_prog(g, scatter, p) && p.Nout <= 64;
-}
-
-int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                cudaStream_t st, double *bn_sums) {
+int prog_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st,
+             double *bn_sums) {
+  const int scatter = op;
   ProgPlan p;
   int nsplit = 1;
   if (!plan_prog(g, scatter, p, &nsplit)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 strided conv: no tiling for this shape");
-  const size_t part_bytes = ((size_t)p.nbt * p.btile_bytes * (p.pair ? 2 : 1) + 255) / 256 * 256;
-  const size_t need = part_bytes * nsplit;
-  if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 strided conv: workspace %zu < %zu", ws_bytes, need);
+  const size_t part_bytes = prog_part_bytes(p);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 strided conv: pointers must be 16-byte aligned");
   // input tensor: gather reads the big side with element strides 2 on z and y; scatter reads the small side densely
@@ -366,7 +358,6 @@ int tc_prog_run(const cgan3d_conv_geom &g, int scatter, const void *in, const vo
   if (r) return r;
   const long long total = (long long)p.B * p.nzt * p.nslabs * p.Xg;
   const int grid = p.pair ? 2 * (int)mn<long long>((total + 1) / 2, (long long)(num_sms() / 2)) : (int)mn<long long>(total, (long long)num_sms());
-  if (bn_sums && p.Nout > 64) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 strided conv: fused BatchNorm statistics need <= 64 channels per launch");
   ProgLaunchArgs la{};
   la.tm = tm; la.g = g; la.scatter = scatter; la.nsplit = nsplit; la.grid = grid; la.wp = wp; la.outp = outp; la.ws = ws;
   la.part_bytes = part_bytes; la.bn_sums = bn_sums; la.st = st;

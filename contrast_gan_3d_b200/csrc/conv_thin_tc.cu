@@ -780,9 +780,6 @@ static bool plan_thin_a(const cgan3d_conv_geom &g, int op, ThinAPlan &best) {
   return true;
 }
 
-static bool plan_thin_c(const cgan3d_conv_geom &g, ThinCPlan &p);
-static size_t thin_c_workspace(const ThinCPlan &p);
-
 // op 0: gather with Cb == 16, Cs == 1;  op 1: scatter with Cb == 1, Cs == 16
 static bool thin_b_shape(const cgan3d_conv_geom &g, int op) {
   if (g.k != 7 || g.stride != 1) return false;
@@ -815,42 +812,27 @@ static bool plan_thin_b(const cgan3d_conv_geom &g, int op, ThinBPlan &p) {
   return true;
 }
 
-bool thin_supported(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16) return false;
-  if (op == 0 || op == 1) {
-    ThinAPlan pa;
-    if (plan_thin_a(g, op, pa)) return true;
-    ThinBPlan pb;
-    return plan_thin_b(g, op, pb);
-  }
-  if (op == 2) {
-    ThinCPlan pc;
-    return thin_w2_supported(g) || plan_thin_c(g, pc);
-  }
-  return false;
-}
-
 // room for two shifted copies of the input (the workspace size callers allocate); the 8-z items read only the first
 static size_t thin_a_repitch_bytes(const ThinAPlan &p) { return (size_t)2 * p.B * p.Xi * p.Yi * p.Zc * 2; }
 
-size_t thin_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
-  if (dtype != CGAN3D_BF16) return 0;
+bool thin_a_query(const cgan3d_conv_geom &g, int op, TcQuery &q) {
   ThinAPlan p;
-  if ((op == 0 || op == 1) && plan_thin_a(g, op, p)) return (size_t)kTapTilesA * kTileBytesA + 256 + thin_a_repitch_bytes(p) + 256;
-  ThinBPlan pb;
-  if ((op == 0 || op == 1) && plan_thin_b(g, op, pb)) return (size_t)kTapTilesB * kTileBytesB + 256;
-  ThinCPlan pc;
-  if (op == 2 && thin_w2_supported(g)) return 0;
-  if (op == 2 && plan_thin_c(g, pc)) return thin_c_workspace(pc);
-  return 0;
+  if (!plan_thin_a(g, op, p)) return false;
+  q = {(size_t)kTapTilesA * kTileBytesA + 256 + thin_a_repitch_bytes(p) + 256, op == 0};
+  return true;
 }
 
-static int run_thin_a(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                      cudaStream_t st, double *bn_sums) {
+bool thin_b_query(const cgan3d_conv_geom &g, int op, TcQuery &q) {
+  ThinBPlan p;
+  if (!plan_thin_b(g, op, p)) return false;
+  q = {(size_t)kTapTilesB * kTileBytesB + 256, false};
+  return true;
+}
+
+int thin_a_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st,
+               double *bn_sums) {
   ThinAPlan p;
   if (!plan_thin_a(g, op, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: shape not supported");
-  const size_t need = thin_workspace_bytes(g, CGAN3D_BF16, op);
-  if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 thin conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(outp) & 15) || (reinterpret_cast<uintptr_t>(ws) & 255))
     return fail(CGAN3D_E_ARG, "tcgen05 thin conv: pointers must be 16-byte aligned (workspace 256)");
   bf16 *wt = reinterpret_cast<bf16 *>(ws);
@@ -884,12 +866,9 @@ static int run_thin_a(const cgan3d_conv_geom &g, int op, const void *in, const v
   return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: mtiles %d not built", p.mtiles);
 }
 
-static int run_thin_b(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-                      cudaStream_t st) {
+int thin_b_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, cudaStream_t st) {
   ThinBPlan p;
   if (!plan_thin_b(g, op, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv (16->1): shape not supported");
-  const size_t need = (size_t)kTapTilesB * kTileBytesB;
-  if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 thin conv: workspace %zu < %zu", ws_bytes, need);
   if ((reinterpret_cast<uintptr_t>(in) & 15) || (reinterpret_cast<uintptr_t>(ws) & 15))
     return fail(CGAN3D_E_ARG, "tcgen05 thin conv: pointers must be 16-byte aligned");
   bf16 *wt = reinterpret_cast<bf16 *>(ws);
@@ -948,15 +927,16 @@ static bool plan_thin_c(const cgan3d_conv_geom &g, ThinCPlan &p) {
   return true;
 }
 
-static size_t thin_c_workspace(const ThinCPlan &p) { return (size_t)p.B * p.Xe * p.Ye * p.Zs * 16 + 256; }
+bool thin_c_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
+  ThinCPlan p;
+  if (!plan_thin_c(g, p)) return false;
+  q = {(size_t)p.B * p.Xe * p.Ye * p.Zs * 16 + 256, false};
+  return true;
+}
 
-int thin_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, size_t ws_bytes,
-                   cudaStream_t st) {
-  if (thin_w2_supported(g)) return thin_w2_run(g, big, small, dw, beta, st);
+int thin_c_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, void *ws, cudaStream_t st) {
   ThinCPlan p;
   if (!plan_thin_c(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin wgrad: shape not supported");
-  const size_t need = thin_c_workspace(p);
-  if (ws == nullptr || ws_bytes < need) return fail(CGAN3D_E_WORKSPACE, "tcgen05 thin wgrad: workspace %zu < %zu", ws_bytes, need);
   const bool first = p.flip == 0;
   const void *s16 = first ? small : big, *q1 = first ? big : small;
   const int Xq = first ? g.Xb : g.Xs, Yq = first ? g.Yb : g.Ys, Zq = first ? g.Zb : g.Zs;
@@ -979,16 +959,6 @@ int thin_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small
   const long long total = (long long)p.B * p.nyt * p.nzt * p.Xe;
   const int grid = (int)mn<long long>(total, (long long)num_sms());
   return tc_launch<wgrad7_thin_tc_kernel>("wgrad7_thin_tc_kernel", grid, 192, p.smem_bytes + 1024, 1, st, tmE, tmS, dw, p);
-}
-
-bool thin_fuses_bnstats(const cgan3d_conv_geom &g, int op) { return op == 0 && thin_a_shape(g, 0); }
-
-int thin_run(const cgan3d_conv_geom &g, int op, const void *in, const void *wp, void *outp, void *ws, size_t ws_bytes,
-             cudaStream_t st, double *bn_sums) {
-  if (bn_sums && !thin_fuses_bnstats(g, op)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: this op cannot fuse the BatchNorm statistics");
-  if ((op == 0 || op == 1) && thin_b_shape(g, op)) return run_thin_b(g, op, in, wp, outp, ws, ws_bytes, st);
-  if (op == 0 || op == 1) return run_thin_a(g, op, in, wp, outp, ws, ws_bytes, st, bn_sums);
-  return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 thin conv: op %d not built", op);
 }
 
 }  // namespace cg

@@ -532,9 +532,11 @@ static bool plan_w2(const cgan3d_conv_geom &g, ThinW2Plan &p) {
   return true;
 }
 
-bool thin_w2_supported(const cgan3d_conv_geom &g) {
+bool thin_w2_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
   ThinW2Plan p;
-  return plan_w2(g, p);
+  if (!plan_w2(g, p)) return false;
+  q = {0, false};
+  return true;
 }
 
 int thin_w2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {

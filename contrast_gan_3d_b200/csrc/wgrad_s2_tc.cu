@@ -285,12 +285,14 @@ static bool plan_ws(const cgan3d_conv_geom &g, WsPlan &p) {
   return true;
 }
 
-bool tc_wgrad_s2_supported(const cgan3d_conv_geom &g) {
+bool wgrad_s2_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
   WsPlan p;
-  return plan_ws(g, p);
+  if (!plan_ws(g, p)) return false;
+  q = {0, false};
+  return true;
 }
 
-int tc_wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {
+int wgrad_s2_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {
   WsPlan p;
   if (!plan_ws(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 strided wgrad: shape not supported");
   if ((reinterpret_cast<uintptr_t>(big) & 15) || (reinterpret_cast<uintptr_t>(small) & 15))

@@ -277,12 +277,14 @@ static bool plan_wgrad(const cgan3d_conv_geom &g, WgPlan &p) {
   return true;
 }
 
-bool tc_wgrad_supported(const cgan3d_conv_geom &g) {
+bool wgrad_prog_query(const cgan3d_conv_geom &g, int, TcQuery &q) {
   WgPlan p;
-  return plan_wgrad(g, p);
+  if (!plan_wgrad(g, p)) return false;
+  q = {0, false};
+  return true;
 }
 
-int tc_wgrad_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {
+int wgrad_prog_run(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta, cudaStream_t st) {
   WgPlan p;
   if (!plan_wgrad(g, p)) return fail(CGAN3D_E_UNSUPPORTED, "tcgen05 wgrad: shape not supported");
   if ((reinterpret_cast<uintptr_t>(big) & 15) || (reinterpret_cast<uintptr_t>(small) & 15))
