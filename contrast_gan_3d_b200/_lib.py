@@ -67,6 +67,9 @@ SIGNATURES = {
     "cgan3d_bn_apply_pad": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _i, _f, _i, _vp]),
     "cgan3d_bn_backward_reduce": (_i, [_vp, _vp, _i, _i64, _i, _vp, _vp, _vp, _i, _f, _vp, _vp]),
     "cgan3d_bn_backward_apply": (_i, [_vp, _vp, _vp, _i, _i64, _i, _vp, _vp, _vp, _i, _f, _vp, _vp, _vp, _f, _vp]),
+    "cgan3d_bn_apply_dropout": (_i, [_vp, _vp, _vp, _i, _i64, _i, _vp, _vp, _vp, _i, _f, _f, _vp, _vp]),
+    "cgan3d_bn_backward_reduce_dropout": (_i, [_vp, _vp, _vp, _i, _i64, _i, _vp, _vp, _vp, _i, _f, _f, _vp, _vp]),
+    "cgan3d_bn_backward_apply_dropout": (_i, [_vp, _vp, _vp, _vp, _i, _i64, _i, _vp, _vp, _vp, _i, _f, _f, _vp, _vp, _vp, _f, _vp]),
     "cgan3d_bias_act": (_i, [_vp, _vp, _i, _i64, _i, _vp, _i, _f, _vp]),
     "cgan3d_bias_act_backward": (_i, [_vp, _vp, _vp, _i, _i64, _i, _vp, _i, _f, _vp, _vp]),
     "cgan3d_col_sums": (_i, [_vp, _i, _i64, _i, _vp, _vp]),

@@ -20,26 +20,9 @@ constexpr int kNearestPad = 12;   // scipy.ndimage._interpolation._prepad_for_sp
 constexpr int kPartials = 64;     // stage-1 blocks per (sample, axis) of the field reduction
 constexpr double kPole = -0.26794919243112270;  // sqrt(3) - 2
 
-__device__ __forceinline__ uint32_t philox_x(uint32_t ctr, uint64_t seed) {
-  uint32_t c0 = ctr, c1 = 0, c2 = 0, c3 = 0;
-  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-    const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-    c0 = hi1 ^ c1 ^ k0;
-    c1 = lo1;
-    c2 = hi0 ^ c3 ^ k1;
-    c3 = lo0;
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  return c0;
-}
-
-// element e of a sample's [3][PX][PY][PZ] noise: 2u - 1 with u = k * 2^-24, exact in fp32
+// element e of a sample's [3][PX][PY][PZ] noise: 2u - 1 with u = k * 2^-24, exact in fp32 (word 0 of counter (e, 0, 0, 0))
 __device__ __forceinline__ float noise_at(uint32_t e, uint64_t seed) {
-  return (float)(philox_x(e, seed) >> 8) * 0x1p-23f - 1.f;
+  return (float)(philox4x32_10(e, 0, 0, 0, seed).x >> 8) * 0x1p-23f - 1.f;
 }
 
 __global__ void __launch_bounds__(256) elastic_noise_kernel(const uint64_t *__restrict__ seeds, float *__restrict__ out,

@@ -8,6 +8,23 @@
 
 namespace cg {
 
+// ---------------------------------------------------------------- dropout keep law (reference model/blocks.py:68-88)
+// Element e (the channels-last linear index) is kept iff u(e) >= thresh, where u(e) is word e & 3 of Philox4x32-10 at
+// counter (lo32(e >> 2), hi32(e >> 2), 0, 0) under the 64-bit seed, and thresh = floor(p * 2^32) (2^32 at p = 1: nothing
+// is kept).  One Philox evaluation serves four elements.  Returns the keep bits of e0 .. e0 + 7 (e0 % 8 == 0), bit k for
+// e0 + k: byte e0 / 8 of the bitmask that the backward passes read.
+__device__ __forceinline__ uint32_t dropout_keep8(uint64_t e0, uint64_t seed, uint64_t thresh) {
+  uint32_t bits = 0;
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const uint64_t q = (e0 >> 2) + h;
+    const uint4 w = philox4x32_10((uint32_t)q, (uint32_t)(q >> 32), 0, 0, seed);
+    bits |= ((uint32_t)(w.x >= thresh) | (uint32_t)(w.y >= thresh) << 1 | (uint32_t)(w.z >= thresh) << 2 |
+             (uint32_t)(w.w >= thresh) << 3) << (4 * h);
+  }
+  return bits;
+}
+
 // ---------------------------------------------------------------- column reductions
 // Block of 256 threads covers `lanes = 256 / Cw` rows at a time; thread (lane, c) walks rows
 // lane, lane+lanes, ... of its block's strip.  Per-thread fp32 partials over a short run are
@@ -96,15 +113,21 @@ __global__ void __launch_bounds__(256) col_sums_kernel(const T *__restrict__ x, 
   col_reduce_body<1>(n_rows, C, rpb, sums, [&](int64_t r, int c, float v[1]) { v[0] = to_f(x[r * C + c]); });
 }
 
-template <typename T>
+// DROP: dz is multiplied by keep * scale first (dropout between this normalisation and its consumer, scale = 1 / (1 - p))
+template <typename T, bool DROP = false>
 __global__ void __launch_bounds__(256)
 bn_bwd_reduce_kernel(const T *__restrict__ dz, const T *__restrict__ y, int64_t n_rows, int C, int rpb,
                      const float *__restrict__ mi, const float *__restrict__ gamma, const float *__restrict__ beta,
-                     int act, float slope, double *sums) {
+                     int act, float slope, double *sums, const uint8_t *__restrict__ keep_bits = nullptr, float scale = 1.f) {
   col_reduce_body<2>(n_rows, C, rpb, sums, [&](int64_t r, int c, float v[2]) {
     const float xh = (to_f(y[r * C + c]) - mi[c]) * mi[C + c];
     const float pre = gamma[c] * xh + beta[c];
-    const float g = to_f(dz[r * C + c]) * act_bwd(pre, act, slope);
+    float d = to_f(dz[r * C + c]);
+    if constexpr (DROP) {
+      const int64_t e = r * C + c;
+      d = (keep_bits[e >> 3] >> (e & 7) & 1) ? d * scale : 0.f;
+    }
+    const float g = d * act_bwd(pre, act, slope);
     v[0] = g;
     v[1] = g * xh;
   });
@@ -303,11 +326,11 @@ struct BnC8 {
   }
 };
 
-template <typename T, int ACT, int U = 4>
+template <typename T, int ACT, bool DROP = false, int U = 4>
 __global__ void __launch_bounds__(256, 2)
 bn_bwd_reduce8_kernel(const T *__restrict__ dz, const T *__restrict__ y, int64_t n_rows, int C, int rpb,
                       const float *__restrict__ mi, const float *__restrict__ gamma, const float *__restrict__ beta, int act,
-                      float slope, double *sums) {
+                      float slope, double *sums, const uint8_t *__restrict__ keep_bits = nullptr, float scale = 1.f) {
   const int c0 = (threadIdx.x % (C >> 3)) * 8;
   struct { float a[8], b[8], invstd[8], nm[8]; } k8;  // only what the streaming loop needs (register budget: 2 blocks/SM)
 #pragma unroll
@@ -319,13 +342,22 @@ bn_bwd_reduce8_kernel(const T *__restrict__ dz, const T *__restrict__ y, int64_t
     k8.b[k] = beta[c0 + k] - mean * k8.a[k];
   }
   constexpr int NV = (int)sizeof(T) / 2;
-  col_reduce8_body<2, U, 2 * NV>(
+  // DROP: the row's keep byte (its 8 channels) travels as one more raw slot, fetched together with the row's data
+  col_reduce8_body<2, U, 2 * NV + DROP>(
       n_rows, C, sums,
-      [&](int64_t r, uint4 *raw) { load8raw(y + r * C + c0, raw); load8raw(dz + r * C + c0, raw + NV); },
+      [&](int64_t r, uint4 *raw) {
+        load8raw(y + r * C + c0, raw);
+        load8raw(dz + r * C + c0, raw + NV);
+        if constexpr (DROP) raw[2 * NV].x = keep_bits[(r * C + c0) >> 3];
+      },
       [&](int64_t, const uint4 *raw, float (&v)[2][8]) {
         float yy[8], dd[8];
         unpack8<T>(raw, yy);
         unpack8<T>(raw + NV, dd);
+        if constexpr (DROP) {
+#pragma unroll
+          for (int k = 0; k < 8; ++k) dd[k] = (raw[2 * NV].x >> k & 1u) ? dd[k] * scale : 0.f;
+        }
 #pragma unroll
         for (int k = 0; k < 8; ++k) {
           // streams sum g and sum g*y; sum g*xhat = invstd * sum g*y - mean*invstd * sum g is applied to the totals
@@ -341,16 +373,21 @@ bn_bwd_reduce8_kernel(const T *__restrict__ dz, const T *__restrict__ y, int64_t
 }
 
 // The elementwise kernels walk the tensor with a stride that is a multiple of C, so a thread always sees the same 8 channels.
-template <typename T>
+// DROP: dropout after the activation (no residual): z = keep ? act(.) * scale : 0, and thread i writes keep byte i (the
+// keep bits of its 8 elements), so consecutive threads write consecutive bytes.
+template <typename T, bool DROP = false>
 __global__ void __launch_bounds__(256)
 bn_apply8_kernel(const T *__restrict__ y, T *__restrict__ z, int64_t total8, int C, const float *__restrict__ mi,
                  const float *__restrict__ gamma, const float *__restrict__ beta, int act, float slope,
-                 const T *__restrict__ residual) {
+                 const T *__restrict__ residual, uint8_t *__restrict__ keep_bits = nullptr,
+                 const int64_t *__restrict__ seed_dev = nullptr, uint64_t thresh = 0, float scale = 1.f) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   const int c0 = (int)((i * 8) % C);
   BnC8 k8;
   k8.load(mi, gamma, beta, C, c0);
+  uint64_t seed = 0;
+  if constexpr (DROP) seed = (uint64_t)*seed_dev;
   for (; i < total8; i += 2 * stride) {
     const int64_t e0 = i * 8, e1 = (i + stride) * 8;
     const bool two = i + stride < total8;
@@ -364,6 +401,16 @@ bn_apply8_kernel(const T *__restrict__ y, T *__restrict__ z, int64_t total8, int
       float t1 = act_fwd(fmaf(k8.a[k], v1.v[k], k8.b[k]), act, slope);
       if (residual) { t0 += r0.v[k]; t1 += r1.v[k]; }
       v0.v[k] = t0; v1.v[k] = t1;
+    }
+    if constexpr (DROP) {
+      const uint32_t kb0 = dropout_keep8((uint64_t)e0, seed, thresh), kb1 = two ? dropout_keep8((uint64_t)e1, seed, thresh) : 0u;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        v0.v[k] = (kb0 >> k & 1u) ? v0.v[k] * scale : 0.f;
+        v1.v[k] = (kb1 >> k & 1u) ? v1.v[k] * scale : 0.f;
+      }
+      keep_bits[i] = (uint8_t)kb0;
+      if (two) keep_bits[i + stride] = (uint8_t)kb1;
     }
     v0.store(z + e0);
     if (two) v1.store(z + e1);
@@ -409,11 +456,12 @@ bn_apply_pad8_kernel(const T *__restrict__ y, T *__restrict__ zp, int X, int Y, 
   }
 }
 
-template <typename T, int ACT>
+template <typename T, int ACT, bool DROP = false>
 __global__ void __launch_bounds__(256, 3)
 bn_bwd_apply8_kernel(const T *__restrict__ dz, const T *__restrict__ y, T *__restrict__ dy, int64_t total8, int C, double inv_n,
                      const float *__restrict__ mi, const float *__restrict__ gamma, const float *__restrict__ beta, int act,
-                     float slope, const double *__restrict__ sums, float *__restrict__ dgamma, float *__restrict__ dbeta, float acc) {
+                     float slope, const double *__restrict__ sums, float *__restrict__ dgamma, float *__restrict__ dbeta, float acc,
+                     const uint8_t *__restrict__ keep_bits = nullptr, float scale = 1.f) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
   if (blockIdx.x == 0) {  // the parameter gradients are the reduction's totals: dbeta = sum g, dgamma = sum g * xhat
@@ -435,6 +483,14 @@ bn_bwd_apply8_kernel(const T *__restrict__ dz, const T *__restrict__ y, T *__res
     y0.load(y + e0);
     d0.load(dz + e0);
     if (two) { y1.load(y + e1); d1.load(dz + e1); }
+    if constexpr (DROP) {
+      const uint32_t kb0 = keep_bits[i], kb1 = two ? keep_bits[i + stride] : 0u;
+#pragma unroll
+      for (int k = 0; k < 8; ++k) {
+        d0.v[k] = (kb0 >> k & 1u) ? d0.v[k] * scale : 0.f;
+        d1.v[k] = (kb1 >> k & 1u) ? d1.v[k] * scale : 0.f;
+      }
+    }
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
       const float xh0 = fmaf(y0.v[k], k8.invstd[k], k8.nm[k]), xh1 = fmaf(y1.v[k], k8.invstd[k], k8.nm[k]);
@@ -542,12 +598,36 @@ bn_apply_kernel(const T *__restrict__ y, T *__restrict__ z, int64_t total, int C
   }
 }
 
+// bn_apply + dropout for any C: thread j owns the 8 elements of keep byte j (the bits past the last element are 0)
 template <typename T>
+__global__ void __launch_bounds__(256)
+bn_apply_dropout_kernel(const T *__restrict__ y, T *__restrict__ z, uint8_t *__restrict__ keep_bits, int64_t total, int C,
+                        const float *__restrict__ mi, const float *__restrict__ gamma, const float *__restrict__ beta, int act,
+                        float slope, const int64_t *__restrict__ seed_dev, uint64_t thresh, float scale) {
+  const uint64_t seed = (uint64_t)*seed_dev;
+  const int64_t nbytes = (total + 7) >> 3;
+  for (int64_t j = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; j < nbytes; j += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t e0 = j * 8;
+    const int n = (int)mn<int64_t>(8, total - e0);
+    const uint32_t bits = dropout_keep8((uint64_t)e0, seed, thresh) & ((1u << n) - 1u);
+    int c = (int)(e0 % C);
+    for (int k = 0; k < n; ++k) {
+      float v = gamma[c] * ((to_f(y[e0 + k]) - mi[c]) * mi[C + c]) + beta[c];  // the arithmetic of bn_apply_kernel
+      v = act_fwd(v, act, slope);
+      z[e0 + k] = from_f<T>((bits >> k & 1u) ? v * scale : 0.f);
+      if (++c == C) c = 0;
+    }
+    keep_bits[j] = (uint8_t)bits;
+  }
+}
+
+template <typename T, bool DROP = false>
 __global__ void __launch_bounds__(256)
 bn_bwd_apply_kernel(const T *__restrict__ dz, const T *__restrict__ y, T *__restrict__ dy, int64_t total, int C,
                     double inv_n, const float *__restrict__ mi, const float *__restrict__ gamma,
                     const float *__restrict__ beta, int act, float slope, const double *__restrict__ sums,
-                    float *__restrict__ dgamma, float *__restrict__ dbeta, float acc) {
+                    float *__restrict__ dgamma, float *__restrict__ dbeta, float acc,
+                    const uint8_t *__restrict__ keep_bits = nullptr, float scale = 1.f) {
   if (blockIdx.x == 0) {
     for (int c = threadIdx.x; c < C; c += blockDim.x) {
       if (dbeta) dbeta[c] = (acc != 0.f ? dbeta[c] : 0.f) + (float)sums[c];
@@ -559,7 +639,9 @@ bn_bwd_apply_kernel(const T *__restrict__ dz, const T *__restrict__ y, T *__rest
     const float invstd = mi[C + c];
     const float xh = (to_f(y[i]) - mi[c]) * invstd;
     const float pre = gamma[c] * xh + beta[c];
-    const float g = to_f(dz[i]) * act_bwd(pre, act, slope);
+    float d = to_f(dz[i]);
+    if constexpr (DROP) d = (keep_bits[i >> 3] >> (i & 7) & 1) ? d * scale : 0.f;
+    const float g = d * act_bwd(pre, act, slope);
     const float mg = (float)(sums[c] * inv_n), mgx = (float)(sums[C + c] * inv_n);
     dy[i] = from_f<T>(gamma[c] * invstd * (g - mg - xh * mgx));
   }
@@ -634,6 +716,119 @@ using namespace cg;
 
 #define CG_DTYPE_OK(d, name) \
   if ((d) != CGAN3D_F32 && (d) != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, name ": unknown dtype %d", (d))
+
+// p -> (threshold, scale) of the keep law; false for p outside [0, 1].  scale is 0 at p = 1 (everything is dropped: the
+// outputs and gradients are 0, not 0 * inf).
+static bool dropout_consts(float p, uint64_t *thresh, float *scale) {
+  if (!(p >= 0.f && p <= 1.f)) return false;
+  *thresh = (uint64_t)floor((double)p * 4294967296.0);
+  *scale = p < 1.f ? (float)(1.0 / (1.0 - (double)p)) : 0.f;
+  return true;
+}
+
+// the activation as a template argument for the vec8 kernels (-1: runtime switch), then the dropout flag
+template <typename F>
+static void with_act_drop(int act, bool drop, F &&go) {
+  auto pick_act = [&](auto drop_tag) {
+    if (act == CGAN3D_ACT_RELU) go(std::integral_constant<int, CGAN3D_ACT_RELU>{}, drop_tag);
+    else if (act == CGAN3D_ACT_LRELU) go(std::integral_constant<int, CGAN3D_ACT_LRELU>{}, drop_tag);
+    else if (act == CGAN3D_ACT_NONE) go(std::integral_constant<int, CGAN3D_ACT_NONE>{}, drop_tag);
+    else go(std::integral_constant<int, -1>{}, drop_tag);
+  };
+  if (drop) pick_act(std::true_type{});
+  else pick_act(std::false_type{});
+}
+
+// keep_bits == nullptr: no dropout (the kernels' DROP = false instantiations)
+static int bn_backward_reduce_impl(const char *name, const void *dz, const void *y, int dtype, int64_t n_rows, int C,
+                                   const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
+                                   double *sums, const uint8_t *keep_bits, float scale, void *stream) {
+  CG_CHECK_ARG(dz && y && mean_invstd && gamma && beta && sums, "%s: NULL pointer", name);
+  CG_DTYPE_OK(dtype, "bn_backward_reduce");
+  CG_CHECK_SHAPE(n_rows > 0 && C > 0 && (C <= 256 || C % 256 == 0), "%s: bad sizes", name);
+  cudaStream_t st = as_stream(stream);
+  cudaError_t e = cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), st);
+  if (e != cudaSuccess) return cuda_fail(e, "bn_backward_reduce memset");
+  if (vec8_ok(C, dz, y)) {
+    ColGrid g8 = col_grid8(n_rows, C, 2);
+    with_act_drop(act, keep_bits != nullptr, [&](auto act_tag, auto drop_tag) {
+      constexpr int A = decltype(act_tag)::value;
+      constexpr bool D = decltype(drop_tag)::value;
+      if (dtype == CGAN3D_F32)
+        // fp32 with the keep byte: two rows in flight per thread instead of four fit the 128 registers without spilling
+        bn_bwd_reduce8_kernel<float, A, D, D ? 2 : 4><<<g8.blocks, 256, g8.smem, st>>>((const float *)dz, (const float *)y, n_rows, C,
+                                                                            g8.rows_per_block, mean_invstd, gamma, beta, act, slope,
+                                                                            sums, keep_bits, scale);
+      else
+        bn_bwd_reduce8_kernel<__nv_bfloat16, A, D><<<g8.blocks, 256, g8.smem, st>>>(
+            (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, n_rows, C, g8.rows_per_block, mean_invstd, gamma, beta, act, slope,
+            sums, keep_bits, scale);
+    });
+    CG_LAUNCH_CHECK("bn_backward_reduce(vec8)");
+    return 0;
+  }
+  ColGrid g = col_grid(n_rows, C, 2);
+  auto go = [&](auto drop_tag) {
+    constexpr bool D = decltype(drop_tag)::value;
+    if (dtype == CGAN3D_F32)
+      bn_bwd_reduce_kernel<float, D><<<g.blocks, 256, g.smem, st>>>((const float *)dz, (const float *)y, n_rows, C,
+                                                                    g.rows_per_block, mean_invstd, gamma, beta, act, slope, sums,
+                                                                    keep_bits, scale);
+    else
+      bn_bwd_reduce_kernel<__nv_bfloat16, D><<<g.blocks, 256, g.smem, st>>>((const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y,
+                                                                            n_rows, C, g.rows_per_block, mean_invstd, gamma,
+                                                                            beta, act, slope, sums, keep_bits, scale);
+  };
+  if (keep_bits) go(std::true_type{});
+  else go(std::false_type{});
+  CG_LAUNCH_CHECK("bn_backward_reduce");
+  return 0;
+}
+
+static int bn_backward_apply_impl(const char *name, const void *dz, const void *y, void *dy, int dtype, int64_t n_rows, int C,
+                                  const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
+                                  const double *sums, float *dgamma, float *dbeta, float grad_beta, const uint8_t *keep_bits,
+                                  float scale, void *stream) {
+  CG_CHECK_ARG(dz && y && dy && mean_invstd && gamma && beta && sums, "%s: NULL pointer", name);
+  CG_CHECK_ARG(grad_beta == 0.f || grad_beta == 1.f, "%s: grad_beta must be 0 (overwrite) or 1 (accumulate)", name);
+  CG_DTYPE_OK(dtype, "bn_backward_apply");
+  CG_CHECK_SHAPE(n_rows > 0 && C > 0, "%s: bad sizes", name);
+  cudaStream_t st = as_stream(stream);
+  const int64_t total = n_rows * C;
+  const double inv_n = 1.0 / (double)n_rows;
+  if (vec8_ok(C, dz, y, dy)) {
+    const int64_t t8 = total / 8;
+    with_act_drop(act, keep_bits != nullptr, [&](auto act_tag, auto drop_tag) {
+      constexpr int A = decltype(act_tag)::value;
+      constexpr bool D = decltype(drop_tag)::value;
+      if (dtype == CGAN3D_F32)
+        bn_bwd_apply8_kernel<float, A, D><<<ew_blocks(t8), 256, 0, st>>>((const float *)dz, (const float *)y, (float *)dy, t8, C,
+                                                                         inv_n, mean_invstd, gamma, beta, act, slope, sums, dgamma,
+                                                                         dbeta, grad_beta, keep_bits, scale);
+      else
+        bn_bwd_apply8_kernel<__nv_bfloat16, A, D><<<ew_blocks(t8), 256, 0, st>>>(
+            (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, (__nv_bfloat16 *)dy, t8, C, inv_n, mean_invstd, gamma, beta, act,
+            slope, sums, dgamma, dbeta, grad_beta, keep_bits, scale);
+    });
+    CG_LAUNCH_CHECK("bn_backward_apply(vec8)");
+    return 0;
+  }
+  auto go = [&](auto drop_tag) {
+    constexpr bool D = decltype(drop_tag)::value;
+    if (dtype == CGAN3D_F32)
+      bn_bwd_apply_kernel<float, D><<<ew_blocks(total), 256, 0, st>>>((const float *)dz, (const float *)y, (float *)dy, total, C,
+                                                                      inv_n, mean_invstd, gamma, beta, act, slope, sums, dgamma,
+                                                                      dbeta, grad_beta, keep_bits, scale);
+    else
+      bn_bwd_apply_kernel<__nv_bfloat16, D><<<ew_blocks(total), 256, 0, st>>>(
+          (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, (__nv_bfloat16 *)dy, total, C, inv_n, mean_invstd, gamma, beta,
+          act, slope, sums, dgamma, dbeta, grad_beta, keep_bits, scale);
+  };
+  if (keep_bits) go(std::true_type{});
+  else go(std::false_type{});
+  CG_LAUNCH_CHECK("bn_backward_apply");
+  return 0;
+}
 
 extern "C" {
 
@@ -756,80 +951,75 @@ int cgan3d_bn_apply_pad(const void *y, void *z_padded, int dtype, int B, int X, 
   return 0;
 }
 
-int cgan3d_bn_backward_reduce(const void *dz, const void *y, int dtype, int64_t n_rows, int C, const float *mean_invstd,
-                              const float *gamma, const float *beta, int act, float slope, double *sums, void *stream) {
-  CG_CHECK_ARG(dz && y && mean_invstd && gamma && beta && sums, "bn_backward_reduce: NULL pointer");
-  CG_DTYPE_OK(dtype, "bn_backward_reduce");
-  CG_CHECK_SHAPE(n_rows > 0 && C > 0 && (C <= 256 || C % 256 == 0), "bn_backward_reduce: bad sizes");
+int cgan3d_bn_apply_dropout(const void *y, void *z, uint8_t *keep_bits, int dtype, int64_t n_rows, int C,
+                            const float *mean_invstd, const float *gamma, const float *beta, int act, float slope, float p,
+                            const int64_t *seed_dev, void *stream) {
+  CG_CHECK_ARG(y && z && keep_bits && mean_invstd && gamma && beta && seed_dev, "bn_apply_dropout: NULL pointer");
+  CG_DTYPE_OK(dtype, "bn_apply_dropout");
+  CG_CHECK_SHAPE(n_rows >= 0 && C > 0, "bn_apply_dropout: bad sizes");
+  uint64_t thresh;
+  float scale;
+  if (!dropout_consts(p, &thresh, &scale)) return fail(CGAN3D_E_ARG, "bn_apply_dropout: p = %g is outside [0, 1]", (double)p);
+  const int64_t total = n_rows * C;
+  if (total == 0) return 0;
   cudaStream_t st = as_stream(stream);
-  cudaError_t e = cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), st);
-  if (e != cudaSuccess) return cuda_fail(e, "bn_backward_reduce memset");
-  if (vec8_ok(C, dz, y)) {
-    ColGrid g8 = col_grid8(n_rows, C, 2);
-    auto go = [&](auto act_tag) {
-      constexpr int A = decltype(act_tag)::value;
-      if (dtype == CGAN3D_F32)
-        bn_bwd_reduce8_kernel<float, A><<<g8.blocks, 256, g8.smem, st>>>((const float *)dz, (const float *)y, n_rows, C,
-                                                                         g8.rows_per_block, mean_invstd, gamma, beta, act, slope, sums);
-      else
-        bn_bwd_reduce8_kernel<__nv_bfloat16, A><<<g8.blocks, 256, g8.smem, st>>>(
-            (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, n_rows, C, g8.rows_per_block, mean_invstd, gamma, beta, act, slope, sums);
-    };
-    if (act == CGAN3D_ACT_RELU) go(std::integral_constant<int, CGAN3D_ACT_RELU>{});
-    else if (act == CGAN3D_ACT_LRELU) go(std::integral_constant<int, CGAN3D_ACT_LRELU>{});
-    else if (act == CGAN3D_ACT_NONE) go(std::integral_constant<int, CGAN3D_ACT_NONE>{});
-    else go(std::integral_constant<int, -1>{});
-    CG_LAUNCH_CHECK("bn_backward_reduce(vec8)");
+  if (vec8_ok(C, y, z)) {
+    const int64_t t8 = total / 8;
+    if (dtype == CGAN3D_F32)
+      bn_apply8_kernel<float, true><<<ew_blocks(t8), 256, 0, st>>>((const float *)y, (float *)z, t8, C, mean_invstd, gamma, beta, act,
+                                                                   slope, nullptr, keep_bits, seed_dev, thresh, scale);
+    else
+      bn_apply8_kernel<__nv_bfloat16, true><<<ew_blocks(t8), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, t8, C,
+                                                                           mean_invstd, gamma, beta, act, slope, nullptr, keep_bits,
+                                                                           seed_dev, thresh, scale);
+    CG_LAUNCH_CHECK("bn_apply_dropout(vec8)");
     return 0;
   }
-  ColGrid g = col_grid(n_rows, C, 2);
+  const int64_t nbytes = (total + 7) / 8;
   if (dtype == CGAN3D_F32)
-    bn_bwd_reduce_kernel<float><<<g.blocks, 256, g.smem, st>>>((const float *)dz, (const float *)y, n_rows, C,
-                                                               g.rows_per_block, mean_invstd, gamma, beta, act, slope, sums);
+    bn_apply_dropout_kernel<float><<<ew_blocks(nbytes), 256, 0, st>>>((const float *)y, (float *)z, keep_bits, total, C, mean_invstd,
+                                                                      gamma, beta, act, slope, seed_dev, thresh, scale);
   else
-    bn_bwd_reduce_kernel<__nv_bfloat16><<<g.blocks, 256, g.smem, st>>>((const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y,
-                                                                       n_rows, C, g.rows_per_block, mean_invstd, gamma,
-                                                                       beta, act, slope, sums);
-  CG_LAUNCH_CHECK("bn_backward_reduce");
+    bn_apply_dropout_kernel<__nv_bfloat16><<<ew_blocks(nbytes), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, keep_bits,
+                                                                              total, C, mean_invstd, gamma, beta, act, slope,
+                                                                              seed_dev, thresh, scale);
+  CG_LAUNCH_CHECK("bn_apply_dropout");
   return 0;
+}
+
+int cgan3d_bn_backward_reduce(const void *dz, const void *y, int dtype, int64_t n_rows, int C, const float *mean_invstd,
+                              const float *gamma, const float *beta, int act, float slope, double *sums, void *stream) {
+  return bn_backward_reduce_impl("bn_backward_reduce", dz, y, dtype, n_rows, C, mean_invstd, gamma, beta, act, slope, sums,
+                                 nullptr, 1.f, stream);
+}
+
+int cgan3d_bn_backward_reduce_dropout(const void *dz, const void *y, const uint8_t *keep_bits, int dtype, int64_t n_rows, int C,
+                                      const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
+                                      float p, double *sums, void *stream) {
+  uint64_t thresh;
+  float scale;
+  CG_CHECK_ARG(keep_bits, "bn_backward_reduce_dropout: NULL pointer");
+  if (!dropout_consts(p, &thresh, &scale)) return fail(CGAN3D_E_ARG, "bn_backward_reduce_dropout: p = %g is outside [0, 1]", (double)p);
+  return bn_backward_reduce_impl("bn_backward_reduce_dropout", dz, y, dtype, n_rows, C, mean_invstd, gamma, beta, act, slope, sums,
+                                 keep_bits, scale, stream);
 }
 
 int cgan3d_bn_backward_apply(const void *dz, const void *y, void *dy, int dtype, int64_t n_rows, int C,
                              const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
                              const double *sums, float *dgamma, float *dbeta, float grad_beta, void *stream) {
-  CG_CHECK_ARG(dz && y && dy && mean_invstd && gamma && beta && sums, "bn_backward_apply: NULL pointer");
-  CG_CHECK_ARG(grad_beta == 0.f || grad_beta == 1.f, "bn_backward_apply: grad_beta must be 0 (overwrite) or 1 (accumulate)");
-  CG_DTYPE_OK(dtype, "bn_backward_apply");
-  CG_CHECK_SHAPE(n_rows > 0 && C > 0, "bn_backward_apply: bad sizes");
-  cudaStream_t st = as_stream(stream);
-  const int64_t total = n_rows * C;
-  const double inv_n = 1.0 / (double)n_rows;
-  if (vec8_ok(C, dz, y, dy)) {
-    const int64_t t8 = total / 8;
-    auto go = [&](auto act_tag) {
-      constexpr int A = decltype(act_tag)::value;
-      if (dtype == CGAN3D_F32)
-        bn_bwd_apply8_kernel<float, A><<<ew_blocks(t8), 256, 0, st>>>((const float *)dz, (const float *)y, (float *)dy, t8, C, inv_n,
-                                                                      mean_invstd, gamma, beta, act, slope, sums, dgamma, dbeta, grad_beta);
-      else
-        bn_bwd_apply8_kernel<__nv_bfloat16, A><<<ew_blocks(t8), 256, 0, st>>>((const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y,
-                                                                              (__nv_bfloat16 *)dy, t8, C, inv_n, mean_invstd, gamma,
-                                                                              beta, act, slope, sums, dgamma, dbeta, grad_beta);
-    };
-    if (act == CGAN3D_ACT_RELU) go(std::integral_constant<int, CGAN3D_ACT_RELU>{});
-    else if (act == CGAN3D_ACT_LRELU) go(std::integral_constant<int, CGAN3D_ACT_LRELU>{});
-    else if (act == CGAN3D_ACT_NONE) go(std::integral_constant<int, CGAN3D_ACT_NONE>{});
-    else go(std::integral_constant<int, -1>{});
-    CG_LAUNCH_CHECK("bn_backward_apply(vec8)");
-  } else if (dtype == CGAN3D_F32)
-    bn_bwd_apply_kernel<float><<<ew_blocks(total), 256, 0, st>>>((const float *)dz, (const float *)y, (float *)dy, total, C,
-                                                                 inv_n, mean_invstd, gamma, beta, act, slope, sums, dgamma, dbeta, grad_beta);
-  else
-    bn_bwd_apply_kernel<__nv_bfloat16><<<ew_blocks(total), 256, 0, st>>>(
-        (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, (__nv_bfloat16 *)dy, total, C, inv_n, mean_invstd, gamma, beta,
-        act, slope, sums, dgamma, dbeta, grad_beta);
-  CG_LAUNCH_CHECK("bn_backward_apply");
-  return 0;
+  return bn_backward_apply_impl("bn_backward_apply", dz, y, dy, dtype, n_rows, C, mean_invstd, gamma, beta, act, slope, sums,
+                                dgamma, dbeta, grad_beta, nullptr, 1.f, stream);
+}
+
+int cgan3d_bn_backward_apply_dropout(const void *dz, const void *y, const uint8_t *keep_bits, void *dy, int dtype, int64_t n_rows,
+                                     int C, const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
+                                     float p, const double *sums, float *dgamma, float *dbeta, float grad_beta, void *stream) {
+  uint64_t thresh;
+  float scale;
+  CG_CHECK_ARG(keep_bits, "bn_backward_apply_dropout: NULL pointer");
+  if (!dropout_consts(p, &thresh, &scale)) return fail(CGAN3D_E_ARG, "bn_backward_apply_dropout: p = %g is outside [0, 1]", (double)p);
+  return bn_backward_apply_impl("bn_backward_apply_dropout", dz, y, dy, dtype, n_rows, C, mean_invstd, gamma, beta, act, slope,
+                                sums, dgamma, dbeta, grad_beta, keep_bits, scale, stream);
 }
 
 int cgan3d_bias_act(const void *y, void *z, int dtype, int64_t n_rows, int C, const float *bias, int act, float slope,

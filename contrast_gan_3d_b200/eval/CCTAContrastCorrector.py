@@ -3,7 +3,9 @@
 
 The int16 volume is uploaded once; tiling, int16->f32 scaling, stitching (average where tiles overlap) and the
 HU unscale are device kernels.  Like the reference, the generator is NOT switched to eval mode: BatchNorm uses the
-statistics of the tiles sharing a batch (SURVEY §8a, a14) and tiles go through in row-major (x, y, z) order."""
+statistics of the tiles sharing a batch (SURVEY §8a, a14) and tiles go through in row-major (x, y, z) order.
+For the same reason a generator built with resnet_dropout_prob > 0 keeps its dropout active here: two calls on the same
+volume give different corrections, and torch.manual_seed before a call reproduces it."""
 from __future__ import annotations
 
 from dataclasses import dataclass, field

@@ -88,14 +88,16 @@ class ConvBlock(nn.Module):
                                  pad=padding, reflect=padding_mode == "reflect", out_pad=output_padding)
         self.compute_dtype = kwargs.get("compute_dtype", torch.float32)
 
-    def forward_cl(self, x: Tensor, residual: Optional[Tensor] = None, pad_out: int = 0) -> Tensor:
+    def forward_cl(self, x: Tensor, residual: Optional[Tensor] = None, pad_out: int = 0, dropout: float = 0.0):
         """pad_out > 0 returns the output with the reflection padding of its consumer already applied (fused into the
-        normalise + activation pass); the consumer must then be told that its input is pre-padded."""
+        normalise + activation pass); the consumer must then be told that its input is pre-padded.
+        dropout = p > 0 (BatchNorm blocks) applies nn.Dropout(p) to the output in the same pass and returns
+        (output, keep bitmask) (ops.ConvBlockFn)."""
         bn = self.normalization if isinstance(self.normalization, nn.BatchNorm3d) else None
         cfg = ops.BlockCfg(spec=self.spec, act=self.act_code, slope=self.negative_slope, dtype=self.compute_dtype,
                            training=self.training or (bn is not None and not bn.track_running_stats),
                            momentum=0.1 if bn is None or bn.momentum is None else bn.momentum,
-                           eps=1e-5 if bn is None else bn.eps, pad_out=pad_out)
+                           eps=1e-5 if bn is None else bn.eps, pad_out=pad_out, dropout=dropout)
         if bn is not None:
             return ops.ConvBlockFn.apply(x, self.conv.weight, None, bn.weight, bn.bias, residual, bn.running_mean,
                                          bn.running_var, bn.num_batches_tracked, cfg)
@@ -133,21 +135,34 @@ class ConvBlock(nn.Module):
 
 
 class ResNetBlock(nn.Module):
+    """x + block1(dropout(block0(x))) (reference model/blocks.py:56-88).
+
+    dropout_prob > 0: `self.dropout` is nn.Dropout(dropout_prob) (parameter-free: the state_dict is that of p = 0) and,
+    while it is in train mode, runs fused into block0's normalise pass.  `self.dropout_mask` holds the keep bitmask of the
+    last forward that drew one (uint8, bit e & 7 of byte e >> 3 for the channels-last index e of block0's output), else
+    None; under a CUDA graph it is the graph's static tensor, rewritten by every replay."""
+
     def __init__(self, is_2D: bool, channels_in: int, channels_out: int, kernel_size: int = 3,
                  dropout_prob: float = 0.0, padding_mode: str = "zeros", **kwargs):
         super().__init__()
         padding_amount = 1
         self.block0 = ConvBlock(is_2D, channels_in, channels_out, kernel_size, padding_mode=padding_mode,
                                 padding=padding_amount, activation_fn=nn.Identity, **kwargs)
-        if dropout_prob > 0:
-            raise NotImplementedError("resnet_dropout_prob > 0 is not on the hot path (reference default is 0)")
-        self.dropout = nn.Identity()
+        # nn.Dropout rejects p outside [0, 1] with torch's ValueError
+        self.dropout = nn.Dropout(dropout_prob) if dropout_prob != 0 else nn.Identity()
+        if isinstance(self.dropout, nn.Dropout) and not isinstance(self.block0.normalization, nn.BatchNorm3d):
+            raise NotImplementedError("ResNet dropout is fused into block0's BatchNorm pass; blocks without BatchNorm have none")
+        self.dropout_mask: Optional[Tensor] = None
         self.block1 = ConvBlock(is_2D, channels_out, channels_out, kernel_size, padding_mode=padding_mode,
                                 padding=padding_amount, **kwargs)
 
     def forward_cl(self, x: Tensor) -> Tensor:
-        # x + block1(dropout(block0(x))): the skip add is fused into block1's normalise/activate pass
-        return self.block1.forward_cl(self.block0.forward_cl(x), residual=x)
+        # x + block1(dropout(block0(x))): the dropout is fused into block0's normalise pass, the skip add into block1's
+        if isinstance(self.dropout, nn.Dropout) and self.dropout.training and self.dropout.p > 0:
+            h, self.dropout_mask = self.block0.forward_cl(x, dropout=self.dropout.p)
+        else:
+            h = self.block0.forward_cl(x)
+        return self.block1.forward_cl(h, residual=x)
 
     def forward(self, x: Tensor) -> Tensor:
         return from_channels_last(self.forward_cl(to_channels_last(x)).float())

@@ -310,11 +310,17 @@ class BlockCfg:
     eps: float = 1e-5
     pad_out: int = 0          # > 0: return reflect_pad(output, pad_out) -- the padding of the consumer, fused into the normalise pass
     pre_padded: bool = False  # the input already carries this layer's reflection padding (produced with pad_out)
+    dropout: float = 0.0      # > 0: element-wise dropout after the activation (BatchNorm blocks, no residual / pad_out)
 
 
 class ConvBlockFn(torch.autograd.Function):
     """act(norm(conv(x))) [+ residual]  — reference ConvBlock.forward (model/blocks.py:52-53) and the
-    skip connection of ResNetBlock.forward (:87-88), as one autograd node."""
+    skip connection of ResNetBlock.forward (:87-88), as one autograd node.
+
+    With cfg.dropout = p > 0 the node also applies nn.Dropout(p) to its output (the dropout of ResNetBlock, :68-88), fused
+    into the normalise pass, and returns (output, keep bitmask): uint8 [ceil(numel / 8)], bit e & 7 of byte e >> 3 set
+    when the channels-last element e was kept.  The mask's seed is drawn from torch's CUDA generator on the device, one
+    per call, so torch.manual_seed reproduces the masks and every replay of a captured CUDA graph draws new ones."""
 
     @staticmethod
     def forward(ctx, x, weight, bias, gamma, beta, residual, running_mean, running_var, nbt, cfg: BlockCfg):
@@ -334,7 +340,7 @@ class ConvBlockFn(torch.autograd.Function):
             y, sums = conv_bnstats(g, xin, wp, spec.transposed)  # batch statistics from the conv epilogue
         else:
             y = conv_scatter(g, xin, wp) if spec.transposed else conv_gather(g, xin, wp)
-        mi = None
+        mi = keep = None
         padded = False
         if gamma is not None:
             mi = torch.empty(2 * Co, dtype=torch.float32, device=x.device)
@@ -350,7 +356,15 @@ class ConvBlockFn(torch.autograd.Function):
             if residual is not None:
                 res = cast(residual.detach().contiguous(), cfg.dtype)
             po = cfg.pad_out
-            if po and res is None and not cfg.out_f32 and Co % 8 == 0:
+            if cfg.dropout > 0:
+                if res is not None or po:
+                    raise NotImplementedError("dropout is fused only into a block without residual or padded output")
+                seed = torch.randint(-2 ** 63, 2 ** 63 - 1, (1,), dtype=torch.int64, device=x.device)
+                keep = torch.empty((y.numel() + 7) // 8, dtype=torch.uint8, device=y.device)
+                z = torch.empty_like(y)
+                call("cgan3d_bn_apply_dropout", _p(y), _p(z), _p(keep), dt, n_rows, Co, _p(mi), _p(gamma.detach()),
+                     _p(beta.detach()), cfg.act, cfg.slope, cfg.dropout, _p(seed), _st())
+            elif po and res is None and not cfg.out_f32 and Co % 8 == 0:
                 # normalise + activate straight into the consumer's reflection-padded input
                 z = torch.empty((B, out_sp[0] + 2 * po, out_sp[1] + 2 * po, out_sp[2] + 2 * po, Co), dtype=y.dtype, device=y.device)
                 call("cgan3d_bn_apply_pad", _p(y), _p(z), dt, B, out_sp[0], out_sp[1], out_sp[2], Co, _p(mi), _p(gamma.detach()),
@@ -362,6 +376,8 @@ class ConvBlockFn(torch.autograd.Function):
                      cfg.act, cfg.slope, _p(res), _st())
         else:
             assert residual is None
+            if cfg.dropout > 0:
+                raise NotImplementedError("dropout is fused only into BatchNorm blocks")
             if bias is None and cfg.act == _lib.ACT_NONE:
                 z = y
             else:
@@ -383,14 +399,17 @@ class ConvBlockFn(torch.autograd.Function):
         ctx.has_res = residual is not None
         ctx.res_dtype = None if residual is None else residual.dtype
         ctx.in_spatial = (X, Y, Z)
-        ctx.save_for_backward(xin, wp, y, mi, gamma, beta, bias)
+        ctx.save_for_backward(xin, wp, y, mi, gamma, beta, bias, keep)
+        if keep is not None:
+            ctx.mark_non_differentiable(keep)
+            return z, keep
         return z
 
     @staticmethod
-    def backward(ctx, dz):
+    def backward(ctx, dz, *_):
         cfg, g = ctx.cfg, ctx.g
         spec = cfg.spec
-        xin, wp, y, mi, gamma, beta, bias = ctx.saved_tensors
+        xin, wp, y, mi, gamma, beta, bias, keep = ctx.saved_tensors
         dt = _dt(cfg.dtype)
         dz = cast(dz.contiguous(), cfg.dtype)
         if cfg.pad_out:
@@ -402,8 +421,12 @@ class ConvBlockFn(torch.autograd.Function):
             if not cfg.training:
                 raise NotImplementedError("backward through eval-mode BatchNorm is not part of the hot path")
             sums = torch.empty(2 * Co, dtype=torch.float64, device=y.device)
-            call("cgan3d_bn_backward_reduce", _p(dz), _p(y), dt, n_rows, Co, _p(mi), _p(gamma), _p(beta), cfg.act,
-                 cfg.slope, _p(sums), _st())
+            if keep is not None:
+                call("cgan3d_bn_backward_reduce_dropout", _p(dz), _p(y), _p(keep), dt, n_rows, Co, _p(mi), _p(gamma), _p(beta),
+                     cfg.act, cfg.slope, cfg.dropout, _p(sums), _st())
+            else:
+                call("cgan3d_bn_backward_reduce", _p(dz), _p(y), dt, n_rows, Co, _p(mi), _p(gamma), _p(beta), cfg.act,
+                     cfg.slope, _p(sums), _st())
             dy = torch.empty_like(y)
             pbias, pgamma, pbeta = ctx.small_params
             # parameter gradients: accumulated into the gradient bucket by the same launch when a sink is active
@@ -412,8 +435,12 @@ class ConvBlockFn(torch.autograd.Function):
             if not direct:
                 tg = torch.empty(Co, dtype=torch.float32, device=y.device)
                 tb = torch.empty(Co, dtype=torch.float32, device=y.device)
-            call("cgan3d_bn_backward_apply", _p(dz), _p(y), _p(dy), dt, n_rows, Co, _p(mi), _p(gamma), _p(beta),
-                 cfg.act, cfg.slope, _p(sums), _p(tg), _p(tb), 1.0 if direct else 0.0, _st())
+            if keep is not None:
+                call("cgan3d_bn_backward_apply_dropout", _p(dz), _p(y), _p(keep), _p(dy), dt, n_rows, Co, _p(mi), _p(gamma),
+                     _p(beta), cfg.act, cfg.slope, cfg.dropout, _p(sums), _p(tg), _p(tb), 1.0 if direct else 0.0, _st())
+            else:
+                call("cgan3d_bn_backward_apply", _p(dz), _p(y), _p(dy), dt, n_rows, Co, _p(mi), _p(gamma), _p(beta),
+                     cfg.act, cfg.slope, _p(sums), _p(tg), _p(tb), 1.0 if direct else 0.0, _st())
             _grad_handled(pgamma, direct)
             _grad_handled(pbeta, direct)
             dgamma, dbeta = (None, None) if direct else (tg, tb)

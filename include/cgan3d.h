@@ -132,11 +132,25 @@ int cgan3d_bn_apply(const void *y, void *z, int dtype, int64_t n_rows, int C, co
 int cgan3d_bn_apply_pad(const void *y, void *z_padded, int dtype, int B, int X, int Y, int Z, int C,
                         const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
                         int pad, void *stream);
+/* bn_apply followed by the ResNet block's dropout (nn.Dropout(p) between block0 and block1, reference
+ * model/blocks.py:68-88, in train mode): z = keep ? act(gamma * (y - mean) * invstd + beta) / (1 - p) : 0 in fp32, rounded
+ * once; no residual.  keep_bits (ceil(n_rows * C / 8) bytes) receives bit e & 7 of byte e >> 3 = keep(e) for the
+ * channels-last linear index e.  Keep law: keep(e) <=> u >= floor(p * 2^32), u = word e & 3 of Philox4x32-10 with key
+ * (lo32 seed, hi32 seed) and counter (lo32(e >> 2), hi32(e >> 2), 0, 0); p in [0, 1] (as fp32), p = 1 writes zeros.  The
+ * 64-bit seed is read from device memory (*seed_dev), so the call can be captured in a CUDA graph.                    */
+int cgan3d_bn_apply_dropout(const void *y, void *z, uint8_t *keep_bits, int dtype, int64_t n_rows, int C,
+                            const float *mean_invstd, const float *gamma, const float *beta, int act, float slope, float p,
+                            const int64_t *seed_dev, void *stream);
 /* backward of bn_apply (train mode): given dz, y -> dy, dgamma, dbeta.
  * Pass 1 (reduce): sums[0..C) = sum g, sums[C..2C) = sum g*xhat, g = dz * act'(.)          */
 int cgan3d_bn_backward_reduce(const void *dz, const void *y, int dtype, int64_t n_rows, int C,
                               const float *mean_invstd, const float *gamma, const float *beta, int act,
                               float slope, double *sums, void *stream);
+/* the same through bn_apply_dropout (the dropout backward of reference model/blocks.py:68-88 fused in):
+ * g = dz * keep / (1 - p) * act'(.), keep read from the bitmask that bn_apply_dropout wrote                             */
+int cgan3d_bn_backward_reduce_dropout(const void *dz, const void *y, const uint8_t *keep_bits, int dtype, int64_t n_rows,
+                                      int C, const float *mean_invstd, const float *gamma, const float *beta, int act,
+                                      float slope, float p, double *sums, void *stream);
 /* Pass 2: dy = gamma*invstd*(g - sum_g/n - xhat*sum_gx/n); the same launch writes the parameter gradients dgamma = sum
  * g*xhat, dbeta = sum g (fp32 [C], may be NULL): grad_beta = 0 overwrites them, 1 accumulates into them (the caller's
  * gradient buffer: a layer applied twice per backward, reference trainer/Trainer.py:114-116).                          */
@@ -144,6 +158,11 @@ int cgan3d_bn_backward_apply(const void *dz, const void *y, void *dy, int dtype,
                              const float *mean_invstd, const float *gamma, const float *beta, int act,
                              float slope, const double *sums, float *dgamma, float *dbeta, float grad_beta,
                              void *stream);
+/* pass 2 through bn_apply_dropout (reference model/blocks.py:68-88): g as in cgan3d_bn_backward_reduce_dropout */
+int cgan3d_bn_backward_apply_dropout(const void *dz, const void *y, const uint8_t *keep_bits, void *dy, int dtype,
+                                     int64_t n_rows, int C, const float *mean_invstd, const float *gamma,
+                                     const float *beta, int act, float slope, float p, const double *sums, float *dgamma,
+                                     float *dbeta, float grad_beta, void *stream);
 /* bias + activation without norm (critic first layer, blocks.py:34 bias=True under Identity norm):
  * z = act(y + bias); backward: dy = dz * act'(y + bias), dbias = sum dy                     */
 int cgan3d_bias_act(const void *y, void *z, int dtype, int64_t n_rows, int C, const float *bias, int act,
