@@ -24,6 +24,11 @@ int cuda_fail(cudaError_t e, const char *where);
   do {                                                  \
     if (!(cond)) return cg::fail(CGAN3D_E_SHAPE, __VA_ARGS__); \
   } while (0)
+#define CG_CHECK_DTYPE(dtype, name)                                           \
+  do {                                                                        \
+    if ((dtype) != CGAN3D_F32 && (dtype) != CGAN3D_BF16)                      \
+      return cg::fail(CGAN3D_E_DTYPE, "%s: unknown dtype %d", name, (dtype)); \
+  } while (0)
 #define CG_LAUNCH_CHECK(where)                          \
   do {                                                  \
     cudaError_t e__ = cudaGetLastError();               \
@@ -31,6 +36,18 @@ int cuda_fail(cudaError_t e, const char *where);
   } while (0)
 
 static inline cudaStream_t as_stream(void *s) { return reinterpret_cast<cudaStream_t>(s); }
+
+// with_dtype(dtype, f) calls f with the tensor element type of a checked dtype (CGAN3D_F32 -> float, else bf16) as a tag,
+// so a launch is written once: [&](auto t) { using T = typename decltype(t)::type; kernel<T><<<...>>>((const T *)p, ...); }
+template <typename T>
+struct type_tag {
+  using type = T;
+};
+template <typename F>
+static inline auto with_dtype(int dtype, F &&f) {
+  if (dtype == CGAN3D_F32) return f(type_tag<float>{});
+  return f(type_tag<bf16>{});
+}
 
 __device__ __forceinline__ float to_f(float v) { return v; }
 __device__ __forceinline__ float to_f(__nv_bfloat16 v) { return __bfloat162float(v); }
@@ -112,5 +129,8 @@ __host__ __device__ __forceinline__ T mn(T a, T b) { return a < b ? a : b; }
 template <typename T>
 __host__ __device__ __forceinline__ T mx(T a, T b) { return a > b ? a : b; }
 static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
+
+// blocks of 256 threads for the grid-strided element-wise kernels over n items: one item per thread, at most 16 blocks per SM
+static inline int ew_blocks(int64_t n) { return (int)mx<int64_t>(1, mn<int64_t>((n + 255) / 256, (int64_t)num_sms() * 16)); }
 
 }  // namespace cg

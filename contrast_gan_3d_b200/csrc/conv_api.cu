@@ -6,7 +6,7 @@ namespace cg {
 
 static int check_geom(const cgan3d_conv_geom *g, int dtype) {
   CG_CHECK_ARG(g != nullptr, "conv: geometry is NULL");
-  if (dtype != CGAN3D_F32 && dtype != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, "conv: unknown dtype %d", dtype);
+  CG_CHECK_DTYPE(dtype, "conv");
   CG_CHECK_SHAPE(g->B >= 0 && g->Xb > 0 && g->Yb > 0 && g->Zb > 0 && g->Cb > 0 && g->Cs > 0, "conv: bad sizes");
   CG_CHECK_SHAPE(g->k >= 1 && g->k <= 7 && (g->stride == 1 || g->stride == 2) && g->pad >= 0 && g->pad < g->k,
                  "conv: k=%d stride=%d pad=%d unsupported", g->k, g->stride, g->pad);
@@ -101,7 +101,7 @@ extern "C" {
 
 int cgan3d_pack_weights(const float *w, void *packed, int dtype, int Cs, int Cb, int k, void *stream) {
   CG_CHECK_ARG(w && packed, "pack_weights: NULL pointer");
-  if (dtype != CGAN3D_F32 && dtype != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, "pack_weights: unknown dtype %d", dtype);
+  CG_CHECK_DTYPE(dtype, "pack_weights");
   CG_CHECK_SHAPE(Cs > 0 && Cb > 0 && k > 0 && k <= 7, "pack_weights: bad sizes");
   return pack_weights(w, packed, dtype, Cs, Cb, k, as_stream(stream));
 }
@@ -182,7 +182,7 @@ int cgan3d_conv_wgrad(const cgan3d_conv_geom *g, int dtype, const void *big, con
 int cgan3d_reflect_pad(const void *in, void *out, int dtype, int B, int X, int Y, int Z, int C, int pad,
                        void *stream) {
   CG_CHECK_ARG(in && out, "reflect_pad: NULL pointer");
-  if (dtype != CGAN3D_F32 && dtype != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, "reflect_pad: unknown dtype");
+  CG_CHECK_DTYPE(dtype, "reflect_pad");
   CG_CHECK_SHAPE(pad >= 0 && pad < X && pad < Y && pad < Z && C > 0 && B >= 0,
                  "reflect_pad: pad %d must be smaller than every extent (%d,%d,%d)", pad, X, Y, Z);
   if (B == 0) return 0;
@@ -192,7 +192,7 @@ int cgan3d_reflect_pad(const void *in, void *out, int dtype, int B, int X, int Y
 int cgan3d_reflect_pad_backward(const void *padded_grad, void *in_grad, int dtype, int B, int X, int Y, int Z, int C,
                                 int pad, void *stream) {
   CG_CHECK_ARG(padded_grad && in_grad, "reflect_pad_backward: NULL pointer");
-  if (dtype != CGAN3D_F32 && dtype != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, "reflect_pad_backward: unknown dtype");
+  CG_CHECK_DTYPE(dtype, "reflect_pad_backward");
   CG_CHECK_SHAPE(pad >= 0 && pad < X && pad < Y && pad < Z && C > 0 && B >= 0, "reflect_pad_backward: bad pad");
   if (B == 0) return 0;
   return reflect_pad_backward(padded_grad, in_grad, dtype, B, X, Y, Z, C, pad, as_stream(stream));

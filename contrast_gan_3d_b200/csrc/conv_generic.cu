@@ -678,26 +678,12 @@ static int launch_wgrad(const cgan3d_conv_geom &g, const T *big, const T *small,
     }                                                                                 \
   } while (0)
 
-template <typename T>
-static int gather_t(const cgan3d_conv_geom &g, const void *big, const void *wp, const float *bias, void *small,
-                    cudaStream_t st) {
-  CG_KS_DISPATCH(launch_gather, g, (const T *)big, (const T *)wp, bias, (T *)small, st);
-}
-template <typename T>
-static int scatter_t(const cgan3d_conv_geom &g, const void *small, const void *wp, const float *bias, void *big,
-                     cudaStream_t st) {
-  CG_KS_DISPATCH(launch_scatter, g, (const T *)small, (const T *)wp, bias, (T *)big, st);
-}
-template <typename T>
-static int wgrad_t(const cgan3d_conv_geom &g, const void *big, const void *small, float *dw, float beta,
-                   cudaStream_t st) {
-  CG_KS_DISPATCH(launch_wgrad, g, (const T *)big, (const T *)small, dw, beta, st);
-}
-
 int generic_gather(const cgan3d_conv_geom &g, int dtype, const void *big, const void *wp, const float *bias,
                    void *small, cudaStream_t st) {
-  return dtype == CGAN3D_F32 ? gather_t<float>(g, big, wp, bias, small, st)
-                             : gather_t<__nv_bfloat16>(g, big, wp, bias, small, st);
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    CG_KS_DISPATCH(launch_gather, g, (const T *)big, (const T *)wp, bias, (T *)small, st);
+  });
 }
 // [tap][Cb][Cs] -> [taps-1-tap][Cs][Cb]
 template <typename T>
@@ -716,50 +702,45 @@ size_t generic_workspace_bytes(const cgan3d_conv_geom &g, int dtype, int op) {
   return 0;
 }
 
-template <typename T>
-static int scatter_tw_t(const cgan3d_conv_geom &g, const void *small, const void *wp, const float *bias, void *big, void *ws,
-                        cudaStream_t st) {
-  CG_KS_DISPATCH(launch_scatter_tw, g, (const T *)small, (const T *)wp, bias, (T *)big, (T *)ws, st);
-}
-
 int generic_scatter(const cgan3d_conv_geom &g, int dtype, const void *small, const void *wp, const float *bias,
                     void *big, void *ws, size_t ws_bytes, cudaStream_t st) {
-  if (g.stride == 1 && ws != nullptr && ws_bytes >= generic_workspace_bytes(g, dtype, 1) &&
-      (reinterpret_cast<uintptr_t>(ws) & 15) == 0) {
-    // dgrad of a stride-1 conv == conv of the small side with the flipped filter, pad' = k-1-pad (register-tiled gather)
-    const int taps = g.k * g.k * g.k;
-    const int64_t total = (int64_t)taps * g.Cb * g.Cs;
-    const int blocks = (int)mn<int64_t>((total + 255) / 256, 1024);
-    if (dtype == CGAN3D_F32)
-      flip_transpose_kernel<float><<<blocks, 256, 0, st>>>((const float *)wp, (float *)ws, g.Cb, g.Cs, taps);
-    else
-      flip_transpose_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16 *)wp, (__nv_bfloat16 *)ws, g.Cb, g.Cs, taps);
-    CG_LAUNCH_CHECK("flip_transpose");
-    cgan3d_conv_geom f = g;
-    f.Xb = g.Xs; f.Yb = g.Ys; f.Zb = g.Zs; f.Cb = g.Cs;
-    f.Xs = g.Xb; f.Ys = g.Yb; f.Zs = g.Zb; f.Cs = g.Cb;
-    f.pad = g.k - 1 - g.pad;
-    return generic_gather(f, dtype, small, ws, bias, big, st);
-  }
-  if (g.stride > 1 && g.Cb % 8 == 0 && ws != nullptr && ws_bytes >= generic_workspace_bytes(g, dtype, 1) &&
-      (reinterpret_cast<uintptr_t>(ws) & 15) == 0)
-    return dtype == CGAN3D_F32 ? scatter_tw_t<float>(g, small, wp, bias, big, ws, st)
-                               : scatter_tw_t<__nv_bfloat16>(g, small, wp, bias, big, ws, st);
-  return dtype == CGAN3D_F32 ? scatter_t<float>(g, small, wp, bias, big, st)
-                             : scatter_t<__nv_bfloat16>(g, small, wp, bias, big, st);
+  const bool ws_ok = ws != nullptr && ws_bytes >= generic_workspace_bytes(g, dtype, 1) && (reinterpret_cast<uintptr_t>(ws) & 15) == 0;
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (g.stride == 1 && ws_ok) {
+      // dgrad of a stride-1 conv == conv of the small side with the flipped filter, pad' = k-1-pad (register-tiled gather)
+      const int taps = g.k * g.k * g.k;
+      const int64_t total = (int64_t)taps * g.Cb * g.Cs;
+      const int blocks = (int)mn<int64_t>((total + 255) / 256, 1024);
+      flip_transpose_kernel<T><<<blocks, 256, 0, st>>>((const T *)wp, (T *)ws, g.Cb, g.Cs, taps);
+      CG_LAUNCH_CHECK("flip_transpose");
+      cgan3d_conv_geom f = g;
+      f.Xb = g.Xs; f.Yb = g.Ys; f.Zb = g.Zs; f.Cb = g.Cs;
+      f.Xs = g.Xb; f.Ys = g.Yb; f.Zs = g.Zb; f.Cs = g.Cb;
+      f.pad = g.k - 1 - g.pad;
+      return generic_gather(f, dtype, small, ws, bias, big, st);
+    }
+    if (g.stride > 1 && g.Cb % 8 == 0 && ws_ok)
+      CG_KS_DISPATCH(launch_scatter_tw, g, (const T *)small, (const T *)wp, bias, (T *)big, (T *)ws, st);
+    CG_KS_DISPATCH(launch_scatter, g, (const T *)small, (const T *)wp, bias, (T *)big, st);
+  });
 }
 int generic_wgrad(const cgan3d_conv_geom &g, int dtype, const void *big, const void *small, float *dw, float beta,
                   cudaStream_t st) {
-  return dtype == CGAN3D_F32 ? wgrad_t<float>(g, big, small, dw, beta, st)
-                             : wgrad_t<__nv_bfloat16>(g, big, small, dw, beta, st);
+  return with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    CG_KS_DISPATCH(launch_wgrad, g, (const T *)big, (const T *)small, dw, beta, st);
+  });
 }
 
 int pack_weights(const float *w, void *packed, int dtype, int Cs, int Cb, int k, cudaStream_t st) {
   const int taps = k * k * k;
   const int64_t total = (int64_t)taps * Cb * Cs;
   const int blocks = (int)mn<int64_t>((total + 255) / 256, 4096);
-  if (dtype == CGAN3D_F32) pack_weights_kernel<float><<<blocks, 256, 0, st>>>(w, (float *)packed, Cs, Cb, taps);
-  else pack_weights_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>(w, (__nv_bfloat16 *)packed, Cs, Cb, taps);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    pack_weights_kernel<T><<<blocks, 256, 0, st>>>(w, (T *)packed, Cs, Cb, taps);
+  });
   CG_LAUNCH_CHECK("pack_weights");
   return 0;
 }
@@ -907,26 +888,24 @@ int reflect_pad(const void *in, void *out, int dtype, int B, int X, int Y, int Z
     const dim3 grid((unsigned)Yp, (unsigned)Xp, (unsigned)B);
     if ((C * esz) % 16 == 0 && !((uintptr_t)in & 15) && !((uintptr_t)out & 15))
       reflect_pad_line_kernel<uint4><<<grid, 256, 0, st>>>((const uint4 *)in, (uint4 *)out, X, Y, Z, C * esz / 16, pad);
-    else if ((Z + 2 * pad) * C <= 512) {  // short lines: a warp per line
-      const dim3 gridw((unsigned)((Yp + 31) / 32), (unsigned)Xp, (unsigned)B);
-      if (dtype == CGAN3D_F32)
-        reflect_pad_warpline_kernel<float><<<gridw, 256, 0, st>>>((const float *)in, (float *)out, X, Y, Z, C, pad);
-      else
-        reflect_pad_warpline_kernel<__nv_bfloat16><<<gridw, 256, 0, st>>>((const __nv_bfloat16 *)in, (__nv_bfloat16 *)out, X, Y, Z, C, pad);
-    } else if (dtype == CGAN3D_F32)
-      reflect_pad_line_kernel<float><<<grid, 256, 0, st>>>((const float *)in, (float *)out, X, Y, Z, C, pad);
     else
-      reflect_pad_line_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>((const __nv_bfloat16 *)in, (__nv_bfloat16 *)out, X, Y, Z, C, pad);
+      with_dtype(dtype, [&](auto t) {
+        using T = typename decltype(t)::type;
+        if ((Z + 2 * pad) * C <= 512) {  // short lines: a warp per line
+          const dim3 gridw((unsigned)((Yp + 31) / 32), (unsigned)Xp, (unsigned)B);
+          reflect_pad_warpline_kernel<T><<<gridw, 256, 0, st>>>((const T *)in, (T *)out, X, Y, Z, C, pad);
+        } else
+          reflect_pad_line_kernel<T><<<grid, 256, 0, st>>>((const T *)in, (T *)out, X, Y, Z, C, pad);
+      });
     CG_LAUNCH_CHECK("reflect_pad(line)");
     return 0;
   }
   const int64_t total = (int64_t)B * (X + 2 * pad) * (Y + 2 * pad) * (Z + 2 * pad) * C;
   const int blocks = (int)mn<int64_t>((total + 255) / 256, (int64_t)num_sms() * 16);
-  if (dtype == CGAN3D_F32)
-    reflect_pad_kernel<float><<<blocks, 256, 0, st>>>((const float *)in, (float *)out, B, X, Y, Z, C, pad);
-  else
-    reflect_pad_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16 *)in, (__nv_bfloat16 *)out, B, X,
-                                                              Y, Z, C, pad);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    reflect_pad_kernel<T><<<blocks, 256, 0, st>>>((const T *)in, (T *)out, B, X, Y, Z, C, pad);
+  });
   CG_LAUNCH_CHECK("reflect_pad");
   return 0;
 }
@@ -934,25 +913,21 @@ int reflect_pad(const void *in, void *out, int dtype, int B, int X, int Y, int Z
 int reflect_pad_backward(const void *gp, void *gi, int dtype, int B, int X, int Y, int Z, int C, int pad,
                          cudaStream_t st) {
   const int esz = dtype == CGAN3D_F32 ? 4 : 2;
-  if ((C * esz) % 16 == 0 && !((uintptr_t)gp & 15) && !((uintptr_t)gi & 15) && X <= 65535 && B <= 65535) {
-    const int cpv = C * esz / 16;
-    const int lpb = (int64_t)B * X * Y >= 65536 && Z * cpv <= 512 ? 4 : 1;
-    const dim3 bl((unsigned)((Y + lpb - 1) / lpb), (unsigned)X, (unsigned)B);
-    if (dtype == CGAN3D_F32)
-      reflect_pad_bwd_vec_kernel<float><<<bl, 256, 0, st>>>((const uint4 *)gp, (uint4 *)gi, B, X, Y, Z, cpv, pad, lpb);
-    else
-      reflect_pad_bwd_vec_kernel<__nv_bfloat16><<<bl, 256, 0, st>>>((const uint4 *)gp, (uint4 *)gi, B, X, Y, Z, cpv, pad, lpb);
-    CG_LAUNCH_CHECK("reflect_pad_bwd_vec");
-    return 0;
-  }
-  const int64_t total = (int64_t)B * X * Y * Z * C;
-  const int blocks = (int)mn<int64_t>((total + 255) / 256, (int64_t)num_sms() * 16);
-  if (dtype == CGAN3D_F32)
-    reflect_pad_bwd_kernel<float><<<blocks, 256, 0, st>>>((const float *)gp, (float *)gi, B, X, Y, Z, C, pad);
-  else
-    reflect_pad_bwd_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16 *)gp, (__nv_bfloat16 *)gi, B,
-                                                                  X, Y, Z, C, pad);
-  CG_LAUNCH_CHECK("reflect_pad_backward");
+  const bool vec = (C * esz) % 16 == 0 && !((uintptr_t)gp & 15) && !((uintptr_t)gi & 15) && X <= 65535 && B <= 65535;
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (vec) {
+      const int cpv = C * esz / 16;
+      const int lpb = (int64_t)B * X * Y >= 65536 && Z * cpv <= 512 ? 4 : 1;
+      const dim3 bl((unsigned)((Y + lpb - 1) / lpb), (unsigned)X, (unsigned)B);
+      reflect_pad_bwd_vec_kernel<T><<<bl, 256, 0, st>>>((const uint4 *)gp, (uint4 *)gi, B, X, Y, Z, cpv, pad, lpb);
+    } else {
+      const int64_t total = (int64_t)B * X * Y * Z * C;
+      const int blocks = (int)mn<int64_t>((total + 255) / 256, (int64_t)num_sms() * 16);
+      reflect_pad_bwd_kernel<T><<<blocks, 256, 0, st>>>((const T *)gp, (T *)gi, B, X, Y, Z, C, pad);
+    }
+  });
+  CG_LAUNCH_CHECK(vec ? "reflect_pad_bwd_vec" : "reflect_pad_backward");
   return 0;
 }
 

@@ -344,8 +344,6 @@ scale_i16_kernel(const int16_t *__restrict__ hu, float *__restrict__ out, int64_
     for (int64_t i = (n8 << 3) + threadIdx.x; i < n; i += blockDim.x) out[i] = ((float)hu[i] - shift) / factor;
 }
 
-static inline int ew_blocks2(int64_t n) { return (int)mx<int64_t>(1, mn<int64_t>((n + 255) / 256, (int64_t)num_sms() * 16)); }
-
 }  // namespace cg
 
 using namespace cg;
@@ -377,22 +375,24 @@ int cgan3d_gen_loss_backward(const float *s, const float *t, const uint8_t *mask
                              const float *coef, const float *upstream, const float *d_extra, float *ds, void *stream) {
   CG_CHECK_ARG(s && t && coef && ds, "gen_loss_backward: NULL pointer");
   if (n <= 0) return 0;
-  gen_loss_backward_kernel<<<ew_blocks2(n), 256, 0, as_stream(stream)>>>(s, t, mask, n, hu_lo, hu_hi, coef, upstream,
-                                                                         d_extra, ds);
+  gen_loss_backward_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(s, t, mask, n, hu_lo, hu_hi, coef, upstream,
+                                                                        d_extra, ds);
   CG_LAUNCH_CHECK("gen_loss_backward");
   return 0;
 }
 
 int cgan3d_mean(const void *x, int dtype, int64_t n, float scale, double *scratch, float *out, void *stream) {
   CG_CHECK_ARG(x && scratch && out, "mean: NULL pointer");
-  if (dtype != CGAN3D_F32 && dtype != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, "mean: unknown dtype %d", dtype);
+  CG_CHECK_DTYPE(dtype, "mean");
   CG_CHECK_SHAPE(n > 0, "mean: empty tensor");
   cudaStream_t st = as_stream(stream);
   cudaError_t e = cudaMemsetAsync(scratch, 0, sizeof(double), st);
   if (e != cudaSuccess) return cuda_fail(e, "mean memset");
   const int blocks = (int)mx<int64_t>(1, mn<int64_t>((n + 255) / 256, (int64_t)num_sms() * 4));
-  if (dtype == CGAN3D_F32) sum_kernel<float><<<blocks, 256, 0, st>>>((const float *)x, n, scratch);
-  else sum_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16 *)x, n, scratch);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    sum_kernel<T><<<blocks, 256, 0, st>>>((const T *)x, n, scratch);
+  });
   CG_LAUNCH_CHECK("mean(sum)");
   mean_finalize_kernel<<<1, 32, 0, st>>>(scratch, n, scale, out);
   CG_LAUNCH_CHECK("mean(finalize)");
@@ -401,11 +401,13 @@ int cgan3d_mean(const void *x, int dtype, int64_t n, float scale, double *scratc
 
 int cgan3d_fill(void *x, int dtype, int64_t n, const float *value_dev, float scale, void *stream) {
   CG_CHECK_ARG(x, "fill: NULL pointer");
-  if (dtype != CGAN3D_F32 && dtype != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, "fill: unknown dtype %d", dtype);
+  CG_CHECK_DTYPE(dtype, "fill");
   if (n <= 0) return 0;
   cudaStream_t st = as_stream(stream);
-  if (dtype == CGAN3D_F32) fill_kernel<float><<<ew_blocks2(n), 256, 0, st>>>((float *)x, n, value_dev, scale);
-  else fill_kernel<__nv_bfloat16><<<ew_blocks2(n), 256, 0, st>>>((__nv_bfloat16 *)x, n, value_dev, scale);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    fill_kernel<T><<<ew_blocks(n), 256, 0, st>>>((T *)x, n, value_dev, scale);
+  });
   CG_LAUNCH_CHECK("fill");
   return 0;
 }
@@ -415,8 +417,8 @@ int cgan3d_adam_step(float *param, const float *grad, float *exp_avg, float *exp
   CG_CHECK_ARG(param && grad && exp_avg && exp_avg_sq, "adam_step: NULL pointer");
   CG_CHECK_ARG(step >= 1, "adam_step: step must be >= 1");
   if (n <= 0) return 0;
-  adam_kernel<<<ew_blocks2(n), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step,
-                                                            clip);
+  adam_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(param, grad, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step,
+                                                           clip);
   CG_LAUNCH_CHECK("adam_step");
   return 0;
 }
@@ -507,8 +509,8 @@ int cgan3d_crop_scale(const int16_t *vol, int X, int Y, int Z, int lbx, int lby,
   CG_CHECK_SHAPE(lbx >= 0 && lby >= 0 && lbz >= 0 && lbx + PX <= XP && lby + PY <= YP && lbz + PZ <= ZP,
                  "crop_scale: crop [%d,%d,%d]+patch outside the padded volume", lbx, lby, lbz);
   const int64_t total = (int64_t)PX * PY * PZ;
-  crop_scale_kernel<<<ew_blocks2(total), 256, 0, as_stream(stream)>>>(vol, X, Y, Z, lbx, lby, lbz, PX, PY, PZ, px0, py0, pz0,
-                                                                      shift, factor, data, mask);
+  crop_scale_kernel<<<ew_blocks(total), 256, 0, as_stream(stream)>>>(vol, X, Y, Z, lbx, lby, lbz, PX, PY, PZ, px0, py0, pz0,
+                                                                     shift, factor, data, mask);
   CG_LAUNCH_CHECK("crop_scale");
   return 0;
 }
@@ -519,8 +521,8 @@ int cgan3d_tile_extract(const int16_t *vol, int X, int Y, int Z, int x0, int y0,
   CG_CHECK_SHAPE(x0 >= 0 && y0 >= 0 && z0 >= 0 && x0 + PX <= X && y0 + PY <= Y && z0 + PZ <= Z && factor != 0.f,
                  "tile_extract: tile outside the volume");
   const int64_t total = (int64_t)PX * PY * PZ;
-  tile_extract_kernel<<<ew_blocks2(total), 256, 0, as_stream(stream)>>>(vol, X, Y, Z, x0, y0, z0, PX, PY, PZ, shift, factor,
-                                                                        tile);
+  tile_extract_kernel<<<ew_blocks(total), 256, 0, as_stream(stream)>>>(vol, X, Y, Z, x0, y0, z0, PX, PY, PZ, shift, factor,
+                                                                       tile);
   CG_LAUNCH_CHECK("tile_extract");
   return 0;
 }
@@ -531,7 +533,7 @@ int cgan3d_tile_accumulate(const float *tile, float *acc, float *cnt, int X, int
   CG_CHECK_SHAPE(x0 >= 0 && y0 >= 0 && z0 >= 0 && x0 + PX <= X && y0 + PY <= Y && z0 + PZ <= Z,
                  "tile_accumulate: tile outside the volume");
   const int64_t total = (int64_t)PX * PY * PZ;
-  tile_accumulate_kernel<<<ew_blocks2(total), 256, 0, as_stream(stream)>>>(tile, acc, cnt, X, Y, Z, x0, y0, z0, PX, PY, PZ);
+  tile_accumulate_kernel<<<ew_blocks(total), 256, 0, as_stream(stream)>>>(tile, acc, cnt, X, Y, Z, x0, y0, z0, PX, PY, PZ);
   CG_LAUNCH_CHECK("tile_accumulate");
   return 0;
 }
@@ -542,7 +544,7 @@ int cgan3d_sub_resized(const float *x, const float *att, float *out, int B, int 
   CG_CHECK_SHAPE(B >= 0 && X > 0 && Y > 0 && Z > 0 && Xa > 0 && Ya > 0 && Za > 0, "sub_resized: bad sizes");
   const int64_t total = (int64_t)B * X * Y * Z;
   if (total == 0) return 0;
-  sub_resized_kernel<<<ew_blocks2(total), 256, 0, as_stream(stream)>>>(x, att, out, B, X, Y, Z, Xa, Ya, Za);
+  sub_resized_kernel<<<ew_blocks(total), 256, 0, as_stream(stream)>>>(x, att, out, B, X, Y, Z, Xa, Ya, Za);
   CG_LAUNCH_CHECK("sub_resized");
   return 0;
 }
@@ -552,7 +554,7 @@ int cgan3d_scale_i16(const int16_t *hu, float *out, int64_t n, float shift, floa
   CG_CHECK_SHAPE(n >= 0 && factor != 0.f, "scale_i16: bad size / zero factor");
   CG_CHECK_ARG(!(reinterpret_cast<uintptr_t>(hu) & 15) && !(reinterpret_cast<uintptr_t>(out) & 15), "scale_i16: pointers must be 16-byte aligned");
   if (n == 0) return 0;
-  scale_i16_kernel<<<ew_blocks2(n >> 3 ? n >> 3 : 1), 256, 0, as_stream(stream)>>>(hu, out, n, shift, factor);
+  scale_i16_kernel<<<ew_blocks(n >> 3 ? n >> 3 : 1), 256, 0, as_stream(stream)>>>(hu, out, n, shift, factor);
   CG_LAUNCH_CHECK("scale_i16");
   return 0;
 }
@@ -560,7 +562,7 @@ int cgan3d_scale_i16(const int16_t *hu, float *out, int64_t n, float shift, floa
 int cgan3d_tile_finalize(const float *acc, const float *cnt, float *out, int64_t n, float shift, float factor, void *stream) {
   CG_CHECK_ARG(acc && cnt && out, "tile_finalize: NULL pointer");
   if (n <= 0) return 0;
-  tile_finalize_kernel<<<ew_blocks2(n), 256, 0, as_stream(stream)>>>(acc, cnt, out, n, shift, factor);
+  tile_finalize_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(acc, cnt, out, n, shift, factor);
   CG_LAUNCH_CHECK("tile_finalize");
   return 0;
 }

@@ -708,14 +708,9 @@ __global__ void __launch_bounds__(256) axpy_kernel(const T *__restrict__ x, T *_
     y[i] = from_f<T>(to_f(y[i]) + to_f(x[i]));
 }
 
-static inline int ew_blocks(int64_t n) { return (int)mx<int64_t>(1, mn<int64_t>((n + 255) / 256, (int64_t)num_sms() * 16)); }
-
 }  // namespace cg
 
 using namespace cg;
-
-#define CG_DTYPE_OK(d, name) \
-  if ((d) != CGAN3D_F32 && (d) != CGAN3D_BF16) return fail(CGAN3D_E_DTYPE, name ": unknown dtype %d", (d))
 
 // p -> (threshold, scale) of the keep law; false for p outside [0, 1].  scale is 0 at p = 1 (everything is dropped: the
 // outputs and gradients are 0, not 0 * inf).
@@ -726,7 +721,8 @@ static bool dropout_consts(float p, uint64_t *thresh, float *scale) {
   return true;
 }
 
-// the activation as a template argument for the vec8 kernels (-1: runtime switch), then the dropout flag
+// the activation as a template argument for the vec8 kernels (-1: runtime switch; the scalar kernels always switch at run
+// time), then the dropout flag
 template <typename F>
 static void with_act_drop(int act, bool drop, F &&go) {
   auto pick_act = [&](auto drop_tag) {
@@ -744,44 +740,29 @@ static int bn_backward_reduce_impl(const char *name, const void *dz, const void 
                                    const float *mean_invstd, const float *gamma, const float *beta, int act, float slope,
                                    double *sums, const uint8_t *keep_bits, float scale, void *stream) {
   CG_CHECK_ARG(dz && y && mean_invstd && gamma && beta && sums, "%s: NULL pointer", name);
-  CG_DTYPE_OK(dtype, "bn_backward_reduce");
+  CG_CHECK_DTYPE(dtype, name);
   CG_CHECK_SHAPE(n_rows > 0 && C > 0 && (C <= 256 || C % 256 == 0), "%s: bad sizes", name);
   cudaStream_t st = as_stream(stream);
   cudaError_t e = cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), st);
   if (e != cudaSuccess) return cuda_fail(e, "bn_backward_reduce memset");
-  if (vec8_ok(C, dz, y)) {
-    ColGrid g8 = col_grid8(n_rows, C, 2);
+  const bool v8 = vec8_ok(C, dz, y);
+  const ColGrid g = v8 ? col_grid8(n_rows, C, 2) : col_grid(n_rows, C, 2);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
     with_act_drop(act, keep_bits != nullptr, [&](auto act_tag, auto drop_tag) {
       constexpr int A = decltype(act_tag)::value;
       constexpr bool D = decltype(drop_tag)::value;
-      if (dtype == CGAN3D_F32)
-        // fp32 with the keep byte: two rows in flight per thread instead of four fit the 128 registers without spilling
-        bn_bwd_reduce8_kernel<float, A, D, D ? 2 : 4><<<g8.blocks, 256, g8.smem, st>>>((const float *)dz, (const float *)y, n_rows, C,
-                                                                            g8.rows_per_block, mean_invstd, gamma, beta, act, slope,
-                                                                            sums, keep_bits, scale);
+      // fp32 with the keep byte: two rows in flight per thread instead of four fit the 128 registers without spilling
+      constexpr int U = std::is_same<T, float>::value && D ? 2 : 4;
+      if (v8)
+        bn_bwd_reduce8_kernel<T, A, D, U><<<g.blocks, 256, g.smem, st>>>((const T *)dz, (const T *)y, n_rows, C, g.rows_per_block,
+                                                                         mean_invstd, gamma, beta, act, slope, sums, keep_bits, scale);
       else
-        bn_bwd_reduce8_kernel<__nv_bfloat16, A, D><<<g8.blocks, 256, g8.smem, st>>>(
-            (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, n_rows, C, g8.rows_per_block, mean_invstd, gamma, beta, act, slope,
-            sums, keep_bits, scale);
+        bn_bwd_reduce_kernel<T, D><<<g.blocks, 256, g.smem, st>>>((const T *)dz, (const T *)y, n_rows, C, g.rows_per_block,
+                                                                  mean_invstd, gamma, beta, act, slope, sums, keep_bits, scale);
     });
-    CG_LAUNCH_CHECK("bn_backward_reduce(vec8)");
-    return 0;
-  }
-  ColGrid g = col_grid(n_rows, C, 2);
-  auto go = [&](auto drop_tag) {
-    constexpr bool D = decltype(drop_tag)::value;
-    if (dtype == CGAN3D_F32)
-      bn_bwd_reduce_kernel<float, D><<<g.blocks, 256, g.smem, st>>>((const float *)dz, (const float *)y, n_rows, C,
-                                                                    g.rows_per_block, mean_invstd, gamma, beta, act, slope, sums,
-                                                                    keep_bits, scale);
-    else
-      bn_bwd_reduce_kernel<__nv_bfloat16, D><<<g.blocks, 256, g.smem, st>>>((const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y,
-                                                                            n_rows, C, g.rows_per_block, mean_invstd, gamma,
-                                                                            beta, act, slope, sums, keep_bits, scale);
-  };
-  if (keep_bits) go(std::true_type{});
-  else go(std::false_type{});
-  CG_LAUNCH_CHECK("bn_backward_reduce");
+  });
+  CG_LAUNCH_CHECK(v8 ? "bn_backward_reduce(vec8)" : "bn_backward_reduce");
   return 0;
 }
 
@@ -791,42 +772,28 @@ static int bn_backward_apply_impl(const char *name, const void *dz, const void *
                                   float scale, void *stream) {
   CG_CHECK_ARG(dz && y && dy && mean_invstd && gamma && beta && sums, "%s: NULL pointer", name);
   CG_CHECK_ARG(grad_beta == 0.f || grad_beta == 1.f, "%s: grad_beta must be 0 (overwrite) or 1 (accumulate)", name);
-  CG_DTYPE_OK(dtype, "bn_backward_apply");
+  CG_CHECK_DTYPE(dtype, name);
   CG_CHECK_SHAPE(n_rows > 0 && C > 0, "%s: bad sizes", name);
   cudaStream_t st = as_stream(stream);
-  const int64_t total = n_rows * C;
+  const int64_t total = n_rows * C, t8 = total / 8;
   const double inv_n = 1.0 / (double)n_rows;
-  if (vec8_ok(C, dz, y, dy)) {
-    const int64_t t8 = total / 8;
+  const bool v8 = vec8_ok(C, dz, y, dy);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
     with_act_drop(act, keep_bits != nullptr, [&](auto act_tag, auto drop_tag) {
       constexpr int A = decltype(act_tag)::value;
       constexpr bool D = decltype(drop_tag)::value;
-      if (dtype == CGAN3D_F32)
-        bn_bwd_apply8_kernel<float, A, D><<<ew_blocks(t8), 256, 0, st>>>((const float *)dz, (const float *)y, (float *)dy, t8, C,
-                                                                         inv_n, mean_invstd, gamma, beta, act, slope, sums, dgamma,
-                                                                         dbeta, grad_beta, keep_bits, scale);
+      if (v8)
+        bn_bwd_apply8_kernel<T, A, D><<<ew_blocks(t8), 256, 0, st>>>((const T *)dz, (const T *)y, (T *)dy, t8, C, inv_n, mean_invstd,
+                                                                     gamma, beta, act, slope, sums, dgamma, dbeta, grad_beta,
+                                                                     keep_bits, scale);
       else
-        bn_bwd_apply8_kernel<__nv_bfloat16, A, D><<<ew_blocks(t8), 256, 0, st>>>(
-            (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, (__nv_bfloat16 *)dy, t8, C, inv_n, mean_invstd, gamma, beta, act,
-            slope, sums, dgamma, dbeta, grad_beta, keep_bits, scale);
+        bn_bwd_apply_kernel<T, D><<<ew_blocks(total), 256, 0, st>>>((const T *)dz, (const T *)y, (T *)dy, total, C, inv_n,
+                                                                    mean_invstd, gamma, beta, act, slope, sums, dgamma, dbeta,
+                                                                    grad_beta, keep_bits, scale);
     });
-    CG_LAUNCH_CHECK("bn_backward_apply(vec8)");
-    return 0;
-  }
-  auto go = [&](auto drop_tag) {
-    constexpr bool D = decltype(drop_tag)::value;
-    if (dtype == CGAN3D_F32)
-      bn_bwd_apply_kernel<float, D><<<ew_blocks(total), 256, 0, st>>>((const float *)dz, (const float *)y, (float *)dy, total, C,
-                                                                      inv_n, mean_invstd, gamma, beta, act, slope, sums, dgamma,
-                                                                      dbeta, grad_beta, keep_bits, scale);
-    else
-      bn_bwd_apply_kernel<__nv_bfloat16, D><<<ew_blocks(total), 256, 0, st>>>(
-          (const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y, (__nv_bfloat16 *)dy, total, C, inv_n, mean_invstd, gamma, beta,
-          act, slope, sums, dgamma, dbeta, grad_beta, keep_bits, scale);
-  };
-  if (keep_bits) go(std::true_type{});
-  else go(std::false_type{});
-  CG_LAUNCH_CHECK("bn_backward_apply");
+  });
+  CG_LAUNCH_CHECK(v8 ? "bn_backward_apply(vec8)" : "bn_backward_apply");
   return 0;
 }
 
@@ -834,43 +801,36 @@ extern "C" {
 
 int cgan3d_bn_stats(const void *y, int dtype, int64_t n_rows, int C, double *sums, void *stream) {
   CG_CHECK_ARG(y && sums, "bn_stats: NULL pointer");
-  CG_DTYPE_OK(dtype, "bn_stats");
+  CG_CHECK_DTYPE(dtype, "bn_stats");
   CG_CHECK_SHAPE(n_rows >= 0 && C > 0 && (C <= 256 || C % 256 == 0), "bn_stats: bad sizes");
   cudaStream_t st = as_stream(stream);
   cudaError_t e = cudaMemsetAsync(sums, 0, 2 * (size_t)C * sizeof(double), st);
   if (e != cudaSuccess) return cuda_fail(e, "bn_stats memset");
   if (n_rows == 0) return 0;
-  if (vec8_ok(C, y)) {
-    ColGrid g8 = col_grid8(n_rows, C, 2);
-    if (dtype == CGAN3D_F32)
-      bn_stats8_kernel<float><<<g8.blocks, 256, g8.smem, st>>>((const float *)y, n_rows, C, g8.rows_per_block, sums);
-    else
-      bn_stats8_kernel<__nv_bfloat16><<<g8.blocks, 256, g8.smem, st>>>((const __nv_bfloat16 *)y, n_rows, C, g8.rows_per_block, sums);
-    CG_LAUNCH_CHECK("bn_stats(vec8)");
-    return 0;
-  }
-  ColGrid g = col_grid(n_rows, C, 2);
-  if (dtype == CGAN3D_F32)
-    bn_stats_kernel<float><<<g.blocks, 256, g.smem, st>>>((const float *)y, n_rows, C, g.rows_per_block, sums);
-  else
-    bn_stats_kernel<__nv_bfloat16><<<g.blocks, 256, g.smem, st>>>((const __nv_bfloat16 *)y, n_rows, C, g.rows_per_block, sums);
-  CG_LAUNCH_CHECK("bn_stats");
+  const bool v8 = vec8_ok(C, y);
+  const ColGrid g = v8 ? col_grid8(n_rows, C, 2) : col_grid(n_rows, C, 2);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (v8) bn_stats8_kernel<T><<<g.blocks, 256, g.smem, st>>>((const T *)y, n_rows, C, g.rows_per_block, sums);
+    else bn_stats_kernel<T><<<g.blocks, 256, g.smem, st>>>((const T *)y, n_rows, C, g.rows_per_block, sums);
+  });
+  CG_LAUNCH_CHECK(v8 ? "bn_stats(vec8)" : "bn_stats");
   return 0;
 }
 
 int cgan3d_col_sums(const void *x, int dtype, int64_t n_rows, int C, double *sums, void *stream) {
   CG_CHECK_ARG(x && sums, "col_sums: NULL pointer");
-  CG_DTYPE_OK(dtype, "col_sums");
+  CG_CHECK_DTYPE(dtype, "col_sums");
   CG_CHECK_SHAPE(n_rows >= 0 && C > 0 && (C <= 256 || C % 256 == 0), "col_sums: bad sizes");
   cudaStream_t st = as_stream(stream);
   cudaError_t e = cudaMemsetAsync(sums, 0, (size_t)C * sizeof(double), st);
   if (e != cudaSuccess) return cuda_fail(e, "col_sums memset");
   if (n_rows == 0) return 0;
-  ColGrid g = col_grid(n_rows, C, 1);
-  if (dtype == CGAN3D_F32)
-    col_sums_kernel<float><<<g.blocks, 256, g.smem, st>>>((const float *)x, n_rows, C, g.rows_per_block, sums);
-  else
-    col_sums_kernel<__nv_bfloat16><<<g.blocks, 256, g.smem, st>>>((const __nv_bfloat16 *)x, n_rows, C, g.rows_per_block, sums);
+  const ColGrid g = col_grid(n_rows, C, 1);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    col_sums_kernel<T><<<g.blocks, 256, g.smem, st>>>((const T *)x, n_rows, C, g.rows_per_block, sums);
+  });
   CG_LAUNCH_CHECK("col_sums");
   return 0;
 }
@@ -905,48 +865,40 @@ int cgan3d_sums_to_f32(const double *sums, float *out, int n, float scale, float
 int cgan3d_bn_apply(const void *y, void *z, int dtype, int64_t n_rows, int C, const float *mean_invstd,
                     const float *gamma, const float *beta, int act, float slope, const void *residual, void *stream) {
   CG_CHECK_ARG(y && z && mean_invstd && gamma && beta, "bn_apply: NULL pointer");
-  CG_DTYPE_OK(dtype, "bn_apply");
+  CG_CHECK_DTYPE(dtype, "bn_apply");
   CG_CHECK_SHAPE(n_rows >= 0 && C > 0, "bn_apply: bad sizes");
-  const int64_t total = n_rows * C;
+  const int64_t total = n_rows * C, t8 = total / 8;
   if (total == 0) return 0;
   cudaStream_t st = as_stream(stream);
-  if (vec8_ok(C, y, z, residual)) {
-    const int64_t t8 = total / 8;
-    if (dtype == CGAN3D_F32)
-      bn_apply8_kernel<float><<<ew_blocks(t8), 256, 0, st>>>((const float *)y, (float *)z, t8, C, mean_invstd, gamma, beta, act,
-                                                             slope, (const float *)residual);
+  const bool v8 = vec8_ok(C, y, z, residual);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (v8)
+      bn_apply8_kernel<T><<<ew_blocks(t8), 256, 0, st>>>((const T *)y, (T *)z, t8, C, mean_invstd, gamma, beta, act, slope,
+                                                         (const T *)residual);
     else
-      bn_apply8_kernel<__nv_bfloat16><<<ew_blocks(t8), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, t8, C, mean_invstd,
-                                                                     gamma, beta, act, slope, (const __nv_bfloat16 *)residual);
-    CG_LAUNCH_CHECK("bn_apply(vec8)");
-    return 0;
-  }
-  if (dtype == CGAN3D_F32)
-    bn_apply_kernel<float><<<ew_blocks(total), 256, 0, st>>>((const float *)y, (float *)z, total, C, mean_invstd, gamma,
-                                                             beta, act, slope, (const float *)residual);
-  else
-    bn_apply_kernel<__nv_bfloat16><<<ew_blocks(total), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, total,
-                                                                     C, mean_invstd, gamma, beta, act, slope,
-                                                                     (const __nv_bfloat16 *)residual);
-  CG_LAUNCH_CHECK("bn_apply");
+      bn_apply_kernel<T><<<ew_blocks(total), 256, 0, st>>>((const T *)y, (T *)z, total, C, mean_invstd, gamma, beta, act, slope,
+                                                           (const T *)residual);
+  });
+  CG_LAUNCH_CHECK(v8 ? "bn_apply(vec8)" : "bn_apply");
   return 0;
 }
 
 int cgan3d_bn_apply_pad(const void *y, void *z_padded, int dtype, int B, int X, int Y, int Z, int C, const float *mean_invstd,
                         const float *gamma, const float *beta, int act, float slope, int pad, void *stream) {
   CG_CHECK_ARG(y && z_padded && mean_invstd && gamma && beta, "bn_apply_pad: NULL pointer");
-  CG_DTYPE_OK(dtype, "bn_apply_pad");
+  CG_CHECK_DTYPE(dtype, "bn_apply_pad");
   CG_CHECK_SHAPE(B > 0 && X > 0 && Y > 0 && Z > 0 && C > 0 && pad > 0 && pad < X && pad < Y && pad < Z, "bn_apply_pad: bad sizes");
   if (C % 8 || !vec8_ok(C, y, z_padded) || X + 2 * pad > 65535 || B > 65535)
     return fail(CGAN3D_E_UNSUPPORTED, "bn_apply_pad: needs C %% 8 == 0 and 16-byte aligned tensors");
   cudaStream_t st = as_stream(stream);
   const dim3 grid((unsigned)(Y + 2 * pad), (unsigned)(X + 2 * pad), (unsigned)B);
   const size_t smem = 2 * (size_t)C * sizeof(float);
-  if (dtype == CGAN3D_F32)
-    bn_apply_pad8_kernel<float><<<grid, 256, smem, st>>>((const float *)y, (float *)z_padded, X, Y, Z, C, pad, mean_invstd, gamma, beta, act, slope);
-  else
-    bn_apply_pad8_kernel<__nv_bfloat16><<<grid, 256, smem, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z_padded, X, Y, Z, C, pad,
-                                                                 mean_invstd, gamma, beta, act, slope);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    bn_apply_pad8_kernel<T><<<grid, 256, smem, st>>>((const T *)y, (T *)z_padded, X, Y, Z, C, pad, mean_invstd, gamma, beta, act,
+                                                     slope);
+  });
   CG_LAUNCH_CHECK("bn_apply_pad");
   return 0;
 }
@@ -955,35 +907,25 @@ int cgan3d_bn_apply_dropout(const void *y, void *z, uint8_t *keep_bits, int dtyp
                             const float *mean_invstd, const float *gamma, const float *beta, int act, float slope, float p,
                             const int64_t *seed_dev, void *stream) {
   CG_CHECK_ARG(y && z && keep_bits && mean_invstd && gamma && beta && seed_dev, "bn_apply_dropout: NULL pointer");
-  CG_DTYPE_OK(dtype, "bn_apply_dropout");
+  CG_CHECK_DTYPE(dtype, "bn_apply_dropout");
   CG_CHECK_SHAPE(n_rows >= 0 && C > 0, "bn_apply_dropout: bad sizes");
   uint64_t thresh;
   float scale;
   if (!dropout_consts(p, &thresh, &scale)) return fail(CGAN3D_E_ARG, "bn_apply_dropout: p = %g is outside [0, 1]", (double)p);
-  const int64_t total = n_rows * C;
+  const int64_t total = n_rows * C, t8 = total / 8, nbytes = (total + 7) / 8;
   if (total == 0) return 0;
   cudaStream_t st = as_stream(stream);
-  if (vec8_ok(C, y, z)) {
-    const int64_t t8 = total / 8;
-    if (dtype == CGAN3D_F32)
-      bn_apply8_kernel<float, true><<<ew_blocks(t8), 256, 0, st>>>((const float *)y, (float *)z, t8, C, mean_invstd, gamma, beta, act,
-                                                                   slope, nullptr, keep_bits, seed_dev, thresh, scale);
+  const bool v8 = vec8_ok(C, y, z);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (v8)
+      bn_apply8_kernel<T, true><<<ew_blocks(t8), 256, 0, st>>>((const T *)y, (T *)z, t8, C, mean_invstd, gamma, beta, act, slope,
+                                                               nullptr, keep_bits, seed_dev, thresh, scale);
     else
-      bn_apply8_kernel<__nv_bfloat16, true><<<ew_blocks(t8), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, t8, C,
-                                                                           mean_invstd, gamma, beta, act, slope, nullptr, keep_bits,
-                                                                           seed_dev, thresh, scale);
-    CG_LAUNCH_CHECK("bn_apply_dropout(vec8)");
-    return 0;
-  }
-  const int64_t nbytes = (total + 7) / 8;
-  if (dtype == CGAN3D_F32)
-    bn_apply_dropout_kernel<float><<<ew_blocks(nbytes), 256, 0, st>>>((const float *)y, (float *)z, keep_bits, total, C, mean_invstd,
-                                                                      gamma, beta, act, slope, seed_dev, thresh, scale);
-  else
-    bn_apply_dropout_kernel<__nv_bfloat16><<<ew_blocks(nbytes), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, keep_bits,
-                                                                              total, C, mean_invstd, gamma, beta, act, slope,
-                                                                              seed_dev, thresh, scale);
-  CG_LAUNCH_CHECK("bn_apply_dropout");
+      bn_apply_dropout_kernel<T><<<ew_blocks(nbytes), 256, 0, st>>>((const T *)y, (T *)z, keep_bits, total, C, mean_invstd, gamma,
+                                                                    beta, act, slope, seed_dev, thresh, scale);
+  });
+  CG_LAUNCH_CHECK(v8 ? "bn_apply_dropout(vec8)" : "bn_apply_dropout");
   return 0;
 }
 
@@ -1022,61 +964,45 @@ int cgan3d_bn_backward_apply_dropout(const void *dz, const void *y, const uint8_
                                 sums, dgamma, dbeta, grad_beta, keep_bits, scale, stream);
 }
 
+
 int cgan3d_bias_act(const void *y, void *z, int dtype, int64_t n_rows, int C, const float *bias, int act, float slope,
                     void *stream) {
   CG_CHECK_ARG(y && z, "bias_act: NULL pointer");
-  CG_DTYPE_OK(dtype, "bias_act");
+  CG_CHECK_DTYPE(dtype, "bias_act");
   CG_CHECK_SHAPE(n_rows >= 0 && C > 0, "bias_act: bad sizes");
-  const int64_t total = n_rows * C;
+  const int64_t total = n_rows * C, t8 = total / 8;
   if (total == 0) return 0;
   cudaStream_t st = as_stream(stream);
-  if (vec8_ok(C, y, z)) {
-    const int64_t t8 = total / 8;
-    if (dtype == CGAN3D_F32)
-      bias_act8_kernel<float><<<ew_blocks(t8), 256, 0, st>>>((const float *)y, (float *)z, t8, C, bias, act, slope);
-    else
-      bias_act8_kernel<__nv_bfloat16><<<ew_blocks(t8), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, t8, C, bias, act,
-                                                                     slope);
-    CG_LAUNCH_CHECK("bias_act(vec8)");
-    return 0;
-  }
-  if (dtype == CGAN3D_F32)
-    bias_act_kernel<float><<<ew_blocks(total), 256, 0, st>>>((const float *)y, (float *)z, total, C, bias, act, slope);
-  else
-    bias_act_kernel<__nv_bfloat16><<<ew_blocks(total), 256, 0, st>>>((const __nv_bfloat16 *)y, (__nv_bfloat16 *)z, total, C,
-                                                                     bias, act, slope);
-  CG_LAUNCH_CHECK("bias_act");
+  const bool v8 = vec8_ok(C, y, z);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (v8) bias_act8_kernel<T><<<ew_blocks(t8), 256, 0, st>>>((const T *)y, (T *)z, t8, C, bias, act, slope);
+    else bias_act_kernel<T><<<ew_blocks(total), 256, 0, st>>>((const T *)y, (T *)z, total, C, bias, act, slope);
+  });
+  CG_LAUNCH_CHECK(v8 ? "bias_act(vec8)" : "bias_act");
   return 0;
 }
 
 int cgan3d_bias_act_backward(const void *dz, const void *y, void *dy, int dtype, int64_t n_rows, int C, const float *bias,
                              int act, float slope, double *dbias_sums, void *stream) {
   CG_CHECK_ARG(dz && y && dy && dbias_sums, "bias_act_backward: NULL pointer");
-  CG_DTYPE_OK(dtype, "bias_act_backward");
+  CG_CHECK_DTYPE(dtype, "bias_act_backward");
   CG_CHECK_SHAPE(n_rows > 0 && C > 0 && (C <= 256 || C % 256 == 0), "bias_act_backward: bad sizes");
   cudaStream_t st = as_stream(stream);
   cudaError_t e = cudaMemsetAsync(dbias_sums, 0, (size_t)C * sizeof(double), st);
   if (e != cudaSuccess) return cuda_fail(e, "bias_act_backward memset");
-  if (vec8_ok(C, dz, y, dy)) {
-    ColGrid g8 = col_grid8(n_rows, C, 1);
-    if (dtype == CGAN3D_F32)
-      bias_act_bwd8_kernel<float><<<g8.blocks, 256, g8.smem, st>>>((const float *)dz, (const float *)y, (float *)dy, n_rows, C, bias,
-                                                                   act, slope, dbias_sums);
+  const bool v8 = vec8_ok(C, dz, y, dy);
+  const ColGrid g = v8 ? col_grid8(n_rows, C, 1) : col_grid(n_rows, C, 1);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    if (v8)
+      bias_act_bwd8_kernel<T><<<g.blocks, 256, g.smem, st>>>((const T *)dz, (const T *)y, (T *)dy, n_rows, C, bias, act, slope,
+                                                             dbias_sums);
     else
-      bias_act_bwd8_kernel<__nv_bfloat16><<<g8.blocks, 256, g8.smem, st>>>((const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y,
-                                                                           (__nv_bfloat16 *)dy, n_rows, C, bias, act, slope, dbias_sums);
-    CG_LAUNCH_CHECK("bias_act_backward(vec8)");
-    return 0;
-  }
-  ColGrid g = col_grid(n_rows, C, 1);
-  if (dtype == CGAN3D_F32)
-    bias_act_bwd_kernel<float><<<g.blocks, 256, g.smem, st>>>((const float *)dz, (const float *)y, (float *)dy, n_rows, C,
-                                                              g.rows_per_block, bias, act, slope, dbias_sums);
-  else
-    bias_act_bwd_kernel<__nv_bfloat16><<<g.blocks, 256, g.smem, st>>>((const __nv_bfloat16 *)dz, (const __nv_bfloat16 *)y,
-                                                                      (__nv_bfloat16 *)dy, n_rows, C, g.rows_per_block,
-                                                                      bias, act, slope, dbias_sums);
-  CG_LAUNCH_CHECK("bias_act_backward");
+      bias_act_bwd_kernel<T><<<g.blocks, 256, g.smem, st>>>((const T *)dz, (const T *)y, (T *)dy, n_rows, C, g.rows_per_block, bias,
+                                                            act, slope, dbias_sums);
+  });
+  CG_LAUNCH_CHECK(v8 ? "bias_act_backward(vec8)" : "bias_act_backward");
   return 0;
 }
 
@@ -1084,14 +1010,13 @@ int cgan3d_tanh_residual(const void *y, const float *bias, const float *x, float
                          int64_t n, void *stream) {
   CG_CHECK_ARG(y && attenuation, "tanh_residual: NULL pointer");
   CG_CHECK_ARG(opt_hat == nullptr || x != nullptr, "tanh_residual: opt_hat requires x");
-  CG_DTYPE_OK(dtype, "tanh_residual");
+  CG_CHECK_DTYPE(dtype, "tanh_residual");
   if (n <= 0) return 0;
   cudaStream_t st = as_stream(stream);
-  if (dtype == CGAN3D_F32)
-    tanh_residual_kernel<float><<<ew_blocks(n), 256, 0, st>>>((const float *)y, bias, x, attenuation, opt_hat, n);
-  else
-    tanh_residual_kernel<__nv_bfloat16><<<ew_blocks(n), 256, 0, st>>>((const __nv_bfloat16 *)y, bias, x, attenuation,
-                                                                      opt_hat, n);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    tanh_residual_kernel<T><<<ew_blocks(n), 256, 0, st>>>((const T *)y, bias, x, attenuation, opt_hat, n);
+  });
   CG_LAUNCH_CHECK("tanh_residual");
   return 0;
 }
@@ -1099,48 +1024,47 @@ int cgan3d_tanh_residual(const void *y, const float *bias, const float *x, float
 int cgan3d_tanh_residual_backward(const float *d_opt_hat, const float *d_att, const float *attenuation, void *dy,
                                   int dtype, int64_t n, double *dbias_sum, void *stream) {
   CG_CHECK_ARG(attenuation && dy && (d_opt_hat || d_att), "tanh_residual_backward: NULL pointer");
-  CG_DTYPE_OK(dtype, "tanh_residual_backward");
+  CG_CHECK_DTYPE(dtype, "tanh_residual_backward");
   if (n <= 0) return 0;
   cudaStream_t st = as_stream(stream);
   if (dbias_sum) {
     cudaError_t e = cudaMemsetAsync(dbias_sum, 0, sizeof(double), st);
     if (e != cudaSuccess) return cuda_fail(e, "tanh_residual_backward memset");
   }
-  if (dtype == CGAN3D_F32)
-    tanh_residual_bwd_kernel<float><<<ew_blocks(n), 256, 0, st>>>(d_opt_hat, d_att, attenuation, (float *)dy, n, dbias_sum);
-  else
-    tanh_residual_bwd_kernel<__nv_bfloat16><<<ew_blocks(n), 256, 0, st>>>(d_opt_hat, d_att, attenuation,
-                                                                          (__nv_bfloat16 *)dy, n, dbias_sum);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    tanh_residual_bwd_kernel<T><<<ew_blocks(n), 256, 0, st>>>(d_opt_hat, d_att, attenuation, (T *)dy, n, dbias_sum);
+  });
   CG_LAUNCH_CHECK("tanh_residual_backward");
   return 0;
 }
 
 int cgan3d_cast(const void *in, int in_dtype, void *out, int out_dtype, int64_t n, void *stream) {
   CG_CHECK_ARG(in && out, "cast: NULL pointer");
-  CG_DTYPE_OK(in_dtype, "cast");
-  CG_DTYPE_OK(out_dtype, "cast");
+  CG_CHECK_DTYPE(in_dtype, "cast");
+  CG_CHECK_DTYPE(out_dtype, "cast");
   if (n <= 0) return 0;
   cudaStream_t st = as_stream(stream);
-  const int nb = ew_blocks(n);
-  if (in_dtype == CGAN3D_F32 && out_dtype == CGAN3D_BF16)
-    cast_kernel<float, __nv_bfloat16><<<nb, 256, 0, st>>>((const float *)in, (__nv_bfloat16 *)out, n);
-  else if (in_dtype == CGAN3D_BF16 && out_dtype == CGAN3D_F32)
-    cast_kernel<__nv_bfloat16, float><<<nb, 256, 0, st>>>((const __nv_bfloat16 *)in, (float *)out, n);
-  else if (in_dtype == CGAN3D_F32)
-    cast_kernel<float, float><<<nb, 256, 0, st>>>((const float *)in, (float *)out, n);
-  else
-    cast_kernel<__nv_bfloat16, __nv_bfloat16><<<nb, 256, 0, st>>>((const __nv_bfloat16 *)in, (__nv_bfloat16 *)out, n);
+  with_dtype(in_dtype, [&](auto ti) {
+    with_dtype(out_dtype, [&](auto to) {
+      using TI = typename decltype(ti)::type;
+      using TO = typename decltype(to)::type;
+      cast_kernel<TI, TO><<<ew_blocks(n), 256, 0, st>>>((const TI *)in, (TO *)out, n);
+    });
+  });
   CG_LAUNCH_CHECK("cast");
   return 0;
 }
 
 int cgan3d_axpy(const void *x, void *y, int dtype, int64_t n, void *stream) {
   CG_CHECK_ARG(x && y, "axpy: NULL pointer");
-  CG_DTYPE_OK(dtype, "axpy");
+  CG_CHECK_DTYPE(dtype, "axpy");
   if (n <= 0) return 0;
   cudaStream_t st = as_stream(stream);
-  if (dtype == CGAN3D_F32) axpy_kernel<float><<<ew_blocks(n), 256, 0, st>>>((const float *)x, (float *)y, n);
-  else axpy_kernel<__nv_bfloat16><<<ew_blocks(n), 256, 0, st>>>((const __nv_bfloat16 *)x, (__nv_bfloat16 *)y, n);
+  with_dtype(dtype, [&](auto t) {
+    using T = typename decltype(t)::type;
+    axpy_kernel<T><<<ew_blocks(n), 256, 0, st>>>((const T *)x, (T *)y, n);
+  });
   CG_LAUNCH_CHECK("axpy");
   return 0;
 }
