@@ -25,6 +25,7 @@ class ConvGeom(C.Structure):
         return tuple(getattr(self, n) for n, _ in self._fields_)
 
 
+BLEND_AVG, BLEND_GAUSSIAN = 0, 1
 BORDER_CONSTANT, BORDER_NEAREST = 0, 1
 SPATIAL_TRANSFORM, SPATIAL_ELASTIC = 1, 2
 
@@ -93,6 +94,8 @@ SIGNATURES = {
     "cgan3d_tile_extract": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp, _vp]),
     "cgan3d_tile_accumulate": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "cgan3d_tile_finalize": (_i, [_vp, _vp, _vp, _i64, _f, _f, _vp]),
+    "cgan3d_tile_extract_grid": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp, _vp]),
+    "cgan3d_tile_stitch": (_i, [_vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp, _vp]),
     "cgan3d_sub_resized": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "cgan3d_elastic_noise": (_i, [_i, _i, _i, _i, _vp, _vp, _vp]),
     "cgan3d_elastic_workspace_bytes": (_sz, [_i, _i, _i, _i]),

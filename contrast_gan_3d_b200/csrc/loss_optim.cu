@@ -303,6 +303,101 @@ tile_finalize_kernel(const float *__restrict__ acc, const float *__restrict__ cn
     out[i] = (acc[i] / cnt[i]) * factor + shift;
 }
 
+// One axis of the corrector's tile grid (CCTAContrastCorrector.grid_tiles): `reg` regular starts 0, s, 2s, ... <= S - P,
+// then the squeezed start S - P when the last regular tile stops short of the end.  Tile t of the grid is
+// (ix, iy, iz) with t = (ix * ny + iy) * nz + iz.
+struct GridAxis {
+  int S, P, s, reg, n;
+};
+static inline GridAxis grid_axis(int S, int P, int s) {
+  const int reg = (S - P) / s + 1;
+  return GridAxis{S, P, s, reg, reg + ((reg - 1) * s + P < S ? 1 : 0)};
+}
+__device__ __forceinline__ int grid_start(const GridAxis &a, int k) { return k < a.reg ? k * a.s : a.S - a.P; }
+
+// The tiles of one axis that cover coordinate v, in ascending order: regular tiles k0 .. k0 + nreg - 1, then the
+// squeezed tile (index reg) when it exists and covers v.  n <= ceil(P / s) + 1.
+struct Cover {
+  int k0, nreg, n;
+};
+__device__ __forceinline__ Cover grid_cover(const GridAxis &a, int v) {
+  const int k0 = v >= a.P ? (v - a.P) / a.s + 1 : 0;
+  const int k1 = mn(v / a.s, a.reg - 1);
+  const int nreg = mx(0, k1 - k0 + 1);
+  return Cover{k0, nreg, nreg + (a.n > a.reg && v >= a.S - a.P ? 1 : 0)};
+}
+__device__ __forceinline__ int cover_tile(const Cover &c, const GridAxis &a, int j) { return j < c.nreg ? c.k0 + j : a.reg; }
+
+// tiles [n][PX][PY][PZ] of grid tiles t0 .. t0 + n - 1; blockIdx.y = tile, the same expression as tile_extract_kernel
+__global__ void __launch_bounds__(256)
+tile_extract_grid_kernel(const int16_t *__restrict__ vol, int Y, int Z, GridAxis gx, GridAxis gy, GridAxis gz, int t0,
+                         float shift, float factor, float *__restrict__ tiles) {
+  const int PX = gx.P, PY = gy.P, PZ = gz.P, total = PX * PY * PZ;
+  const int t = t0 + (int)blockIdx.y;
+  const int x0 = grid_start(gx, t / (gz.n * gy.n)), y0 = grid_start(gy, (t / gz.n) % gy.n), z0 = grid_start(gz, t % gz.n);
+  float *tile = tiles + (int64_t)blockIdx.y * total;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
+    const int z = i % PZ, y = (i / PZ) % PY, x = i / (PZ * PY);
+    const float hu = (float)vol[((int64_t)(x0 + x) * Y + (y0 + y)) * Z + (z0 + z)];
+    tile[i] = (hu - shift) / factor;
+  }
+}
+
+// out(v) = sum_t w(v - o_t) c_t(v) / sum_t w(v - o_t) over the grid tiles covering v, in ascending tile index; with
+// to_hu the result is unscaled as in tile_finalize_kernel.  One warp per (x, y) row, lanes along z.  For GAUSS = false
+// (w = 1) the operations are exactly those of tile_accumulate_kernel (tile by tile) followed by acc / cnt.
+// GAUSS: w = (wx * wy) * wz, w_a(i) = expf(-(i - (P_a - 1) / 2)^2 / (2 sigma_a^2)), sigma_a = P_a / 8, tabulated per
+// block in shared memory; the weighted mean is kept as a running mean, s += (w / wsum) (c - s), which gives a constant
+// input back exactly (a plain sum / wsum is off by several ulp where many tiles of small weight overlap).
+template <bool GAUSS>
+__global__ void __launch_bounds__(256)
+tile_stitch_kernel(const float *const *__restrict__ tiles, int X, int Y, int Z, GridAxis gx, GridAxis gy, GridAxis gz,
+                   int to_hu, float shift, float factor, float *__restrict__ out) {
+  extern __shared__ float wtab[];  // GAUSS: [PX] x weights, [PY] y weights, [PZ] z weights
+  const int PY = gy.P, PZ = gz.P;
+  if (GAUSS) {
+    const int nw = gx.P + PY + PZ;
+    for (int i = threadIdx.y * blockDim.x + threadIdx.x; i < nw; i += blockDim.x * blockDim.y) {
+      const int P = i < gx.P ? gx.P : i < gx.P + PY ? PY : PZ;
+      const int l = i < gx.P ? i : i < gx.P + PY ? i - gx.P : i - gx.P - PY;
+      const float sig = (float)P * 0.125f, d = (float)l - 0.5f * (float)(P - 1);
+      wtab[i] = expf(-(d * d) / (2.f * sig * sig));
+    }
+    __syncthreads();
+  }
+  const float *wx_t = wtab, *wy_t = wtab + gx.P, *wz_t = wtab + gx.P + PY;
+  for (int row = blockIdx.x * blockDim.y + threadIdx.y; row < X * Y; row += gridDim.x * blockDim.y) {
+    const int x = row / Y, y = row % Y;
+    const Cover cx = grid_cover(gx, x), cy = grid_cover(gy, y);
+    for (int z = threadIdx.x; z < Z; z += blockDim.x) {
+      const Cover cz = grid_cover(gz, z);
+      float s = 0.f, wsum = 0.f;
+      for (int jx = 0; jx < cx.n; ++jx) {
+        const int ix = cover_tile(cx, gx, jx), lx = x - grid_start(gx, ix);
+        for (int jy = 0; jy < cy.n; ++jy) {
+          const int iy = cover_tile(cy, gy, jy), ly = y - grid_start(gy, iy);
+          const int tbase = (ix * gy.n + iy) * gz.n, ebase = (lx * PY + ly) * PZ;
+          const float wxy = GAUSS ? wx_t[lx] * wy_t[ly] : 1.f;
+          for (int jz = 0; jz < cz.n; ++jz) {
+            const int iz = cover_tile(cz, gz, jz), lz = z - grid_start(gz, iz);
+            const float c = tiles[tbase + iz][ebase + lz];
+            if (GAUSS) {
+              const float w = wxy * wz_t[lz];
+              wsum += w;
+              s = fmaf(w / wsum, c - s, s);
+            } else {
+              s += c;
+              wsum += 1.f;
+            }
+          }
+        }
+      }
+      const float q = GAUSS ? s : s / wsum;
+      out[(int64_t)row * Z + z] = to_hu ? q * factor + shift : q;
+    }
+  }
+}
+
 // out = x - nearest_resize(att): the corrector's `patch - nn.Upsample(size=patch)(G(patch))` branch
 // (reference eval/CCTAContrastCorrector.py:42-52,79); index law of aten::upsample_nearest3d (legacy "nearest").
 __device__ __forceinline__ int nearest_src(int dst, int in_size, int out_size) {
@@ -342,6 +437,20 @@ scale_i16_kernel(const int16_t *__restrict__ hu, float *__restrict__ out, int64_
   }
   if (blockIdx.x == 0)
     for (int64_t i = (n8 << 3) + threadIdx.x; i < n; i += blockDim.x) out[i] = ((float)hu[i] - shift) / factor;
+}
+
+// the three axes of the tile grid for a volume, patch and step, checked: 1 <= P <= S and 1 <= s <= P per axis
+static int tile_grid(const char *who, int X, int Y, int Z, int PX, int PY, int PZ, int SX, int SY, int SZ, GridAxis *g) {
+  CG_CHECK_SHAPE(X > 0 && Y > 0 && Z > 0 && PX > 0 && PY > 0 && PZ > 0 && PX <= X && PY <= Y && PZ <= Z,
+                 "%s: patch %dx%dx%d does not fit the volume %dx%dx%d", who, PX, PY, PZ, X, Y, Z);
+  CG_CHECK_SHAPE(SX >= 1 && SY >= 1 && SZ >= 1 && SX <= PX && SY <= PY && SZ <= PZ,
+                 "%s: step %dx%dx%d outside 1..patch (%dx%dx%d)", who, SX, SY, SZ, PX, PY, PZ);
+  CG_CHECK_SHAPE((int64_t)PX * PY * PZ <= INT32_MAX && (int64_t)X * Y <= INT32_MAX, "%s: volume or patch too large", who);
+  g[0] = grid_axis(X, PX, SX);
+  g[1] = grid_axis(Y, PY, SY);
+  g[2] = grid_axis(Z, PZ, SZ);
+  CG_CHECK_SHAPE((int64_t)g[0].n * g[1].n * g[2].n <= INT32_MAX, "%s: too many tiles", who);
+  return 0;
 }
 
 }  // namespace cg
@@ -564,6 +673,41 @@ int cgan3d_tile_finalize(const float *acc, const float *cnt, float *out, int64_t
   if (n <= 0) return 0;
   tile_finalize_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(acc, cnt, out, n, shift, factor);
   CG_LAUNCH_CHECK("tile_finalize");
+  return 0;
+}
+
+int cgan3d_tile_extract_grid(const int16_t *vol, int X, int Y, int Z, int PX, int PY, int PZ, int SX, int SY, int SZ, int t0,
+                             int n, float shift, float factor, float *tiles, void *stream) {
+  CG_CHECK_ARG(vol && tiles, "tile_extract_grid: NULL pointer");
+  GridAxis g[3];
+  if (int rc = tile_grid("tile_extract_grid", X, Y, Z, PX, PY, PZ, SX, SY, SZ, g)) return rc;
+  const int ntiles = g[0].n * g[1].n * g[2].n;
+  CG_CHECK_SHAPE(t0 >= 0 && n >= 0 && n <= ntiles - t0 && n <= 65535, "tile_extract_grid: tiles %d..%d outside the grid of %d (at most 65535 per call)", t0, t0 + n - 1, ntiles);
+  CG_CHECK_ARG(factor != 0.f, "tile_extract_grid: zero factor");
+  if (n == 0) return 0;
+  const int per_tile = (int)mx<int64_t>(1, ew_blocks((int64_t)n * PX * PY * PZ) / n);
+  tile_extract_grid_kernel<<<dim3(per_tile, n), 256, 0, as_stream(stream)>>>(vol, Y, Z, g[0], g[1], g[2], t0, shift, factor,
+                                                                            tiles);
+  CG_LAUNCH_CHECK("tile_extract_grid");
+  return 0;
+}
+
+int cgan3d_tile_stitch(const float *const *tiles, int n, int X, int Y, int Z, int PX, int PY, int PZ, int SX, int SY, int SZ,
+                       int blend, int to_hu, float shift, float factor, float *out, void *stream) {
+  CG_CHECK_ARG(tiles && out, "tile_stitch: NULL pointer");
+  GridAxis g[3];
+  if (int rc = tile_grid("tile_stitch", X, Y, Z, PX, PY, PZ, SX, SY, SZ, g)) return rc;
+  CG_CHECK_SHAPE(n == g[0].n * g[1].n * g[2].n, "tile_stitch: %d tiles given, the grid has %d", n, g[0].n * g[1].n * g[2].n);
+  CG_CHECK_ARG(blend == CGAN3D_BLEND_AVG || blend == CGAN3D_BLEND_GAUSSIAN, "tile_stitch: unknown blend %d", blend);
+  const size_t smem = blend == CGAN3D_BLEND_GAUSSIAN ? (size_t)(PX + PY + PZ) * sizeof(float) : 0;
+  CG_CHECK_SHAPE(smem <= 48 * 1024, "tile_stitch: patch %dx%dx%d too large for the weight table", PX, PY, PZ);
+  const dim3 block(32, 8);
+  const int grid = (int)mn<int64_t>(((int64_t)X * Y + 7) / 8, (int64_t)num_sms() * 8);
+  if (blend == CGAN3D_BLEND_GAUSSIAN)
+    tile_stitch_kernel<true><<<grid, block, smem, as_stream(stream)>>>(tiles, X, Y, Z, g[0], g[1], g[2], to_hu, shift, factor, out);
+  else
+    tile_stitch_kernel<false><<<grid, block, 0, as_stream(stream)>>>(tiles, X, Y, Z, g[0], g[1], g[2], to_hu, shift, factor, out);
+  CG_LAUNCH_CHECK("tile_stitch");
   return 0;
 }
 

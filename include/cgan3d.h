@@ -245,6 +245,21 @@ int cgan3d_tile_accumulate(const float *tile, float *acc, float *cnt, int X, int
                            int PX, int PY, int PZ, void *stream);
 int cgan3d_tile_finalize(const float *acc, const float *cnt, float *out, int64_t n, float shift, float factor,
                          void *stream);
+/* Tile grid with step (SX, SY, SZ), 1 <= S_a <= P_a <= extent: starts 0, S, 2S, ... <= extent - P per axis, then
+ * extent - P when the last regular tile stops short of the end; tile t = (ix * ny + iy) * nz + iz (z fastest).
+ * tile_extract_grid writes grid tiles t0 .. t0 + n - 1 (n <= 65535) as tiles[n][PX][PY][PZ], each bit-identical to
+ * cgan3d_tile_extract at its origin.                                                                              */
+#define CGAN3D_BLEND_AVG 0      /* w = 1 */
+#define CGAN3D_BLEND_GAUSSIAN 1 /* w = wx * wy * wz, w_a(i) = exp(-(i - (P_a - 1) / 2)^2 / (2 sigma_a^2)), sigma_a = P_a / 8 */
+int cgan3d_tile_extract_grid(const int16_t *vol, int X, int Y, int Z, int PX, int PY, int PZ, int SX, int SY, int SZ, int t0,
+                             int n, float shift, float factor, float *tiles, void *stream);
+/* out[X][Y][Z] = sum_t w(v - o_t) tiles[t](v - o_t) / sum_t w(v - o_t) over the n grid tiles covering v, summed in
+ * ascending t without atomics (deterministic); tiles is a DEVICE array of n pointers to [PX][PY][PZ] fp32 tiles.  With
+ * to_hu the result is unscaled, (sum / wsum) * factor + shift.  CGAN3D_BLEND_AVG performs the fp32 operations of
+ * cgan3d_tile_accumulate over the tiles in order followed by acc / cnt (and cgan3d_tile_finalize with to_hu);
+ * CGAN3D_BLEND_GAUSSIAN keeps a running weighted mean, m += (w / wsum) (c - m), exact for a constant input.          */
+int cgan3d_tile_stitch(const float *const *tiles, int n, int X, int Y, int Z, int PX, int PY, int PZ, int SX, int SY, int SZ,
+                       int blend, int to_hu, float shift, float factor, float *out, void *stream);
 /* out[B][X][Y][Z] = x - nearest_resize(att[B][Xa][Ya][Za] -> [X][Y][Z]): the corrector's `patch - nn.Upsample(size=
  * inference_patch_size)(G(patch))` branch, taken when the generator does not round-trip the patch size
  * (eval/CCTAContrastCorrector.py:42-52,79); aten::upsample_nearest3d index law (src = floor(dst * in/out)).        */
